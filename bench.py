@@ -4,7 +4,7 @@
 ml-1m run, saved_models/ml-1m.txt/sasrec_baseline_*/params.txt), full training step = forward + loss + backward +
 deterministic sparse embedding gradient + (all-reduce) + TF-Adam.
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--batch_size B] [--impl reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--batch_size B] [--impl reference] [--dump-outputs DIR]
 
 Prints ONE JSON line (rank 0).  `value` = whole-job sequences/s with inputs resident in HBM (CUDA-graph replay, CUDA
 events, max over ranks, L2 flushed between timed steps); `e2e` = the same through `SASRec.train_step(sync=False)` with HOST
@@ -298,6 +298,30 @@ def dp_parity_check(model, eng, c, dev_batches, B, world, rank, dev, shard):
             "global_batch": B * world, "item_table": "row-sharded" if shard else "replicated"}
 
 
+DUMP_LIMIT_BYTES = 64 << 20
+DUMP_TABLE_ROWS = 16384
+
+
+def dump_outputs(out_dir, eng):
+    """Writes what the last timed step handed its caller, as DIR/<name>.npy: `loss` and `auc` (float64, the values
+    `train_step` returns) and `param.<role name>` (float32, every parameter after the step's optimizer update).  A
+    table with more than DUMP_TABLE_ROWS rows is cut to a fixed seeded sample of its rows, the same rows on every run,
+    so that the outputs of two builds can be compared file by file."""
+    loss_sum, auc_sum, cnt = eng.global_sums()[:3].tolist()
+    arrays = {"loss": np.float64(loss_sum / cnt), "auc": np.float64(auc_sum / cnt)}
+    for name, t in eng.P.items():
+        if t.dim() == 2 and t.shape[0] > DUMP_TABLE_ROWS:   # rows picked on the device: only the sample is copied
+            rows = np.sort(np.random.RandomState(0).choice(t.shape[0], DUMP_TABLE_ROWS, replace=False))
+            t = t[torch.from_numpy(rows).to(t.device)]
+        arrays["param." + name] = t.cpu().numpy()
+    total = sum(v.nbytes for v in arrays.values())
+    if total > DUMP_LIMIT_BYTES:
+        raise RuntimeError(f"--dump-outputs would write {total} bytes (limit {DUMP_LIMIT_BYTES})")
+    os.makedirs(out_dir, exist_ok=True)
+    for name, v in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), v)
+
+
 def bench_config(batch_per_gpu, gpus):
     """the workload both arms name (identical dict in both lines; how each arm ran it is under `notes` / `sample`)"""
     return {"workload": WORKLOAD, "batch_per_gpu": batch_per_gpu, "global_batch": batch_per_gpu * gpus}
@@ -321,7 +345,13 @@ def main():
                     "table, its gradient and Adam slots per GPU, lookups over NVLink peer memory (default for "
                     "--config c5 when --gpus > 1)")
     ap.add_argument("--no_dp_parity", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write the loss, AUC and parameters "
+                    "of the last timed step (rank 0) as DIR/<name>.npy; same arguments, same inputs")
     a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
+    if a.dump_outputs and a.impl != "b200":
+        ap.error("--dump-outputs applies to --impl b200")
     select_config(a.config)
     if a.model:
         global WORKLOAD
@@ -412,6 +442,8 @@ def main():
         torch.distributed.all_reduce(t, op=torch.distributed.ReduceOp.MAX)
     t_dev = float(t.item())
     value = world * B * a.steps / t_dev
+    if a.dump_outputs and rank == 0:
+        dump_outputs(a.dump_outputs, eng)
 
     # ---- (2) end to end through the public API with host batches
     for i in range(3):

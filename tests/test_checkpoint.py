@@ -4,6 +4,7 @@ tests/golden/ml1m_sasrec_ckpt.npz, produced by tests/golden/make_golden.py with 
 LayerNorm betas are non-zero, so padded query rows are live and fully-masked rows are uniform over all T keys
 (SURVEY A-6/A-8) — the cases a textbook attention kernel gets wrong."""
 import os
+import struct
 
 import numpy as np
 import pytest
@@ -15,7 +16,6 @@ from cast_b200 import checkpoint as ck
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 FIX = os.path.join(HERE, "golden", "ml1m_sasrec_ckpt.npz")
-REF = "/root/reference/saved_models/ml-1m.txt/sasrec_baseline_10-19-2019-21-23-42/model.ckpt"
 
 
 def fixture_params():
@@ -41,13 +41,139 @@ def test_writer_reader_round_trip(tmp_path):
         assert np.array_equal(back[k], p[k]), k
 
 
-@pytest.mark.skipif(not os.path.isfile(REF + ".index"), reason="reference tree not present (GPU box)")
-def test_reader_parses_the_reference_checkpoint():
-    tfv = ck.read_bundle(REF)
-    assert len(tfv) == 99 and int(tfv["global_step"]) == 9400
+def test_block_entries_decodes_prefix_shared_keys():
+    """Known answer, bytes written by hand in the LevelDB block format TensorFlow's table writer uses: each entry is
+    varint(shared) varint(unshared) varint(value length) key-suffix value, a restart point every 2 entries here."""
+    body = (b"\x00\x05\x01apple" + b"1"       # offset 0, restart
+            + b"\x05\x01\x01t" + b"2"          # "apple" + "t"
+            + b"\x00\x05\x01apply" + b"3"      # offset 14, restart
+            + b"\x05\x05\x01/Adam" + b"4")     # "apply" + "/Adam"
+    block = body + struct.pack("<III", 0, 14, 2)
+    assert list(ck._block_entries(block)) == [(b"apple", b"1"), (b"applet", b"2"), (b"apply", b"3"),
+                                              (b"apply/Adam", b"4")]
+
+
+def _tf_block(pairs, restart_interval):
+    """One table block as TensorFlow's (LevelDB's) BlockBuilder lays it out: a key shares its prefix with the previous
+    key except at a restart point, every `restart_interval` entries."""
+    body, restarts, prev = bytearray(), [], b""
+    for i, (k, v) in enumerate(pairs):
+        shared = 0
+        if i % restart_interval == 0:
+            restarts.append(len(body))
+        else:
+            while shared < min(len(k), len(prev)) and k[shared] == prev[shared]:
+                shared += 1
+        body += ck._put_varint(shared) + ck._put_varint(len(k) - shared) + ck._put_varint(len(v)) + k[shared:] + v
+        prev = k
+    for r in restarts or [0]:
+        body += struct.pack("<I", r)
+    return bytes(body + struct.pack("<I", max(1, len(restarts))))
+
+
+def _separator(start, limit):
+    """LevelDB's BytewiseComparator::FindShortestSeparator: the index key between two data blocks"""
+    n = 0
+    while n < min(len(start), len(limit)) and start[n] == limit[n]:
+        n += 1
+    if n < min(len(start), len(limit)) and start[n] < 0xFF and start[n] + 1 < limit[n]:
+        return start[:n] + bytes([start[n] + 1])
+    return start
+
+
+def _successor(key):
+    """... FindShortSuccessor: the index key after the last data block"""
+    for i, b in enumerate(key):
+        if b != 0xFF:
+            return key[:i] + bytes([b + 1])
+    return key
+
+
+def _tf_table(pairs, block_size):
+    """SSTable with TensorFlow's defaults: data blocks cut at `block_size` bytes with a restart point every 16 keys,
+    an empty meta-index block, an index block of shortened separator keys (restart interval 1), the 48-byte footer.
+    Returns (file bytes, number of data blocks)."""
+    out, index, cur, last = bytearray(), [], [], None
+
+    def emit(block):
+        handle = ck._put_varint(len(out)) + ck._put_varint(len(block))
+        out.extend(ck._with_trailer(block))
+        return handle
+
+    for k, v in pairs:
+        if last is not None:
+            index.append((_separator(last[0], k), last[1]))
+            last = None
+        cur.append((k, v))
+        if len(_tf_block(cur, 16)) >= block_size:
+            last, cur = (k, emit(_tf_block(cur, 16))), []
+    if cur:
+        last = (cur[-1][0], emit(_tf_block(cur, 16)))
+    index.append((_successor(last[0]), last[1]))
+    meta = emit(_tf_block([], 16))
+    idx = emit(_tf_block(index, 1))
+    footer = meta + idx
+    return bytes(out + footer + b"\x00" * (40 - len(footer)) + struct.pack("<Q", ck._MAGIC)), len(index)
+
+
+def _tf_entry(dtype, shape, offset, size, crc):
+    """BundleEntryProto: dtype, shape, offset (omitted when 0), size, crc32c"""
+    dims = b"".join(b"\x12" + ck._put_varint(len(d)) + d for d in (b"\x08" + ck._put_varint(s) for s in shape))
+    e = b"\x08" + ck._put_varint(dtype) + b"\x12" + ck._put_varint(len(dims)) + dims
+    if offset:
+        e += b"\x20" + ck._put_varint(offset)
+    return e + b"\x28" + ck._put_varint(size) + b"\x35" + struct.pack("<I", crc)
+
+
+@pytest.mark.parametrize("block_size", [262144, 1024], ids=["tf_default_blocks", "small_blocks"])
+def test_reader_parses_a_tensorflow_layout_index(tmp_path, block_size):
+    """The reference's ml-1m SASRec checkpoint as tf.train.Saver wrote it: its 99 entries (32 weights, their Adam and
+    Adam_1 slots, beta1_power, beta2_power, global_step) with the masked crc32c TensorFlow stored for each
+    (tests/golden/ref_bundle_crc.npz), in an index laid out the way TensorFlow's table writer lays it out (prefix-shared
+    keys, restart points every 16 keys, shortened index keys; several data blocks when they are small).  The weights
+    are the fixture's, the other tensors seeded, stored in the data file in shuffled order at recorded offsets."""
+    g = np.load(os.path.join(HERE, "golden", "ref_bundle_crc.npz"))
+    crcs = dict(zip([str(x) for x in g["names"]], [int(x) for x in g["crcs"]]))
+    weights = ck.to_tf_names("sasrec", fixture_params(), 2)
+    rng = np.random.RandomState(0)
+    tensors = {}
+    for name in crcs:
+        if name in weights:
+            tensors[name] = weights[name]
+        elif name.endswith(("/Adam", "/Adam_1")):
+            tensors[name] = rng.rand(*weights[name.rsplit("/", 1)[0]].shape).astype(np.float32)
+        elif name == "global_step":
+            tensors[name] = np.asarray(np.load(FIX)["global_step"], np.int32)
+        else:
+            tensors[name] = np.asarray(rng.rand(), np.float32)
+    assert len(tensors) == 99
+    data, offsets = bytearray(), {}
+    for name in rng.permutation(sorted(tensors)):
+        offsets[name] = len(data)
+        data += tensors[name].tobytes()
+    pairs = [(b"", b"\x08\x01\x1a\x02\x08\x01")]            # BundleHeaderProto: num_shards 1, version {producer 1}
+    for name in sorted(tensors):
+        a = tensors[name]
+        pairs.append((name.encode(), _tf_entry({np.float32: 1, np.int32: 3}[a.dtype.type], a.shape, offsets[name],
+                                               a.nbytes, crcs[name])))
+    index, n_blocks = _tf_table(pairs, block_size)
+    assert (n_blocks == 1) == (block_size == 262144)
+    prefix = str(tmp_path / "model.ckpt")
+    with open(prefix + ".index", "wb") as f:
+        f.write(index)
+    with open(prefix + ".data-00000-of-00001", "wb") as f:
+        f.write(bytes(data))
+
+    assert ck.read_bundle_crcs(prefix) == crcs
+    tfv = ck.read_bundle(prefix)
+    assert sorted(tfv) == sorted(tensors)
+    assert int(tfv["global_step"]) == 9400 and tfv["global_step"].dtype == np.int32
     assert tfv["SASRec/input_embeddings/lookup_table/Adam_1"].shape == (3417, 50)   # optimizer slots are there too
-    p = ck.to_role_names("sasrec", tfv, 2)
+    for name, a in tensors.items():
+        assert tfv[name].dtype == a.dtype and np.array_equal(tfv[name], a), name
     fx = fixture_params()
+    p = ck.to_role_names("sasrec", tfv, 2)
+    assert sorted(p) == sorted(fx)
     for k in fx:
         assert np.array_equal(p[k], fx[k]), k
 
