@@ -100,6 +100,9 @@ SIGNATURES = {
     "cast_peer_barrier": (I, [P, I, I, P, P]),
     "cast_peer_reduce": (I, [P, I, L, P, P]),
     "cast_score_rank_full_status": (I, [P, L, I, P, P]),
+    "cast_topk_full_workspace_bytes": (SZ, [L, I, I, I]),
+    "cast_topk_full": (I, [P, L, P, I, I, L, I, P, P, I, P, P, P, P, SZ, P]),
+    "cast_topk_full_status": (I, [P, L, I, I, I, P, P]),
 }
 
 

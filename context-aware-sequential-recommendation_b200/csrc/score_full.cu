@@ -17,46 +17,9 @@
 // exact gather kernel, so the tensor-core pass needs no per-user mask.
 //
 // Exact path (mode 1): the same counts by brute-force canonical dots (small catalogs, validation of mode 0).
-#include "cast_rt.cuh"
-#ifndef CAST_EMU
-#include "umma.cuh"
-#endif
+#include "score_full.cuh"
 
 namespace cast {
-
-// canonical logit: sequential k, separately rounded multiply and add
-__device__ __forceinline__ float canonical_dot(const float* __restrict__ u, const float* __restrict__ e, int H) {
-  float acc = 0.f;
-  for (int k = 0; k < H; ++k) acc = __fadd_rn(acc, __fmul_rn(u[k], e[k]));
-  return acc;
-}
-
-constexpr float NORM_SLACK = 1.0001f;  // fp32 norm evaluation error, folded into the bound
-
-// inorm[j] >= |e_j|_2 (row 0 is the zero-pad row of the lookup table: never a candidate)
-__global__ void item_norm_kernel(const float* __restrict__ table, int V, int H, float* __restrict__ inorm) {
-  const int lane = threadIdx.x & 31;
-  const long j = (long)blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
-  if (j >= V) return;
-  float s = 0.f;
-  for (int k = lane; k < H; k += 32) {
-    const float x = table[j * H + k];
-    s = fmaf(x, x, s);
-  }
-  s = warp_sum(s);
-  if (lane == 0) inorm[j] = sqrtf(s) * NORM_SLACK;
-}
-
-// tnorm[t] = max of inorm over the 256 items of tile t (one warp per tile)
-__global__ void tile_norm_kernel(const float* __restrict__ inorm, int V, int tile, float* __restrict__ tnorm) {
-  const int lane = threadIdx.x & 31;
-  const long t = (long)blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
-  if (t * tile >= V) return;
-  float m = 0.f;
-  for (long j = t * tile + lane; j < (t + 1) * tile && j < V; j += 32) m = fmaxf(m, inorm[j]);
-  m = warp_max(m);
-  if (lane == 0) tnorm[t] = m;
-}
 
 // per user: |u|_2 bound and the canonical target score (target id outside [1,V) scores 0 like the zero-pad row)
 __global__ void user_prep_kernel(const float* __restrict__ users, long ldu, const float* __restrict__ table, int V,
@@ -133,89 +96,6 @@ __global__ void rated_subtract_kernel(const float* __restrict__ users, long ldu,
 }
 
 #ifndef CAST_EMU
-// ------------------------------------------------------------------------------------------------ tensor-core path
-// Warp-specialised pipeline, one persistent CTA per SM:
-//   warp 0 (one lane)  producer : TMA 1-D bulk copies (cp.async.bulk) of pre-split operand chunks into a 2-stage
-//                                 shared-memory ring, completion counted on `full[s]` as transaction bytes
-//   warp 1 (one lane)  MMA      : waits full[s], issues 3 x tcgen05.mma per 8 K-elements into one of TWO TMEM
-//                                 accumulators (2 x 256 columns), tcgen05.commit -> empty[s] (stage free) and, after the
-//                                 last K chunk of a tile, -> tfull[acc]
-//   warps 2-9          epilogue : wait tfull[acc], tcgen05.ld the 128 x 256 tile (thread <-> user row, two warps per
-//                                 lane quarter split the columns), two compares per element against per-(user, tile)
-//                                 thresholds, band pairs appended to a list, then arrive on tempty[acc]
-// so the copy of chunk k+1, the MMAs of chunk k and the epilogue of the previous tile overlap.  Operands are split
-// into tf32 hi/lo ONCE by presplit_kernel into the exact shared-memory image of a chunk (K-major slabs, see umma.cuh),
-// so the hot loop executes no conversion instructions at all: the item table is static for a whole evaluation.
-constexpr int SF_EPI_WARPS = 8;                // two warps per TMEM lane quarter (each takes half of the columns)
-constexpr int SF_THREADS = 64 + 32 * SF_EPI_WARPS;
-constexpr int SF_M = 128;                      // users per tile  (UMMA M)
-constexpr int SF_N = 256;                      // items per tile  (UMMA N); 2 accumulators = all 512 TMEM columns
-constexpr int SF_KC = 32;                      // K elements per pipeline chunk
-constexpr int SF_SLABS = SF_KC / 4;
-constexpr int SF_A_PITCH = SF_M * 16 + 16;     // bytes between K slabs of the user tile
-constexpr int SF_B_PITCH = SF_N * 16 + 16;     // bytes between K slabs of the item tile
-constexpr int SF_ABYTES = 2 * SF_SLABS * SF_A_PITCH;   // one user-tile chunk: hi slabs then lo slabs
-constexpr int SF_BBYTES = 2 * SF_SLABS * SF_B_PITCH;   // one item-tile chunk
-constexpr int SF_STAGES = 2;
-constexpr size_t SF_SMEM = (size_t)SF_STAGES * (SF_ABYTES + SF_BBYTES) + 128;
-
-// X [R, ld] row-major fp32 -> out[tile][kchunk][hi|lo][slab][TR rows x 16 B (+16 B pad)]; zero beyond R rows / H cols
-template <int TR>
-__global__ void presplit_kernel(const float* __restrict__ X, long ld, long R, int H, int nkc,
-                                unsigned char* __restrict__ out) {
-  constexpr int PITCH = TR * 16 + 16;
-  constexpr int CBYTES = 2 * SF_SLABS * PITCH;
-  const long tile = blockIdx.x;
-  const int kc = blockIdx.y;
-  unsigned char* dst = out + ((size_t)tile * nkc + kc) * CBYTES;
-  for (int idx = threadIdx.x; idx < TR * SF_SLABS; idx += blockDim.x) {
-    const int r = idx / SF_SLABS, c = idx - r * SF_SLABS;
-    const long row = tile * TR + r;
-    const int k = kc * SF_KC + 4 * c;
-    float x[4] = {0.f, 0.f, 0.f, 0.f};
-    if (row < R) {
-#pragma unroll
-      for (int e = 0; e < 4; ++e)
-        if (k + e < H) x[e] = __ldg(X + row * ld + k + e);
-    }
-    float4 h, l;
-    umma::split_tf32(x[0], h.x, l.x);
-    umma::split_tf32(x[1], h.y, l.y);
-    umma::split_tf32(x[2], h.z, l.z);
-    umma::split_tf32(x[3], h.w, l.w);
-    *reinterpret_cast<float4*>(dst + (size_t)c * PITCH + r * 16) = h;
-    *reinterpret_cast<float4*>(dst + (size_t)(SF_SLABS + c) * PITCH + r * 16) = l;
-  }
-}
-
-struct ScoreFullArgs {
-  const float* users;
-  long ldu;
-  const float* table;
-  const unsigned char* apre;   // pre-split user tiles
-  const unsigned char* bpre;   // pre-split item tiles
-  const float* inorm;
-  const float* tnorm;          // per item tile: max of inorm over the tile
-  const float* tscore;
-  const float* unorm;
-  const int* target;
-  int V, H;
-  long U;
-  int nkc;               // K chunks of SF_KC elements
-  int kpad;              // H rounded up to 8
-  long items_per_split;  // multiple of SF_N
-  int nsplit;
-  long nunits;
-  float cbound;
-  int* cgt;
-  int* ceq;
-  unsigned long long* stats;  // [0] band candidates re-scored exactly  (optional)
-  unsigned long long* band_count;   // device counter of deferred band pairs
-  int2* band_pairs;                 // (user, item) pairs inside the error band, re-scored by band_rescore_kernel
-  unsigned long long band_cap;
-  int* err;
-};
-
 // Deferred exact decisions: one thread per (user, item) pair that the tensor-core pass could not classify.  The
 // canonical dot is a sequential chain, so the parallelism is across pairs (inline in the epilogue it would stall a
 // whole warp per pair: measured 9 ms -> see profiles/r01e).
@@ -235,218 +115,85 @@ __global__ void band_rescore_kernel(const float* __restrict__ users, long ldu, c
   }
 }
 
-__global__ void __launch_bounds__(SF_THREADS, 1) score_full_umma_kernel(ScoreFullArgs a) {
-  extern __shared__ __align__(128) unsigned char sf_smem[];
-  __shared__ __align__(8) uint64_t full[SF_STAGES], empty[SF_STAGES], tfull[2], tempty[2], afull, adone;
-  __shared__ uint32_t tmem_slot;
-  const int t = threadIdx.x, lane = t & 31, warp = t >> 5;
-  // small K: the user tile stays resident (loaded once per work unit) and the ring holds item chunks only
-  const bool a_res = a.nkc <= SF_STAGES;
-  unsigned char* Ares = sf_smem;
-  unsigned char* ring = a_res ? sf_smem + (size_t)SF_STAGES * SF_ABYTES : sf_smem;
-  const int stage_bytes = a_res ? SF_BBYTES : SF_ABYTES + SF_BBYTES;
-  if (warp == 1) umma::tmem_alloc(&tmem_slot, 2 * SF_N);
-  if (t == 0) {
-    for (int i = 0; i < SF_STAGES; ++i) { umma::mbar_init(&full[i], 1); umma::mbar_init(&empty[i], 1); }
-    for (int i = 0; i < 2; ++i) { umma::mbar_init(&tfull[i], 1); umma::mbar_init(&tempty[i], SF_EPI_WARPS); }
-    umma::mbar_init(&afull, 1);
-    umma::mbar_init(&adone, 1);
-  }
-  umma::fence_before_sync();
-  __syncthreads();
-  umma::fence_after_sync();
-  const uint32_t tmem = tmem_slot;
-  bool failed = false;
+// Epilogue of the tensor-core pass (sf_umma_kernel<CountEpi>): two compares per element against per-(user, tile)
+// thresholds, band pairs appended to a list.
+struct CountEpi {
+  struct Params {
+    const float* tscore;
+    const int* target;
+    int* cgt;
+    int* ceq;
+    unsigned long long* stats;        // [0] band candidates re-scored exactly  (optional)
+    unsigned long long* band_count;   // device counter of deferred band pairs
+    int2* band_pairs;                 // (user, item) pairs inside the error band, re-scored by band_rescore_kernel
+    unsigned long long band_cap;
+  };
+  const SfPipe& a;
+  const Params& p;
+  const long me;
+  const int je;
+  const float tsc;
+  const int tgt;
+  int gt = 0;
+  unsigned band = 0;
+  float hi = 0.f, lo = 0.f;
+  bool interior = false;
 
-  if (warp == 0) {
-    // ================================================================== producer
-    if (lane == 0) {
-      uint32_t it = 0;          // ring position counter
-      uint32_t units_done = 0;
-      for (long unit = blockIdx.x; unit < a.nunits && !failed; unit += gridDim.x, ++units_done) {
-        const long ut = unit / a.nsplit;
-        const int sp = (int)(unit - ut * a.nsplit);
-        const long jb = (long)sp * a.items_per_split;
-        const long je = jb + a.items_per_split < a.V ? jb + a.items_per_split : a.V;
-        const unsigned char* asrc = a.apre + (size_t)ut * a.nkc * SF_ABYTES;
-        if (a_res) {
-          if (units_done > 0 && !umma::mbar_wait(&adone, (units_done - 1) & 1)) { failed = true; break; }
-          umma::mbar_arrive_expect_tx(&afull, (uint32_t)(a.nkc * SF_ABYTES));
-          for (int kc = 0; kc < a.nkc; ++kc) umma::bulk_g2s(Ares + (size_t)kc * SF_ABYTES, asrc + (size_t)kc * SF_ABYTES,
-                                                            SF_ABYTES, &afull);
-        }
-        for (long j0 = jb; j0 < je && !failed; j0 += SF_N) {
-          const unsigned char* bsrc = a.bpre + (size_t)(j0 / SF_N) * a.nkc * SF_BBYTES;
-          for (int kc = 0; kc < a.nkc; ++kc, ++it) {
-            const int s = it % SF_STAGES;
-            const uint32_t round = it / SF_STAGES;
-            if (!umma::mbar_wait(&empty[s], (round & 1) ^ 1)) { failed = true; break; }
-            unsigned char* dst = ring + (size_t)s * stage_bytes;
-            if (a_res) {
-              umma::mbar_arrive_expect_tx(&full[s], SF_BBYTES);
-              umma::bulk_g2s(dst, bsrc + (size_t)kc * SF_BBYTES, SF_BBYTES, &full[s]);
-            } else {
-              umma::mbar_arrive_expect_tx(&full[s], SF_ABYTES + SF_BBYTES);
-              umma::bulk_g2s(dst, asrc + (size_t)kc * SF_ABYTES, SF_ABYTES, &full[s]);
-              umma::bulk_g2s(dst + SF_ABYTES, bsrc + (size_t)kc * SF_BBYTES, SF_BBYTES, &full[s]);
-            }
-          }
-        }
+  __device__ __forceinline__ CountEpi(const SfPipe& a_, const Params& p_, long me_, bool live, int, int, int,
+                                      int je_)
+      : a(a_), p(p_), me(me_), je(je_), tsc(live ? p_.tscore[me_] : 0.f), tgt(live ? p_.target[me_] : -1) {}
+
+  // above `hi` is certainly greater, below `lo` certainly smaller, in between the canonical fp32 logit decides
+  // (deferred)
+  __device__ __forceinline__ void tile(int j0, float d) {
+    hi = tsc + d;
+    lo = tsc - d;
+    interior = j0 >= 1 && j0 + SF_N <= je && (tgt < j0 || tgt >= j0 + SF_N);  // no per-item exclusions
+  }
+
+  __device__ __forceinline__ void chunk(const float (&v)[32], int j) {
+    unsigned inband = 0;
+    if (interior) {
+#pragma unroll
+      for (int e = 0; e < 32; ++e) {
+        gt += v[e] > hi ? 1 : 0;
+        inband |= (v[e] >= lo && !(v[e] > hi)) ? (1u << e) : 0u;
+      }
+    } else {
+#pragma unroll
+      for (int e = 0; e < 32; ++e) {
+        const int item = j + e;
+        const bool valid = item >= 1 && item < je && item != tgt;
+        gt += (valid && v[e] > hi) ? 1 : 0;
+        inband |= (valid && v[e] >= lo && !(v[e] > hi)) ? (1u << e) : 0u;
       }
     }
-  } else if (warp == 1) {
-    // ================================================================== MMA issuer
-    if (lane == 0) {
-      const uint32_t idesc = umma::idesc_tf32(SF_M, SF_N);
-      // descriptors are built once; inside the loops a k-step costs four 64-bit adds and three MMAs (the issuing
-      // thread is latency-bound on its own instruction stream)
-      uint64_t dA[SF_STAGES], dB[SF_STAGES];
-#pragma unroll
-      for (int s = 0; s < SF_STAGES; ++s) {
-        const unsigned char* st = ring + (size_t)s * stage_bytes;
-        dA[s] = umma::smem_desc(umma::smem_u32(a_res ? Ares + (size_t)s * SF_ABYTES : st), SF_A_PITCH, 128);
-        dB[s] = umma::smem_desc(umma::smem_u32(a_res ? st : st + SF_ABYTES), SF_B_PITCH, 128);
+    while (inband) {  // rare: hand the pair to band_rescore_kernel
+      const int e = __ffs((int)inband) - 1;
+      inband &= inband - 1;
+      const int item = j + e;
+      const unsigned long long slot = atomicAdd(p.band_count, 1ull);
+      if (slot < p.band_cap) {
+        p.band_pairs[slot] = make_int2((int)me, item);
+      } else {  // list full: decide here (slow path)
+        const float ex = canonical_dot(a.users + me * a.ldu, a.table + (long)item * a.H, a.H);
+        if (ex > tsc) ++gt;
+        else if (ex == tsc) atomicAdd(&p.ceq[me], 1);
       }
-      uint32_t it = 0, tile_no = 0, units_done = 0;
-      for (long unit = blockIdx.x; unit < a.nunits && !failed; unit += gridDim.x, ++units_done) {
-        const long ut = unit / a.nsplit;
-        const int sp = (int)(unit - ut * a.nsplit);
-        const long jb = (long)sp * a.items_per_split;
-        const long je = jb + a.items_per_split < a.V ? jb + a.items_per_split : a.V;
-        if (a_res && !umma::mbar_wait(&afull, units_done & 1)) { failed = true; break; }
-        for (long j0 = jb; j0 < je && !failed; j0 += SF_N, ++tile_no) {
-          const uint32_t acc = tile_no & 1;
-          if (!umma::mbar_wait(&tempty[acc], ((tile_no >> 1) & 1) ^ 1)) { failed = true; break; }
-          umma::fence_after_sync();
-          const uint32_t dcol = tmem + acc * SF_N;
-          for (int kc = 0; kc < a.nkc; ++kc, ++it) {
-            const int s = it % SF_STAGES;
-            if (!umma::mbar_wait(&full[s], (it / SF_STAGES) & 1)) { failed = true; break; }
-            umma::fence_after_sync();
-            // resident user tile: chunk kc lives in slot kc (nkc <= SF_STAGES); streamed: in the ring stage
-            const uint64_t dah = a_res ? (kc == 0 ? dA[0] : dA[1]) : (s == 0 ? dA[0] : dA[1]);
-            const uint64_t dbh = s == 0 ? dB[0] : dB[1];
-            const int kleft = a.kpad - kc * SF_KC;
-            const int ksteps = (kleft < SF_KC ? kleft : SF_KC) / 8;
-#pragma unroll
-            for (int ks = 0; ks < SF_KC / 8; ++ks) {
-              if (ks < ksteps) {
-                const uint64_t ah = umma::desc_advance(dah, 2 * ks * SF_A_PITCH);
-                const uint64_t al = umma::desc_advance(dah, (SF_SLABS + 2 * ks) * SF_A_PITCH);
-                const uint64_t bh = umma::desc_advance(dbh, 2 * ks * SF_B_PITCH);
-                const uint64_t bl = umma::desc_advance(dbh, (SF_SLABS + 2 * ks) * SF_B_PITCH);
-                umma::mma_tf32(dcol, al, bh, idesc, (kc > 0 || ks > 0) ? 1u : 0u);
-                umma::mma_tf32(dcol, ah, bl, idesc, 1u);
-                umma::mma_tf32(dcol, ah, bh, idesc, 1u);
-              }
-            }
-            umma::mma_commit(&empty[s]);   // stage s may be refilled once these MMAs have read it
-          }
-          if (!failed) umma::mma_commit(&tfull[acc]);
-        }
-        if (a_res && !failed) umma::mma_commit(&adone);
-      }
-    }
-  } else {
-    // ================================================================== epilogue (warps 2..9, thread <-> user row)
-    const uint32_t q = warp & 3;               // TMEM lane quarter this warp may read
-    const int chalf = (warp - 2) >> 2;         // which half of the 256 columns it takes
-    uint32_t tile_no = 0;
-    for (long unit = blockIdx.x; unit < a.nunits && !failed; unit += gridDim.x) {
-      const long ut = unit / a.nsplit;
-      const int sp = (int)(unit - ut * a.nsplit);
-      const int jb = (int)((long)sp * a.items_per_split);
-      const int je = (long)jb + a.items_per_split < a.V ? (int)(jb + a.items_per_split) : a.V;
-      const long me = ut * SF_M + q * 32 + lane;
-      const bool live = me < a.U;
-      const float tsc = live ? a.tscore[me] : 0.f;
-      const float nu = live ? a.unorm[me] * a.cbound : 0.f;
-      const int tgt = live ? a.target[me] : -1;
-      int gt = 0;
-      unsigned band = 0;
-      for (int j0 = jb; j0 < je && !failed; j0 += SF_N, ++tile_no) {
-        const uint32_t acc = tile_no & 1;
-        const bool ok = umma::mbar_wait(&tfull[acc], (tile_no >> 1) & 1);
-        if (!__all_sync(0xffffffffu, ok)) { failed = true; break; }
-        umma::fence_after_sync();
-        // |s~ - s| <= nu * |e_j| <= d for every item of the tile: above `hi` is certainly greater, below `lo`
-        // certainly smaller, in between the canonical fp32 logit decides (deferred)
-        const float d = nu * __ldg(a.tnorm + j0 / SF_N);
-        const float hi = tsc + d, lo = tsc - d;
-        const bool interior = j0 >= 1 && j0 + SF_N <= je && (tgt < j0 || tgt >= j0 + SF_N);  // no per-item exclusions
-#pragma unroll 1
-        for (int cb = chalf * (SF_N / 2); cb < (chalf + 1) * (SF_N / 2); cb += 32) {
-          float v[32];
-          umma::tmem_ld32(tmem + ((q * 32u) << 16) + acc * SF_N + (uint32_t)cb, v);
-          if (!live) continue;
-          unsigned inband = 0;
-          if (interior) {
-#pragma unroll
-            for (int e = 0; e < 32; ++e) {
-              gt += v[e] > hi ? 1 : 0;
-              inband |= (v[e] >= lo && !(v[e] > hi)) ? (1u << e) : 0u;
-            }
-          } else {
-#pragma unroll
-            for (int e = 0; e < 32; ++e) {
-              const int item = j0 + cb + e;
-              const bool valid = item >= 1 && item < je && item != tgt;
-              gt += (valid && v[e] > hi) ? 1 : 0;
-              inband |= (valid && v[e] >= lo && !(v[e] > hi)) ? (1u << e) : 0u;
-            }
-          }
-          while (inband) {  // rare: hand the pair to band_rescore_kernel
-            const int e = __ffs((int)inband) - 1;
-            inband &= inband - 1;
-            const int item = j0 + cb + e;
-            const unsigned long long slot = atomicAdd(a.band_count, 1ull);
-            if (slot < a.band_cap) {
-              a.band_pairs[slot] = make_int2((int)me, item);
-            } else {  // list full: decide here (slow path)
-              const float ex = canonical_dot(a.users + me * a.ldu, a.table + (long)item * a.H, a.H);
-              if (ex > tsc) ++gt;
-              else if (ex == tsc) atomicAdd(&a.ceq[me], 1);
-            }
-            ++band;
-          }
-        }
-        umma::fence_before_sync();
-        __syncwarp();
-        if (lane == 0) umma::mbar_arrive(&tempty[acc]);   // this warp's share of the accumulator is free
-      }
-      if (live && !failed) {
-        if (gt) atomicAdd(&a.cgt[me], gt);
-        if (a.stats && band) atomicAdd(&a.stats[0], (unsigned long long)band);
-      }
+      ++band;
     }
   }
-  if (failed) atomicExch(a.err, 1);
-  __syncthreads();
-  if (warp == 1) umma::tmem_free(tmem, 2 * SF_N);
-}
+
+  __device__ __forceinline__ void finish() {
+    if (gt) atomicAdd(&p.cgt[me], gt);
+    if (p.stats && band) atomicAdd(&p.stats[0], (unsigned long long)band);
+  }
+};
 #endif  // !CAST_EMU
 
 }  // namespace cast
 
 using namespace cast;
-
-static inline size_t sf_align(size_t x) { return (x + 255) & ~(size_t)255; }
-
-// tensor-core pass only: pre-split operand images (users: 128-row tiles, items: 256-row tiles)
-static size_t sf_presplit_bytes(long U, int V, int H, size_t* a_bytes) {
-#ifndef CAST_EMU
-  const int kpad = (H + 7) & ~7;
-  const size_t nkc = (size_t)cdiv(kpad, SF_KC);
-  const size_t ab = (size_t)cdiv(U, SF_M) * nkc * SF_ABYTES;
-  const size_t bb = (size_t)cdiv(V, SF_N) * nkc * SF_BBYTES;
-  if (a_bytes) *a_bytes = sf_align(ab);
-  return sf_align(ab) + sf_align(bb);
-#else
-  (void)U; (void)V; (void)H;
-  if (a_bytes) *a_bytes = 0;
-  return 0;
-#endif
-}
 
 // capacity of the deferred band list: 0.5 % of the (user, item) pairs, at least 64k (overflow is handled inline)
 static unsigned long long sf_band_cap(long U, int V) {
@@ -495,52 +242,22 @@ extern "C" int cast_score_rank_full(const float* seq_last, long ld, const float*
     if ((rc = check_launch("score_full(exact)"))) return rc;
   } else {
 #ifndef CAST_EMU
-    CAST_LAUNCH(item_norm_kernel, dim3((unsigned)cdiv(V, 8)), dim3(256), 0, st, table, V, H, inorm);
-    if ((rc = check_launch("score_full(item_norm)"))) return rc;
-    ScoreFullArgs a;
-    a.users = seq_last; a.ldu = ld; a.table = table; a.inorm = inorm; a.tscore = tscore; a.unorm = unorm;
-    a.target = target; a.V = V; a.H = H; a.U = U;
-    a.kpad = (H + 7) & ~7;
-    a.nkc = (int)cdiv(a.kpad, SF_KC);
-    const long utiles = cdiv(U, SF_M);
-    size_t a_bytes = 0;
-    sf_presplit_bytes(U, V, H, &a_bytes);
-    unsigned char* apre = w + sf_align((size_t)V * 4) + 2 * sf_align((size_t)U * 4) + 256;
-    unsigned char* bpre = apre + a_bytes;
-    presplit_kernel<SF_M><<<dim3((unsigned)utiles, (unsigned)a.nkc), 256, 0, st>>>(seq_last, ld, U, H, a.nkc, apre);
-    presplit_kernel<SF_N><<<dim3((unsigned)cdiv(V, SF_N), (unsigned)a.nkc), 256, 0, st>>>(table, H, V, H, a.nkc, bpre);
-    if ((rc = check_launch("score_full(presplit)"))) return rc;
-    a.apre = apre; a.bpre = bpre;
-    size_t pre_total = sf_presplit_bytes(U, V, H, nullptr);
-    a.band_pairs = reinterpret_cast<int2*>(apre + pre_total);
-    a.band_cap = sf_band_cap(U, V);
-    a.band_count = reinterpret_cast<unsigned long long*>(err + 2);   // inside the 256-byte flag block
-    cudaMemsetAsync(a.band_count, 0, sizeof(unsigned long long), st);
-    float* tnorm = reinterpret_cast<float*>(reinterpret_cast<unsigned char*>(a.band_pairs) +
-                                            sf_align((size_t)a.band_cap * sizeof(int2)));
-    tile_norm_kernel<<<dim3((unsigned)cdiv(cdiv(V, SF_N), 8)), dim3(256), 0, st>>>(inorm, V, SF_N, tnorm);
-    a.tnorm = tnorm;
-    const long ntile_items = cdiv(V, SF_N);
-    long nsplit = cdiv(148L * 2, utiles);          // ~2 work units per SM
-    if (nsplit > ntile_items) nsplit = ntile_items;
-    if (nsplit < 1) nsplit = 1;
-    a.items_per_split = cdiv(ntile_items, nsplit) * SF_N;
-    a.nsplit = (int)cdiv(V, a.items_per_split);
-    a.nunits = utiles * a.nsplit;
-    // |s~ - s| <= cbound * |u| * |e_j|: three dropped/rounded split terms (3 * 2^-22) plus one accumulation error of at
-    // most 2^-22 * sum|u_k e_k| per MMA (3 * kpad/8 MMAs per tile); doubled for slack
-    a.cbound = 2.0f * (3.0f + 3.0f * (float)a.kpad / 8.0f) * 2.384185791015625e-07f;
-    a.cgt = count_greater; a.ceq = count_equal; a.stats = stats; a.err = err;
-    static bool configured = false;
-    if (!configured) {
-      cudaFuncSetAttribute(score_full_umma_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)SF_SMEM);
-      configured = true;
-    }
-    const long grid = a.nunits < 148 ? a.nunits : 148;
-    score_full_umma_kernel<<<dim3((unsigned)grid), dim3(SF_THREADS), SF_SMEM, st>>>(a);
-    if ((rc = check_launch("score_full(umma)"))) return rc;
+    SfPipe a;
+    unsigned char* pre = w + sf_align((size_t)V * 4) + 2 * sf_align((size_t)U * 4) + 256;
+    CountEpi::Params ep;
+    ep.band_pairs = reinterpret_cast<int2*>(pre + sf_presplit_bytes(U, V, H, nullptr));
+    ep.band_cap = sf_band_cap(U, V);
+    ep.band_count = reinterpret_cast<unsigned long long*>(err + 2);   // inside the 256-byte flag block
+    cudaMemsetAsync(ep.band_count, 0, sizeof(unsigned long long), st);
+    float* tnorm = reinterpret_cast<float*>(reinterpret_cast<unsigned char*>(ep.band_pairs) +
+                                            sf_align((size_t)ep.band_cap * sizeof(int2)));
+    if ((rc = sf_prepare(a, seq_last, ld, table, V, H, U, pre, inorm, tnorm, st, "score_full(prepare)"))) return rc;
+    a.unorm = unorm; a.err = err;
+    sf_set_split(a, cdiv(148L * 2, cdiv(U, SF_M)));   // ~2 work units per SM
+    ep.tscore = tscore; ep.target = target; ep.cgt = count_greater; ep.ceq = count_equal; ep.stats = stats;
+    if ((rc = sf_launch<CountEpi>(a, ep, st, "score_full(umma)"))) return rc;
     band_rescore_kernel<<<dim3(148 * 8), dim3(256), 0, st>>>(seq_last, ld, table, H, (const float*)tscore,
-                                                             (const int2*)a.band_pairs, a.band_count, a.band_cap,
+                                                             (const int2*)ep.band_pairs, ep.band_count, ep.band_cap,
                                                              count_greater, count_equal);
     if ((rc = check_launch("score_full(band)"))) return rc;
 #endif

@@ -47,6 +47,25 @@ def _draw_negatives(rng, itemnum: int, member: np.ndarray, n: int = 100) -> np.n
     return out
 
 
+def _featurise(hist, T: int, args, log_scale: bool, lo, hi):
+    """One left-padded input row of the newest len(hist) <= T events: item ids, time bins relative to the newest input
+    event (util.py:276-289), hours, weekdays, raw timestamps."""
+    k = len(hist)
+    seq = np.zeros(T, np.int32)
+    timeseq = np.zeros(T, np.int32)
+    hours = np.zeros(T, np.int32)
+    days = np.zeros(T, np.int32)
+    seq[T - k:] = [x.item for x in hist]
+    hours[T - k:] = [x.ts.hour for x in hist]
+    days[T - k:] = [x.ts.day for x in hist]
+    t = np.fromiter((raw_ts(x) for x in hist), dtype=np.int64, count=k)
+    # bins relative to the newest INPUT event; the valid->test delta the reference computes first is overwritten
+    timeseq[T - k:] = timedelta_bins((t[-1] - t).astype(np.float64), args.bin_in_hours, args.max_bins, log_scale, lo, hi)
+    tsraw = np.zeros(T, np.int64)
+    tsraw[T - k:] = t
+    return seq, timeseq, hours, days, tsraw
+
+
 def build_candidates(dataset, args, split: str = "test", rng=None):
     """Everything `model.predict` is fed for every evaluated user, in the reference's user order.
 
@@ -71,25 +90,12 @@ def build_candidates(dataset, args, split: str = "test", rng=None):
         if len(tr) < 1 or len(target_of[u]) < 1:
             continue
         hist = list(tr[-T:]) if split == "valid" else list(tr[-(T - 1):] if T > 1 else []) + [valid[u][0]]
-        k = len(hist)
-        seq = np.zeros(T, np.int32)
-        timeseq = np.zeros(T, np.int32)
-        hours = np.zeros(T, np.int32)
-        days = np.zeros(T, np.int32)
-        seq[T - k:] = [x.item for x in hist]
-        hours[T - k:] = [x.ts.hour for x in hist]
-        days[T - k:] = [x.ts.day for x in hist]
-        t = np.fromiter((raw_ts(x) for x in hist), dtype=np.int64, count=k)
-        # bins relative to the newest INPUT event; the valid->test delta the reference computes first is overwritten
-        timeseq[T - k:] = timedelta_bins((t[-1] - t).astype(np.float64), args.bin_in_hours, args.max_bins, log_scale,
-                                         lo, hi)
+        seq, timeseq, hours, days, tsraw = _featurise(hist, T, args, log_scale, lo, hi)
         items = np.fromiter((x.item for x in tr), dtype=np.int64, count=len(tr))
         member[items] = True
         member[0] = True
         neg = _draw_negatives(rng, itemnum, member)
         member[items] = False
-        tsraw = np.zeros(T, np.int64)
-        tsraw[T - k:] = t
         if trunc is not None:  # util.py:300-315 (--test_model / --test_seq_len)
             seq[:-trunc] = 0
             timeseq[:-trunc] = 0
@@ -108,6 +114,64 @@ def build_candidates(dataset, args, split: str = "test", rng=None):
     return {"u": np.asarray(us, np.int32), "seq": st(seqs, T), "item_idx": st(cands, 101), "timeseq": st(tss, T),
             "hours": st(hrs, T), "days": st(dys, T), "rated": rated,
             "tsraw": np.stack(raws) if raws else np.zeros((0, T), np.int64)}   # for the device-side feature path
+
+
+def build_recommend_inputs(dataset, args):
+    """Inputs for recommending each user's next items: the last maxlen events of train + valid + test (users without
+    events are skipped), featurised as in build_candidates (no --test_seq_len truncation), and the ids of the whole
+    history as the exclusion set.  Draws no random numbers.
+    Returns dict(u [U], seq, timeseq, hours, days [U,T] int32, tsraw [U,T] int64, rated: list of id arrays)."""
+    train, valid, test, usernum = dataset[0], dataset[1], dataset[2], dataset[3]
+    T = args.maxlen
+    log_scale = bool(args.log_scale)
+    lo, hi = get_delta_range(train)
+    us, seqs, tss, hrs, dys, raws, rated = [], [], [], [], [], [], []
+    for u in range(1, usernum + 1):
+        full = list(train.get(u, [])) + list(valid.get(u, [])) + list(test.get(u, []))
+        if not full:
+            continue
+        seq, timeseq, hours, days, tsraw = _featurise(full[-T:], T, args, log_scale, lo, hi)
+        us.append(u)
+        seqs.append(seq)
+        tss.append(timeseq)
+        hrs.append(hours)
+        dys.append(days)
+        raws.append(tsraw)
+        rated.append(np.unique(np.fromiter((x.item for x in full), dtype=np.int64, count=len(full))).astype(np.int32))
+    st = lambda a, dt: np.stack(a) if a else np.zeros((0, T), dt)  # noqa: E731
+    return {"u": np.asarray(us, np.int32), "seq": st(seqs, np.int32), "timeseq": st(tss, np.int32),
+            "hours": st(hrs, np.int32), "days": st(dys, np.int32), "tsraw": st(raws, np.int64), "rated": rated}
+
+
+def recommend_users(model, inputs, k: int, batch_users: int = 256, lo: int = 0, hi: Optional[int] = None,
+                    mode: int = 0):
+    """model.recommend over rows [lo, hi) of build_recommend_inputs' output, with each user's history excluded; fixed
+    batch shape (tail padded as in score_users).  Returns (ids [n,k] int32, scores [n,k] float32)."""
+    hi = len(inputs["u"]) if hi is None else hi
+    n_all = max(0, hi - lo)
+    ids = np.zeros((n_all, k), np.int32)
+    scores = np.zeros((n_all, k), np.float32)
+    B = max(1, min(batch_users, max(1, n_all)))
+    for s in range(lo, hi, B):
+        e = min(hi, s + B)
+        n = e - s
+
+        def pad(a):
+            if n == B:
+                return a[s:e]
+            out = np.zeros((B,) + a.shape[1:], a.dtype)
+            out[:n] = a[s:e]
+            return out
+
+        excl = list(inputs["rated"][s:e]) + [np.zeros(0, np.int32)] * (B - n)
+        if getattr(model, "timefeat", None) is not None:
+            i, sc = model.recommend(pad(inputs["seq"]), k, excl, timestamps=pad(inputs["tsraw"]), mode=mode)
+        else:
+            i, sc = model.recommend(pad(inputs["seq"]), k, excl, pad(inputs["timeseq"]), pad(inputs["hours"]),
+                                    pad(inputs["days"]), mode=mode)
+        ids[s - lo:e - lo] = i[:n]
+        scores[s - lo:e - lo] = sc[:n]
+    return ids, scores
 
 
 def reference_rank(logits_row: np.ndarray) -> int:

@@ -172,6 +172,98 @@ class _Model:
                       eng.P["item_emb"].shape[0], eng.H, B, cand.data_ptr(), Cn, logits.data_ptr(), p(cgt), p(ceq),
                       eng._stream())
 
+    def _id_csr(self, lists, n, local_rows=False):
+        """Per-user id collections -> CSR device tensors (ptr [n+1], idx), ids unique and ascending per user.
+        local_rows=True (row-sharded table): keeps the ids this rank's shard holds, as local rows (id // n_ranks, +1 on
+        ranks > 0) — the map is increasing, so each row stays ascending."""
+        eng = self.engine
+        ptr = np.zeros(n + 1, np.int32)
+        flat = []
+        for u, r in enumerate(lists):
+            ids = np.unique(np.asarray(list(r), dtype=np.int64))
+            if local_rows:
+                rank, world = eng.item_shard
+                ids = ids[(ids % world == rank) & (ids > 0) & (ids < eng.V_items)] // world + (1 if rank else 0)
+            flat.append(ids)
+            ptr[u + 1] = ptr[u] + len(ids)
+        idx = np.concatenate(flat + [np.zeros(1, np.int64)]).astype(np.int32)
+        return torch.from_numpy(ptr).to(eng.device), torch.from_numpy(idx).to(eng.device)
+
+    def _topk(self, last, ld, U, V, k, eptr, eidx, mode):
+        """cast_topk_full over the rows [0, V) of this process's item table; (ids, scores) [U, k] device tensors"""
+        import ctypes
+        eng = self.engine
+        dev = eng.device
+        table = eng.P["item_emb"]
+        ids = torch.empty(U, k, dtype=torch.int32, device=dev)
+        scores = torch.empty(U, k, dtype=torch.float32, device=dev)
+        wsb = eng.lib.cast_topk_full_workspace_bytes(U, V, eng.H, k)
+        ws = self._pinned.get("tkws")     # one buffer, grown on demand (the operand images of a large catalog are GBs)
+        if ws is None or ws.numel() * 4 < wsb:
+            self._pinned["tkws"] = None
+            ws = self._pinned["tkws"] = torch.empty(wsb // 4 + 16, dtype=torch.int32, device=dev)
+        eng._call(eng.lib.cast_topk_full, last.data_ptr(), ld, table.data_ptr(), V, eng.H, U, k, eng._p(eptr),
+                  eng._p(eidx), mode, ids.data_ptr(), scores.data_ptr(), None, ws.data_ptr(), wsb, eng._stream())
+        if mode == 0:
+            flag = ctypes.c_int(0)
+            eng._call(eng.lib.cast_topk_full_status, ws.data_ptr(), U, V, eng.H, k, ctypes.byref(flag), eng._stream())
+            if flag.value != 0:
+                raise RuntimeError("topk_full: tensor-core pass watchdog fired")
+        return ids, scores
+
+    def recommend(self, seq, k=10, exclude=None, time_seq=None, hours=None, days=None, timestamps=None, mode: int = 0):
+        """Exact top-k recommendation from the last position of each sequence: the k items of [1, itemnum] not in
+        exclude[u] (optional, one id collection per user) with the largest canonical fp32 logits (the logits of
+        score_candidates / predict), ties broken by item id ascending.  mode 0 = tcgen05 tensor cores as an exact
+        filter, mode 1 = exact brute force; both return the same bits.  Returns (ids [U,k] int32, scores [U,k] float32);
+        fewer than k eligible items pad the tail with id 0 and score -inf.  With a row-sharded item table this is a
+        collective call (every rank passes its own users, the same count on every rank)."""
+        eng = self.engine
+        if eng.item_shard is not None:
+            return self._recommend_sharded(seq, k, exclude, time_seq, hours, days, timestamps, mode)
+        c = self.forward_eval(seq, time_seq, hours, days, timestamps=timestamps)
+        B, T, H = c.B, eng.T, eng.H
+        eptr, eidx = self._id_csr(exclude, B) if exclude is not None else (None, None)
+        last = c.seq_emb.view(B, T, H)[:, T - 1, :]
+        ids, scores = self._topk(last, T * H, B, eng.P["item_emb"].shape[0], k, eptr, eidx, mode)
+        return ids.cpu().numpy(), scores.cpu().numpy()
+
+    def _recommend_sharded(self, seq, k, exclude, time_seq, hours, days, timestamps, mode):
+        """Top-k with the item table sharded by row: the last-position vectors of all ranks are all-gathered, each rank
+        takes the top k of its own shard (local rows -> global ids, an increasing map, so the tie order holds), the
+        [U, k] lists are all-gathered and merged per user by (score desc, id asc)."""
+        import torch.distributed as dist
+        eng = self.engine
+        rank, world = eng.item_shard
+        dev = eng.device
+        c = self.forward_eval(seq, time_seq, hours, days, timestamps=timestamps)
+        B, T, H = c.B, eng.T, eng.H
+        last = c.seq_emb.view(B, T, H)[:, T - 1, :].contiguous()
+        U = B * world
+        last_all = torch.empty(U, H, dtype=torch.float32, device=dev)
+        dist.all_gather_into_tensor(last_all, last)
+        excl_all = [None] * world
+        dist.all_gather_object(excl_all, None if exclude is None else [sorted(set(int(i) for i in r)) for r in exclude])
+        off = 1 if rank else 0
+        v_loc = (eng.V_items - rank + world - 1) // world + off      # rows of this shard that hold items (+ the pad)
+        ids = torch.zeros(U, k, dtype=torch.int32, device=dev)
+        scores = torch.full((U, k), float("-inf"), dtype=torch.float32, device=dev)
+        if v_loc > 1:
+            eptr = eidx = None
+            if excl_all[0] is not None:
+                eptr, eidx = self._id_csr([r for rl in excl_all for r in rl], U, local_rows=True)
+            rows, scores = self._topk(last_all, H, U, v_loc, k, eptr, eidx, mode)
+            ids = torch.where(rows > 0, (rows - off) * world + rank, rows)
+        parts_i = [torch.empty_like(ids) for _ in range(world)]
+        parts_s = [torch.empty_like(scores) for _ in range(world)]
+        dist.all_gather(parts_i, ids)
+        dist.all_gather(parts_s, scores)
+        all_i = np.concatenate([t.cpu().numpy() for t in parts_i], 1)
+        all_s = np.concatenate([t.cpu().numpy() for t in parts_s], 1)
+        order = np.lexsort((all_i, -all_s), axis=-1)[:, :k]
+        mine = slice(rank * B, (rank + 1) * B)
+        return np.take_along_axis(all_i, order, 1)[mine], np.take_along_axis(all_s, order, 1)[mine]
+
     # ------------------------------------------------------------------ reference protocol
     def _stage_all(self, c, seq, pos, neg, time_seq, hours, days, timestamps):
         self._ts_pending = timestamps if len(self.engine.plan.tables) > 1 else None
@@ -283,16 +375,7 @@ class _Model:
         dev = eng.device
         V = eng.P["item_emb"].shape[0]
         tgt = torch.from_numpy(np.ascontiguousarray(np.asarray(target, dtype=np.int32).reshape(-1))).to(dev)
-        rptr = ridx = None
-        if rated is not None:
-            ptr = np.zeros(B + 1, np.int32)
-            flat = []
-            for u, r in enumerate(rated):
-                ids = np.unique(np.asarray(list(r), dtype=np.int64))
-                flat.append(ids)
-                ptr[u + 1] = ptr[u] + len(ids)
-            idx = np.concatenate(flat + [np.zeros(1, np.int64)]).astype(np.int32)
-            rptr, ridx = torch.from_numpy(ptr).to(dev), torch.from_numpy(idx).to(dev)
+        rptr, ridx = self._id_csr(rated, B) if rated is not None else (None, None)
         cgt = torch.empty(B, dtype=torch.int32, device=dev)
         ceq = torch.empty(B, dtype=torch.int32, device=dev)
         wsb = eng.lib.cast_score_rank_full_workspace_bytes(B, V, H)
@@ -341,18 +424,7 @@ class _Model:
         tl = np.where((tg % world == rank) & (tg > 0) & (tg < eng.V_items), tg // world + off, 0).astype(np.int32)
         rptr = ridx = None
         if rated is not None:
-            ptr = np.zeros(U + 1, np.int32)
-            flat = []
-            u = 0
-            for rl in rated_all:
-                for r in rl:
-                    ids = np.asarray(r, dtype=np.int64)
-                    ids = ids[(ids % world == rank) & (ids > 0) & (ids < eng.V_items)] // world + off
-                    flat.append(ids)
-                    ptr[u + 1] = ptr[u] + len(ids)
-                    u += 1
-            idx = np.concatenate(flat + [np.zeros(1, np.int64)]).astype(np.int32)
-            rptr, ridx = torch.from_numpy(ptr).to(dev), torch.from_numpy(idx).to(dev)
+            rptr, ridx = self._id_csr([r for rl in rated_all for r in rl], U, local_rows=True)
         v_loc = (eng.V_items - rank + world - 1) // world + off      # rows of this shard that hold items (+ the pad)
         cgt = torch.zeros(U, dtype=torch.int32, device=dev)
         ceq = torch.zeros(U, dtype=torch.int32, device=dev)

@@ -387,6 +387,21 @@ int cast_score_rank_full(const float* seq_last, long ld, const float* table, int
 /* Synchronises the stream and reports the tensor-core pass's watchdog flag (0 = ok). */
 int cast_score_rank_full_status(const void* workspace, long U, int V, int* host_flag, void* stream);
 
+/* Exact full-catalog top-K recommendation.  For each user u (row u of seq_last, stride ld >= H): the K rows
+ * j in [1, V) of `table` not in the user's exclusion row, ordered by the canonical logit (the fp32 dot of
+ * cast_score_rank_cand: k ascending, multiply and add rounded separately) descending, then by row ascending;
+ * top_scores are those logits bit for bit.  Fewer than K eligible rows: the tail is (0, -inf).  1 <= K <= 256.
+ * excl_ptr [U+1] / excl_idx (optional CSR): per user, row ids in ascending order; ids outside [1, V) and duplicates
+ * are ignored.  mode 0 = tcgen05 tensor cores as an exact filter (two passes + canonical re-scoring of the admitted
+ * candidates; a user whose candidates overflow the buffer takes the exact path), mode 1 = exact brute force.  Both
+ * modes return the same bits.  stats (optional, [2]): [0] candidates re-scored, [1] users on the exact fallback. */
+size_t cast_topk_full_workspace_bytes(long U, int V, int H, int K);
+int cast_topk_full(const float* seq_last, long ld, const float* table, int V, int H, long U, int K,
+                   const int* excl_ptr, const int* excl_idx, int mode, int* top_ids, float* top_scores,
+                   unsigned long long* stats, void* workspace, size_t workspace_bytes, void* stream);
+/* Synchronises the stream and reports the tensor-core passes' watchdog flag (0 = ok). */
+int cast_topk_full_status(const void* workspace, long U, int V, int H, int K, int* host_flag, void* stream);
+
 #ifdef __cplusplus
 }
 #endif

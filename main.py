@@ -66,7 +66,29 @@ def build_parser():
     p.add_argument("--model_path", default=os.path.abspath("saved_models"))
     p.add_argument("--device_time_features", action="store_true", help="CAST models: the sampler and the evaluation "
                    "hand raw timestamps to the device, which derives time bins / hours / weekdays there")
+    p.add_argument("--recommend", default=0, type=int, help="with --test_model: after the evaluation, write the top K "
+                   "items of every user (whole history excluded) to recommendations_top{K}.npz next to the checkpoint")
     return p
+
+
+def write_recommendations(model, dataset, args, rank, world):
+    """--recommend K: exact top-K of every user from the last maxlen events of train + valid + test, the whole history
+    excluded; users are sharded over the ranks and gathered; rank 0 writes users / items / scores."""
+    from cast_b200 import dist as cdist
+    from cast_b200.evaluation import build_recommend_inputs, recommend_users
+    K = int(args.recommend)
+    rec = build_recommend_inputs(dataset, args)
+    lo, hi = cdist.shard_users(len(rec["u"]), rank, world)
+    ids, scores = recommend_users(model, rec, K, args.eval_batch, lo, hi)
+    if world > 1:
+        import torch.distributed as tdist
+        parts = [None] * world
+        tdist.all_gather_object(parts, (ids, scores))
+        ids = np.concatenate([p[0] for p in parts])
+        scores = np.concatenate([p[1] for p in parts])
+    if rank == 0:
+        np.savez(os.path.join(args.test_model, "recommendations_top{}.npz".format(K)), users=rec["u"], items=ids,
+                 scores=scores)
 
 
 def save_checkpoint(model, args, path):
@@ -177,6 +199,8 @@ def run(args, device=None, lib=None, logger=None):
                     np.save(os.path.join(args.test_model, "avg_attention_weights.npy"), avg_attn)
                     with open(os.path.join(args.test_model, "test_seq_len.txt"), "a") as f:
                         f.write("{},{},{}\n".format(args.test_seq_len, t_test[0], t_test[1]))
+                if getattr(args, "recommend", 0) > 0:
+                    write_recommendations(model, dataset, args, rank, world)
             else:
                 print("{} not found".format(args.test_model))
         finally:
