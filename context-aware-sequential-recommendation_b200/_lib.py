@@ -50,10 +50,7 @@ SIGNATURES = {
     "cast_qkv_bwd_embed": (I, [P, P, P, P, P, P, P, P, P, P, P, P, L, I, P, F, U64, P, I, P, P, P, SZ, P]),
     "cast_colsum_workspace_bytes": (SZ, [L, L]),
     "cast_colsum": (I, [P, L, L, L, P, P, SZ, P]),
-    "cast_attn_set_chunk": (I, [I]),
     "cast_set_pdl": (I, [I]),
-    "cast_attn_set_kg": (I, [I]),
-    "cast_fused_set_backend": (I, [I]),
     "cast_block_bwd_parts": (I, [L, I]),
     "cast_reduce_partials_batch": (I, [I, P, P, P, P, P, P]),
     "cast_layernorm_bwd_parts": (I, [L]),
@@ -136,14 +133,8 @@ def load_library(path: str | None = None) -> C.CDLL:
             f"CUDA extension not found at {p}. Build it with `python -c 'import __graft_entry__ as g; g.build()'` "
             "(nvcc, sm_100a). This package has no CPU / PyTorch fallback.")
     lib = bind(C.CDLL(p))
-    if os.environ.get("CAST_ATTN_CHUNK"):  # tuning hook (32 or 64 columns per streamed attention chunk)
-        check(lib, lib.cast_attn_set_chunk(int(os.environ["CAST_ATTN_CHUNK"])), "cast_attn_set_chunk")
     if os.environ.get("CAST_PDL"):         # A/B hook: 0 = ordinary launches instead of programmatic dependent launch
         check(lib, lib.cast_set_pdl(int(os.environ["CAST_PDL"])), "cast_set_pdl")
-    if os.environ.get("CAST_ATTN_KG"):     # tuning hook (2 or 4 key groups per row block of the attention kernels)
-        check(lib, lib.cast_attn_set_kg(int(os.environ["CAST_ATTN_KG"])), "cast_attn_set_kg")
-    if os.environ.get("CAST_FUSED_BACKEND"):  # A/B hook: 0 = FFMA row kernels, 1 = tensor-core row kernels
-        check(lib, lib.cast_fused_set_backend(int(os.environ["CAST_FUSED_BACKEND"])), "cast_fused_set_backend")
     if path is None:
         _LIB = lib
     return lib

@@ -28,9 +28,6 @@ bool attn_mma_supported(const AttnDims& dm);
 int dispatch_att_mma(int which, const AttnFwdArgs* fa, const AttnBwdArgs* ba, const float* out, const float* resid,
                      float* pbuf, float* dbuf, const AttnDims& dm, cudaStream_t stream);
 
-int attn_mma_set_chunk(int nt);
-int attn_mma_set_kg(int kg);
-
 static int dispatch_by_width(int which, const AttnFwdArgs* fa, const AttnBwdArgs* ba, const AttnDims& dm,
                              cudaStream_t stream) {
   switch (dm.dpad) {
@@ -51,9 +48,6 @@ using namespace cast;
 extern "C" size_t cast_attn_bwd_workspace_bytes(int B, int T, int h) {
   return 2 * (size_t)B * h * T * T * sizeof(float);
 }
-
-extern "C" int cast_attn_set_chunk(int columns) { return attn_mma_set_chunk(columns / 8); }
-extern "C" int cast_attn_set_kg(int key_groups) { return attn_mma_set_kg(key_groups); }
 
 extern "C" int cast_attn_fwd(const float* Q, long ldq, const float* K, long ldk, const float* V, long ldv,
                              const float* queries, const float* kmask, const float* qmask, int B, int T, int H, int h,

@@ -5,9 +5,10 @@
 //   S = Q K^T / sqrt(d);  S = where(key masked | k > q, -2^32+1, S);  P = softmax(S) over all T keys;
 //   P *= query mask;  P = dropout(P);  O = P V + queries.
 //
-// Layout: CTA = 4 warps = 64 rows of one (batch element, head); a warp owns 16 rows and streams 8*NT-column chunks of
-// the other operand through a two-stage cp.async pipeline in shared memory (the next chunk is in flight while the
-// current one is multiplied).  Scores live only in the accumulator fragments: the forward pass keeps a
+// Layout: CTA = 8 warps on 64 rows of one (batch element, head); warps w and w + 4 own the same 16 rows and each
+// takes one 32-column half of every 64-row chunk of the other operand, streamed through a two-stage cp.async pipeline
+// in shared memory (the next chunk is in flight while the current one is multiplied); the two halves' partial results
+// are merged through shared memory at the end.  Scores live only in the accumulator fragments: the forward pass keeps a
 // running row max / row sum (rescaling O when the max moves), and the C fragment of S is fed straight back as the A
 // fragment of P.V by relabelling the contraction index inside each k-step (mma_tf32.cuh), so probabilities never
 // touch shared memory.  Row tiles are aligned to the END of the sequence (sequences are left-padded: the ragged tile
@@ -24,8 +25,9 @@
 
 namespace cast {
 
-constexpr int AM_THREADS = 128;
-constexpr int AM_T = 64;  // rows per CTA (4 warps x 16)
+constexpr int AM_THREADS = 256;  // 8 warps: 4 row blocks of 16 rows x 2 key (or query) groups
+constexpr int AM_T = 64;         // rows per CTA
+constexpr int AM_NT = 4;         // n-tiles of 8 rows a warp takes from each staged 64-row chunk (its half)
 
 // first kept key (kmask != 0) and first query (ids != 0; 0 without ids) of the sequence, T when there is none.
 // One pass, one barrier: strided scan (a thread's first hit is its minimum), warp minimum by shuffles, one slot per
@@ -178,17 +180,16 @@ __device__ __forceinline__ void am_block(const AttnDims& dm, int& b, int& hh, in
 }
 
 // ------------------------------------------------------------------------------------------------ forward
-// KG = 1: 4 warps, each streams whole chunks.  KG = 2: 8 warps; warps w and w+4 own the same 16 rows and split every
-// staged chunk of 16*NT keys in halves (each keeps its own running max / sum / O), merged through shared memory at the
-// end -- the critical path of the late (long) row tiles halves.
-template <int KS, int NT, int KG>
-__global__ void __launch_bounds__(AM_THREADS * KG, (KS <= 7 && NT == 4 && KG <= 2) ? (KG == 1 ? 4 : 2) : 1)
-attn_fwd_mma_kernel(AttnFwdArgs a, AttnDims dm) {
+// Warps w and w+4 own the same 16 rows and split every staged chunk of 64 keys in halves (each keeps its own running
+// max / sum / O), merged through shared memory at the end -- the critical path of the late (long) row tiles halves.
+template <int KS>
+__global__ void __launch_bounds__(AM_THREADS, KS <= 7 ? 2 : 1) attn_fwd_mma_kernel(AttnFwdArgs a, AttnDims dm) {
   cast_pdl_wait();
   // every CTA signals at once: the next kernel of the chain (a row kernel: weights, shared-memory set-up, tensor-memory
   // allocation before its own wait) may take the SMs this grid leaves idle in its long tail (DESIGN.md 4c)
   cast_pdl_trigger();
-  constexpr int DP = 8 * KS, DS = DP + 4, NTO = KS, TW = 8 * NT, TC = TW * KG, NTHR = AM_THREADS * KG, NW = 4 * KG;
+  constexpr int DP = 8 * KS, DS = DP + 4, NTO = KS, NT = AM_NT, TW = 8 * NT, TC = 2 * TW;
+  constexpr int NTHR = AM_THREADS, NW = NTHR / 32;
   CAST_DYN_SMEM(float, sm);
   __shared__ int s_first[AM_FIRST_SLOTS];
   float* Qs = sm;                         // [64][DS]
@@ -258,21 +259,20 @@ attn_fwd_mma_kernel(AttnFwdArgs a, AttnDims dm) {
 #pragma unroll
     for (int c = 0; c < 4; ++c) o[no][c] = 0.f;
 
-  // the residual tile (queries) rides in the stage that is free during the last chunk: rows [0,TC) in the K stage,
-  // rows [TC,64) in the V stage (TC = 32) -- the epilogue then reads it from shared memory
+  // the residual tile (queries) rides in the K stage that is free during the last chunk -- the epilogue then reads it
+  // from shared memory
+  static_assert(TC == AM_T, "a K stage holds the residual tile");
   const float* Rg = a.resid + rowbase * dm.H + hh * d;
   const bool vr = am_vec2_ok(a.resid, dm.H, d, hh);
   const int rst = nch & 1;  // stage not used by the last chunk
-  // KG > 2: the group merge below needs both K stages, so the residual tile goes to the free V stage
-  float* resS = (KG > 2 ? Vst : Kst) + rst * TC * DS;
+  float* resS = Kst + rst * TC * DS;
   for (int ci = 0; ci < nch; ++ci) {
     const int j0s = kbeg + ci * TC, st = ci & 1;
     const int j0 = j0s + kg * TW;  // this warp's part of the staged chunk
     if (ci + 1 < nch) {
       issue(j0s + TC, st ^ 1);
     } else {
-      am_load_rows_async<(TC < AM_T ? TC : AM_T), DS, NW>(resS, Rg, dm.H, q0, T, d, vr);
-      if (TC < AM_T) am_load_rows_async<TC, DS, NW>(Vst + rst * TC * DS, Rg, dm.H, q0 + TC, T, d, vr);
+      am_load_rows_async<AM_T, DS, NW>(resS, Rg, dm.H, q0, T, d, vr);
       cp_async_commit();
     }
     cp_async_wait<1>();
@@ -343,11 +343,12 @@ attn_fwd_mma_kernel(AttnFwdArgs a, AttnDims dm) {
   __syncthreads();
   lA = quad_sum(lA);
   lB = quad_sum(lB);
-  if (KG > 1) {  // fold the other key groups' (max, sum, O) into the first, in group order, through free stages
-    // KG == 2: the K / V stage the last chunk used; KG > 2: both K stages / the V stage the last chunk used
-    float* mo = KG > 2 ? Kst : Kst + ((nch - 1) & 1) * TC * DS;  // [KG - 1][128 threads][4 * NTO]
-    float* ml = Vst + ((nch - 1) & 1) * TC * DS;                  // [KG - 1][128 threads][4]
-    static_assert((KG - 1) * 128 * 4 * NTO <= (KG > 2 ? 2 : 1) * TC * DS && (KG - 1) * 128 * 4 <= TC * DS, "merge space");
+  {  // fold the second key group's (max, sum, O) into the first through the K / V stage the last chunk used
+    // (kg - 1 == 0 here and the V-stage arm of rrow below is never taken; written this way they keep the register
+    // allocation this kernel was measured with; the plain forms move it by up to 5 registers and 32 instructions)
+    float* mo = Kst + ((nch - 1) & 1) * TC * DS;  // [128 threads][4 * NTO]
+    float* ml = Vst + ((nch - 1) & 1) * TC * DS;  // [128 threads][4]
+    static_assert(128 * 4 * NTO <= TC * DS && 128 * 4 <= TC * DS, "merge space");
     const int slot = warp * 32 + lane;
     if (kg > 0) {
       float* mog = mo + (kg - 1) * 128 * 4 * NTO;
@@ -358,26 +359,22 @@ attn_fwd_mma_kernel(AttnFwdArgs a, AttnDims dm) {
     }
     __syncthreads();
     if (kg > 0) return;
+    const float4 st1 = *reinterpret_cast<const float4*>(ml + slot * 4);
+    const float nmA = fmaxf(mA, st1.x), nmB = fmaxf(mB, st1.y);
+    // a group that saw no chunk has max = -inf, sum = 0: its factor is exp(-inf) = 0 (nm is finite for live rows)
+    const float a0A = nmA == -INFINITY ? 0.f : __expf(mA - nmA), a1A = nmA == -INFINITY ? 0.f : __expf(st1.x - nmA);
+    const float a0B = nmB == -INFINITY ? 0.f : __expf(mB - nmB), a1B = nmB == -INFINITY ? 0.f : __expf(st1.y - nmB);
+    lA = lA * a0A + st1.z * a1A;
+    lB = lB * a0B + st1.w * a1B;
+    mA = nmA;
+    mB = nmB;
 #pragma unroll
-    for (int gi = 1; gi < KG; ++gi) {
-      const float* mog = mo + (gi - 1) * 128 * 4 * NTO;
-      const float4 st1 = *reinterpret_cast<const float4*>(ml + ((gi - 1) * 128 + slot) * 4);
-      const float nmA = fmaxf(mA, st1.x), nmB = fmaxf(mB, st1.y);
-      // a group that saw no chunk has max = -inf, sum = 0: its factor is exp(-inf) = 0 (nm is finite for live rows)
-      const float a0A = nmA == -INFINITY ? 0.f : __expf(mA - nmA), a1A = nmA == -INFINITY ? 0.f : __expf(st1.x - nmA);
-      const float a0B = nmB == -INFINITY ? 0.f : __expf(mB - nmB), a1B = nmB == -INFINITY ? 0.f : __expf(st1.y - nmB);
-      lA = lA * a0A + st1.z * a1A;
-      lB = lB * a0B + st1.w * a1B;
-      mA = nmA;
-      mB = nmB;
-#pragma unroll
-      for (int no = 0; no < NTO; ++no) {
-        const float4 o1 = *reinterpret_cast<const float4*>(mog + (slot * NTO + no) * 4);
-        o[no][0] = o[no][0] * a0A + o1.x * a1A;
-        o[no][1] = o[no][1] * a0A + o1.y * a1A;
-        o[no][2] = o[no][2] * a0B + o1.z * a1B;
-        o[no][3] = o[no][3] * a0B + o1.w * a1B;
-      }
+    for (int no = 0; no < NTO; ++no) {
+      const float4 o1 = *reinterpret_cast<const float4*>(mo + (slot * NTO + no) * 4);
+      o[no][0] = o[no][0] * a0A + o1.x * a1A;
+      o[no][1] = o[no][1] * a0A + o1.y * a1A;
+      o[no][2] = o[no][2] * a0B + o1.z * a1B;
+      o[no][3] = o[no][3] * a0B + o1.w * a1B;
     }
   }
 #pragma unroll
@@ -422,9 +419,10 @@ struct AttnBwdMmaArgs {
 
 // ST: also store P~ and dS of every computed score to aa.pbuf / aa.dbuf (then fully-masked "uniform" rows, whose P~
 // reaches all T keys, are walked over the whole key range like in the forward pass)
-template <int KS, int NT, int KG, bool ST>
-__global__ void __launch_bounds__(AM_THREADS * KG, (KS <= 7 && NT == 4 && KG == 2) ? 2 : 1) attn_bwd_dq_mma_kernel(AttnBwdMmaArgs aa, AttnDims dm) {
-  constexpr int DP = 8 * KS, DS = DP + 4, NTO = KS, TW = 8 * NT, TC = TW * KG, NTHR = AM_THREADS * KG, NW = 4 * KG;
+template <int KS, bool ST>
+__global__ void __launch_bounds__(AM_THREADS, KS <= 7 ? 2 : 1) attn_bwd_dq_mma_kernel(AttnBwdMmaArgs aa, AttnDims dm) {
+  constexpr int DP = 8 * KS, DS = DP + 4, NTO = KS, NT = AM_NT, TW = 8 * NT, TC = 2 * TW;
+  constexpr int NTHR = AM_THREADS, NW = NTHR / 32;
   const AttnBwdArgs& a = aa.b;
   CAST_DYN_SMEM(float, sm);
   __shared__ int s_first[AM_FIRST_SLOTS];
@@ -447,15 +445,13 @@ __global__ void __launch_bounds__(AM_THREADS * KG, (KS <= 7 && NT == 4 && KG == 
   // Of this kernel's inputs only dO is produced by the kernel before it in the chain (the FFN backward kernel): the
   // query tile, out / queries, the sequence scan and the first K/V chunk are requested before the wait on that kernel.
   am_load_rows_async<AM_T, DS, NW>(Qs, a.Q + rowbase * a.ldq + hh * d, a.ldq, q0, T, d, am_vec2_ok(a.Q, a.ldq, d, hh));
-  constexpr bool PARK = TC >= AM_T;   // a K/V stage holds a whole row tile (the 8-warp configuration)
+  static_assert(TC == AM_T, "a K/V stage holds a whole row tile");
   float* outS = Kst + TC * DS;
   float* resS = Vst + TC * DS;
-  if (PARK) {
-    am_load_rows_async<AM_T, DS, NW>(outS, aa.out + rowbase * dm.H + hh * d, dm.H, q0, T, d,
-                                     am_vec2_ok(aa.out, dm.H, d, hh));
-    am_load_rows_async<AM_T, DS, NW>(resS, aa.resid + rowbase * dm.H + hh * d, dm.H, q0, T, d,
-                                     am_vec2_ok(aa.resid, dm.H, d, hh));
-  }
+  am_load_rows_async<AM_T, DS, NW>(outS, aa.out + rowbase * dm.H + hh * d, dm.H, q0, T, d,
+                                   am_vec2_ok(aa.out, dm.H, d, hh));
+  am_load_rows_async<AM_T, DS, NW>(resS, aa.resid + rowbase * dm.H + hh * d, dm.H, q0, T, d,
+                                   am_vec2_ok(aa.resid, dm.H, d, hh));
   cp_async_commit();
   int first_key, qstart;
   am_first2(a.kmask + rowbase, a.skip_ids ? a.skip_ids + rowbase : nullptr, T, s_first, first_key, qstart);
@@ -514,12 +510,7 @@ __global__ void __launch_bounds__(AM_THREADS * KG, (KS <= 7 && NT == 4 && KG == 
         for (int u = 0; u < 2; ++u) {
           const int c = lane + 32 * u;
           if (c >= d) continue;
-          if (PARK) {
-            acc = fmaf(dOs[r * DS + c], outS[r * DS + c] - resS[r * DS + c], acc);
-          } else {
-            const long off = (rowbase + i) * dm.H + hh * d + c;
-            acc = fmaf(dOs[r * DS + c], aa.out[off] - aa.resid[off], acc);
-          }
+          acc = fmaf(dOs[r * DS + c], outS[r * DS + c] - resS[r * DS + c], acc);
         }
       }
       const float v = warp_sum(acc);
@@ -620,27 +611,22 @@ __global__ void __launch_bounds__(AM_THREADS * KG, (KS <= 7 && NT == 4 && KG == 
     __syncthreads();
   }
   cp_async_wait<0>();
-  if (KG > 1) {  // dQ = sum of the key groups' partial products, in group order
+  {  // dQ = sum of the two key groups' partial products
     __syncthreads();
-    float* mo = Kst;  // [KG - 1][128 threads][4 * NTO] (both K stages are free now)
-    static_assert((KG - 1) * 128 * 4 * NTO <= 2 * TC * DS, "merge space");
+    float* mo = Kst;  // [128 threads][4 * NTO] (both K stages are free now)
+    static_assert(128 * 4 * NTO <= 2 * TC * DS, "merge space");
     const int slot = warp * 32 + lane;
     if (kg > 0) {
-      float* mog = mo + (kg - 1) * 128 * 4 * NTO;
 #pragma unroll
       for (int no = 0; no < NTO; ++no)
-        *reinterpret_cast<float4*>(mog + (slot * NTO + no) * 4) = make_float4(o[no][0], o[no][1], o[no][2], o[no][3]);
+        *reinterpret_cast<float4*>(mo + (slot * NTO + no) * 4) = make_float4(o[no][0], o[no][1], o[no][2], o[no][3]);
     }
     __syncthreads();
     if (kg > 0) return;
 #pragma unroll
-    for (int gi = 1; gi < KG; ++gi) {
-      const float* mog = mo + (gi - 1) * 128 * 4 * NTO;
-#pragma unroll
-      for (int no = 0; no < NTO; ++no) {
-        const float4 o1 = *reinterpret_cast<const float4*>(mog + (slot * NTO + no) * 4);
-        o[no][0] += o1.x; o[no][1] += o1.y; o[no][2] += o1.z; o[no][3] += o1.w;
-      }
+    for (int no = 0; no < NTO; ++no) {
+      const float4 o1 = *reinterpret_cast<const float4*>(mo + (slot * NTO + no) * 4);
+      o[no][0] += o1.x; o[no][1] += o1.y; o[no][2] += o1.z; o[no][3] += o1.w;
     }
   }
 #pragma unroll
@@ -666,10 +652,11 @@ __global__ void __launch_bounds__(AM_THREADS * KG, (KS <= 7 && NT == 4 && KG == 
 }
 
 // ------------------------------------------------------------------------------------------------ backward: dK, dV
-template <int KS, int NT, int KG>
-__global__ void __launch_bounds__(AM_THREADS * KG, (KS <= 7 && NT == 4 && KG == 2) ? 2 : 1) attn_bwd_dkv_mma_kernel(AttnBwdMmaArgs aa, AttnDims dm) {
+template <int KS>
+__global__ void __launch_bounds__(AM_THREADS, KS <= 7 ? 2 : 1) attn_bwd_dkv_mma_kernel(AttnBwdMmaArgs aa, AttnDims dm) {
   cast_pdl_wait();
-  constexpr int DP = 8 * KS, DS = DP + 4, NTO = KS, TW = 8 * NT, TC = TW * KG, NTHR = AM_THREADS * KG, NW = 4 * KG;
+  constexpr int DP = 8 * KS, DS = DP + 4, NTO = KS, NT = AM_NT, TW = 8 * NT, TC = 2 * TW;
+  constexpr int NTHR = AM_THREADS, NW = NTHR / 32;
   const AttnBwdArgs& a = aa.b;
   CAST_DYN_SMEM(float, sm);
   __shared__ int s_first[AM_FIRST_SLOTS];
@@ -806,7 +793,7 @@ __global__ void __launch_bounds__(AM_THREADS * KG, (KS <= 7 && NT == 4 && KG == 
     cc = cn;
   }
   cp_async_wait<0>();
-  if (KG == 2) {  // dK, dV = sums of the two query groups' partial products
+  {  // dK, dV = sums of the two query groups' partial products
     __syncthreads();
     float* mk = Qst;   // [128 threads][4 * NTO]
     float* mv = dOst;
@@ -1069,70 +1056,40 @@ __global__ void __launch_bounds__(AW_THREADS, 2) attn_bwd_dkv_ws_kernel(AttnBwdM
 }
 
 // ------------------------------------------------------------------------------------------------ dispatch
-static int g_attn_kg = 2;   // key groups per row block in the 8 x NT = 32 configuration (A/B hook: cast_attn_set_kg)
-
-template <int KS, int NT>
+template <int KS>
 static int launch_mma(int which, const AttnFwdArgs* fa, const AttnBwdMmaArgs* ba, const AttnDims& dm,
                       cudaStream_t stream) {
-  constexpr int DS = 8 * KS + 4, TC = 8 * NT;
+  constexpr int DS = 8 * KS + 4, TC = 2 * 8 * AM_NT;  // TC: rows of a staged chunk (both key groups)
   static size_t cfg[3] = {48 * 1024, 48 * 1024, 48 * 1024};
   const int ntile = (int)cdiv(dm.T, AM_T);
   const dim3 grid((unsigned)(dm.B * dm.h), (unsigned)ntile);
   const size_t row = sizeof(float) * DS;
   if (which == 0) {
-    if (NT == 4 && g_attn_kg == 4) {  // 16 warps, one CTA per SM: four key groups per row block
-      constexpr int KG4 = (NT == 4) ? 4 : 1, TC4 = TC * KG4;
-      static size_t cfg4 = 48 * 1024;
-      const size_t smem = (AM_T + 4 * TC4) * row + sizeof(float) * 2 * TC4;
-      auto kf = attn_fwd_mma_kernel<KS, NT, KG4>;
-      if (smem > cfg4) {
-        cudaFuncSetAttribute(kf, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-        cfg4 = smem;
-      }
-      CAST_LAUNCH_DEP(kf, grid, dim3(AM_THREADS * KG4), smem, stream, *fa, dm);
-      return CAST_OK;
-    }
-    constexpr int KGF = (NT == 4) ? 2 : 1;  // 8 warps: two key groups per row block
-    constexpr int TCF = TC * KGF;
-    const size_t smem = (AM_T + 4 * TCF) * row + sizeof(float) * 2 * TCF;
-    auto kf = attn_fwd_mma_kernel<KS, NT, KGF>;
+    const size_t smem = (AM_T + 4 * TC) * row + sizeof(float) * 2 * TC;
+    auto kf = attn_fwd_mma_kernel<KS>;
     if (smem > cfg[0]) {
       cudaFuncSetAttribute(kf, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
       cfg[0] = smem;
     }
-    CAST_LAUNCH_DEP(kf, grid, dim3(AM_THREADS * KGF), smem, stream, *fa, dm);
+    CAST_LAUNCH_DEP(kf, grid, dim3(AM_THREADS), smem, stream, *fa, dm);
   } else if (which == 1) {
-    if (NT == 4 && g_attn_kg == 4 && ba->pbuf) {
-      constexpr int KG4 = (NT == 4) ? 4 : 1, TC4 = TC * KG4;
-      static size_t cfg4 = 48 * 1024;
-      const size_t smem = (2 * AM_T + 4 * TC4) * row + sizeof(float) * (2 * TC4 + AM_T);
-      auto kf = attn_bwd_dq_mma_kernel<KS, NT, KG4, true>;
-      if (smem > cfg4) {
-        cudaFuncSetAttribute(kf, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-        cfg4 = smem;
-      }
-      CAST_LAUNCH_DEP(kf, grid, dim3(AM_THREADS * KG4), smem, stream, *ba, dm);
-      return CAST_OK;
-    }
-    constexpr int KGB = (NT == 4) ? 2 : 1;
-    constexpr int TCB = TC * KGB;
-    const size_t smem = (2 * AM_T + 4 * TCB) * row + sizeof(float) * (2 * TCB + AM_T);
+    const size_t smem = (2 * AM_T + 4 * TC) * row + sizeof(float) * (2 * TC + AM_T);
     if (ba->pbuf) {
       static size_t cfgs = 48 * 1024;
-      auto kf = attn_bwd_dq_mma_kernel<KS, NT, KGB, true>;
+      auto kf = attn_bwd_dq_mma_kernel<KS, true>;
       if (smem > cfgs) {
         cudaFuncSetAttribute(kf, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
         cfgs = smem;
       }
-      CAST_LAUNCH_DEP(kf, grid, dim3(AM_THREADS * KGB), smem, stream, *ba, dm);
+      CAST_LAUNCH_DEP(kf, grid, dim3(AM_THREADS), smem, stream, *ba, dm);
       return CAST_OK;
     }
-    auto kf = attn_bwd_dq_mma_kernel<KS, NT, KGB, false>;
+    auto kf = attn_bwd_dq_mma_kernel<KS, false>;
     if (smem > cfg[1]) {
       cudaFuncSetAttribute(kf, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
       cfg[1] = smem;
     }
-    CAST_LAUNCH_DEP(kf, grid, dim3(AM_THREADS * KGB), smem, stream, *ba, dm);
+    CAST_LAUNCH_DEP(kf, grid, dim3(AM_THREADS), smem, stream, *ba, dm);
   } else {
     if (ba->pbuf) {
       static size_t cfgw = 48 * 1024;
@@ -1145,52 +1102,28 @@ static int launch_mma(int which, const AttnFwdArgs* fa, const AttnBwdMmaArgs* ba
       CAST_LAUNCH_DEP(kw, grid, dim3(AW_THREADS), smemw, stream, *ba, dm);
       return CAST_OK;
     }
-    constexpr int KGB = (NT == 4) ? 2 : 1;
-    constexpr int TCB = TC * KGB;
-    const size_t smem = (2 * AM_T + 4 * TCB) * row + sizeof(float) * 8 * TCB;
-    auto kf = attn_bwd_dkv_mma_kernel<KS, NT, KGB>;
+    const size_t smem = (2 * AM_T + 4 * TC) * row + sizeof(float) * 8 * TC;
+    auto kf = attn_bwd_dkv_mma_kernel<KS>;
     if (smem > cfg[2]) {
       cudaFuncSetAttribute(kf, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
       cfg[2] = smem;
     }
-    CAST_LAUNCH_DEP(kf, grid, dim3(AM_THREADS * KGB), smem, stream, *ba, dm);
+    CAST_LAUNCH_DEP(kf, grid, dim3(AM_THREADS), smem, stream, *ba, dm);
   }
   return CAST_OK;
 }
 
 bool attn_mma_supported(const AttnDims& dm) { return dm.d >= 1 && dm.d <= 64 && (long)dm.B * dm.h < 2147483647L; }
 
-int attn_mma_set_kg(int kg) {
-  if (kg != 2 && kg != 4) return set_error(CAST_ERR_BAD_ARG, "attention (mma): key groups must be 2 or 4");
-  g_attn_kg = kg;
-  return CAST_OK;
-}
-
-static int g_chunk_tiles = 4;  // columns per streamed chunk / 8 (4 or 8); cast_attn_set_chunk (tuning hook)
-int attn_mma_set_chunk(int nt) {
-  if (nt != 4 && nt != 8) return set_error(CAST_ERR_BAD_ARG, "attention (mma): chunk must be 32 or 64 columns");
-  g_chunk_tiles = nt;
-  return CAST_OK;
-}
-
 // which: 0 = forward (fa), 1 = backward dQ, 2 = backward dK/dV (ba + out/resid)
 int dispatch_att_mma(int which, const AttnFwdArgs* fa, const AttnBwdArgs* ba, const float* out, const float* resid,
                      float* pbuf, float* dbuf, const AttnDims& dm, cudaStream_t stream) {
   AttnBwdMmaArgs bm{};
   if (ba) { bm.b = *ba; bm.out = out; bm.resid = resid; bm.pbuf = pbuf; bm.dbuf = dbuf; }
-  const int ks = (dm.d + 7) / 8;
-  if (g_chunk_tiles == 8) {
-    switch (ks) {
-#define CAST_K(K) case K: return launch_mma<K, 8>(which, fa, &bm, dm, stream);
-      CAST_K(1) CAST_K(2) CAST_K(3) CAST_K(4) CAST_K(5) CAST_K(6) CAST_K(7) CAST_K(8)
+  switch ((dm.d + 7) / 8) {
+#define CAST_K(K) case K: return launch_mma<K>(which, fa, &bm, dm, stream);
+    CAST_K(1) CAST_K(2) CAST_K(3) CAST_K(4) CAST_K(5) CAST_K(6) CAST_K(7) CAST_K(8)
 #undef CAST_K
-    }
-  } else {
-    switch (ks) {
-#define CAST_K(K) case K: return launch_mma<K, 4>(which, fa, &bm, dm, stream);
-      CAST_K(1) CAST_K(2) CAST_K(3) CAST_K(4) CAST_K(5) CAST_K(6) CAST_K(7) CAST_K(8)
-#undef CAST_K
-    }
   }
   return set_error(CAST_ERR_UNSUPPORTED, "attention (mma): head width > 64");
 }

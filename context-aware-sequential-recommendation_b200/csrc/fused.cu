@@ -3,16 +3,15 @@
 //   ln_ffn_fwd : LN(y) -> relu(.W1+b1) -> dropout -> .W2+b2 -> dropout -> + LN(y) -> *mask (sasrec.py:81-83, modules.py:298-313)
 //   ffn_bwd    : backward of ln_ffn_fwd incl. dW1, dW2, db1, db2, dgamma, dbeta
 //   qkv_bwd    : backward of ln_qkv_fwd incl. dWq, dWk, dWv, biases, dgamma, dbeta (and the attention residual)
-// One CTA = 64 rows x all H columns; 256 threads as a 16x16 grid, 4x4 register micro-tiles, operands in shared
-// memory (pv_tile: C[64 x H] += A[64 x K] * W[K x H], both LDS.128).  The whole weight matrix (H*H*4 <= 16 KB) sits in
-// shared memory; activations make exactly one HBM round trip per kernel instead of one per op.  Backward kernels
-// are persistent (<= 2 CTAs per SM loop over row tiles) and keep their weight-gradient partials in registers; a fixed-
-// order second stage sums the per-CTA partials straight into the flat gradient buffer => deterministic.
+// One CTA works on 64-row tiles with all H columns; the kernels themselves (fused_mma.cuh) contract on the tensor cores
+// (mma.sync 3xTF32).  The whole weight matrix (H*H*4 <= 16 KB) sits in shared memory; activations make exactly one HBM
+// round trip per kernel instead of one per op.  Backward kernels are persistent (one CTA per SM loops over row tiles)
+// and keep their weight-gradient partials in registers; a fixed-order second stage sums the per-CTA partials straight
+// into the flat gradient buffer => deterministic.
 // Gradient layout contract (flat, contiguous, see engine.param_shapes):
 //   qkv_bwd -> [ln1.beta H | ln1.gamma H | q.w H*H | q.b H | k.w H*H | k.b H | v.w H*H | v.b H]
 //   ffn_bwd -> [ln2.beta H | ln2.gamma H | ffn1.w H*H | ffn1.b H | ffn2.w H*H | ffn2.b H]
 #include "cast_rt.cuh"
-#include "tile_ops.cuh"
 
 namespace cast {
 
@@ -21,7 +20,6 @@ int launch_reduce_partials(const float* partial, int nparts, long count, float* 
 
 constexpr int FR = 64;        // rows per tile
 constexpr int FT = 256;       // threads
-constexpr int FTS = FR + 8;   // stride of transposed tiles ([col][row]); 72 => conflict-free 8x4 transposing stores
 
 struct FDims {
   long N;
@@ -35,49 +33,6 @@ static FDims fdims(long N, int H) {
   d.HP4 = (H + 3) & ~3;
   d.HS = (d.HP4 % 32 == 0) ? d.HP4 + 4 : d.HP4;
   return d;
-}
-
-// row-major tile: dst[r][c] = src[(row0+r)*H + c] (zero outside N rows / H cols, cols padded to HP4)
-__device__ __forceinline__ void f_load_rows(float* __restrict__ dst, const float* __restrict__ src, long row0,
-                                            const FDims& d) {
-  const int lane = threadIdx.x & 31;
-  for (int r = threadIdx.x >> 5; r < FR; r += FT / 32) {
-    const long row = row0 + r;
-    const bool ok = row < d.N;
-    const float* s = src + row * d.H;
-    for (int c = lane; c < d.HP4; c += 32) dst[r * d.HS + c] = (ok && c < d.H) ? s[c] : 0.f;
-  }
-}
-
-// transposed tile: dst[c][r] = src[(row0+r)*H + c]; lanes cover 8 rows x 4 cols so stores hit 32 distinct banks
-__device__ __forceinline__ void f_load_rows_T(float* __restrict__ dst, const float* __restrict__ src, long row0,
-                                              const FDims& d) {
-  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-  const int rl = lane & 7, cl = lane >> 3;
-  for (int rb = warp * 8; rb < FR; rb += (FT / 32) * 8) {
-    const int r = rb + rl;
-    const long row = row0 + r;
-    const bool ok = row < d.N;
-    for (int c = cl; c < d.HP4; c += 4) dst[c * FTS + r] = (ok && c < d.H) ? src[row * d.H + c] : 0.f;
-  }
-}
-
-// weight matrix W[K=H][N=H] row-major -> Ws[k][n] (stride HS), zero padded to HP4 x HP4
-__device__ __forceinline__ void f_load_w(float* __restrict__ Ws, const float* __restrict__ W, const FDims& d) {
-  const int lane = threadIdx.x & 31;
-  for (int k = threadIdx.x >> 5; k < d.HP4; k += FT / 32)
-    for (int n = lane; n < d.HP4; n += 32) Ws[k * d.HS + n] = (k < d.H && n < d.H) ? W[k * d.H + n] : 0.f;
-}
-
-// transposed weight: Wt[n][k] = W[k][n]  (operand of dX = dY * W^T)
-__device__ __forceinline__ void f_load_w_T(float* __restrict__ Wt, const float* __restrict__ W, const FDims& d) {
-  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-  const int kl = lane & 7, nl = lane >> 3;
-  for (int kb = warp * 8; kb < d.HP4; kb += (FT / 32) * 8) {
-    const int k = kb + kl;
-    for (int n = nl; n < d.HP4; n += 4)
-      if (k < d.HP4) Wt[n * d.HS + k] = (k < d.H && n < d.H) ? W[k * d.H + n] : 0.f;
-  }
 }
 
 // LN of the rows of Xs (row-major smem tile) -> Ns (smem) and optionally global y / stats / zero-sum flags
@@ -119,52 +74,14 @@ __device__ __forceinline__ void f_layernorm_rows(const float* __restrict__ Xs, f
   }
 }
 
-__device__ __forceinline__ void zero_acc(float (&acc)[4][4]) {
-#pragma unroll
-  for (int i = 0; i < 4; ++i)
-#pragma unroll
-    for (int j = 0; j < 4; ++j) acc[i][j] = 0.f;
-}
-
 // ---------------------------------------------------------------------------------------------------------
+// kernel arguments (the kernels are in fused_mma.cuh)
 struct LnQkvArgs {
   const float *x, *gamma, *beta, *W[3], *b[3];
   float eps;
   float *qn, *out[3], *mean, *rstd, *kmask, *qmask;
 };
 
-__global__ void __launch_bounds__(FT) ln_qkv_fwd_kernel(LnQkvArgs a, FDims d) {
-  CAST_DYN_SMEM(float, sm);
-  float* Xs = sm;
-  float* Ns = Xs + FR * d.HS;
-  float* Ws = Ns + FR * d.HS;
-  const int t = threadIdx.x, tx = t & 15, ty = t >> 4;
-  const long row0 = (long)blockIdx.x * FR;
-  f_load_rows(Xs, a.x, row0, d);
-  __syncthreads();
-  f_layernorm_rows(Xs, Ns, a.gamma, a.beta, a.eps, row0, d, a.qn, a.mean, a.rstd, a.kmask, a.qmask);
-  const int col = tx * 4;
-  for (int m = 0; m < 3; ++m) {
-    __syncthreads();
-    f_load_w(Ws, a.W[m], d);
-    __syncthreads();
-    if (col < d.HP4) {
-      float acc[4][4];
-      zero_acc(acc);
-      pv_tile<4, 0>(m == 0 ? Ns : Xs, d.HS, Ws, d.HS, d.HP4, col, acc, ty);
-#pragma unroll
-      for (int ii = 0; ii < 4; ++ii) {
-        const long row = row0 + ty * 4 + ii;
-        if (row >= d.N) continue;
-#pragma unroll
-        for (int cc = 0; cc < 4; ++cc)
-          if (col + cc < d.H) a.out[m][row * d.H + col + cc] = acc[ii][cc] + a.b[m][col + cc];
-      }
-    }
-  }
-}
-
-// ---------------------------------------------------------------------------------------------------------
 struct LnFfnArgs {
   const float *y, *gamma, *beta, *W1, *b1, *W2, *b2;
   const int* ids;
@@ -175,74 +92,7 @@ struct LnFfnArgs {
   float *zn, *h1d, *xout, *mean, *rstd;
 };
 
-__global__ void __launch_bounds__(FT) ln_ffn_fwd_kernel(LnFfnArgs a, FDims d) {
-  CAST_DYN_SMEM(float, sm);
-  float* Ys = sm;  // y tile, later the hidden activation
-  float* Ns = Ys + FR * d.HS;
-  float* Ws = Ns + FR * d.HS;
-  const int t = threadIdx.x, tx = t & 15, ty = t >> 4;
-  const long row0 = (long)blockIdx.x * FR;
-  const int col = tx * 4;
-  f_load_rows(Ys, a.y, row0, d);
-  f_load_w(Ws, a.W1, d);
-  __syncthreads();
-  f_layernorm_rows(Ys, Ns, a.gamma, a.beta, a.eps, row0, d, a.zn, a.mean, a.rstd, nullptr, nullptr);
-  __syncthreads();
-  const Drop dh = make_drop(a.rate, a.seed, a.step, a.site_h);
-  const Drop dout = make_drop(a.rate, a.seed, a.step, a.site_o);
-  float acc[4][4];
-  zero_acc(acc);
-  if (col < d.HP4) pv_tile<4, 0>(Ns, d.HS, Ws, d.HS, d.HP4, col, acc, ty);
-  __syncthreads();  // everybody is done with Ws (W1) and with Ys (LN input)
-  if (col < d.HP4) {
-#pragma unroll
-    for (int ii = 0; ii < 4; ++ii) {
-      const int r = ty * 4 + ii;
-      const long row = row0 + r;
-#pragma unroll
-      for (int cc = 0; cc < 4; ++cc) {
-        const int c = col + cc;
-        float h = 0.f;
-        if (c < d.H && row < d.N) {
-          h = fmaxf(acc[ii][cc] + a.b1[c], 0.f) * drop_mul(dh, (unsigned long long)(row * d.H + c));
-          a.h1d[row * d.H + c] = h;
-        }
-        Ys[r * d.HS + c] = h;
-      }
-    }
-  }
-  f_load_w(Ws, a.W2, d);
-  __syncthreads();
-  if (col < d.HP4) {
-    zero_acc(acc);
-    pv_tile<4, 0>(Ys, d.HS, Ws, d.HS, d.HP4, col, acc, ty);
-#pragma unroll
-    for (int ii = 0; ii < 4; ++ii) {
-      const int r = ty * 4 + ii;
-      const long row = row0 + r;
-      if (row >= d.N) continue;
-      const float m = a.ids ? (a.ids[row] != 0 ? 1.f : 0.f) : 1.f;
-#pragma unroll
-      for (int cc = 0; cc < 4; ++cc) {
-        const int c = col + cc;
-        if (c < d.H) {
-          float o = (acc[ii][cc] + a.b2[c]) * drop_mul(dout, (unsigned long long)(row * d.H + c));
-          o += Ns[r * d.HS + c];
-          a.xout[row * d.H + c] = o * m;
-        }
-      }
-    }
-  }
-}
-
-// ---------------------------------------------------------------------------------------------------------
-// shared epilogue of the backward kernels: LayerNorm backward of the rows in Gs (gradient w.r.t. LN output) given the
-// LN input tile Xr (row-major) and saved stats; writes dx (+ optional add tile) to global, accumulates dgamma/dbeta.
-struct LnBwdOut {
-  float dgamma, dbeta;  // column owned by thread (tid % 64) for tid < 128: tid/64 == 0 -> dgamma, == 1 -> dbeta
-};
-
-// Optional last step on the dx rows this helper writes: the gradient of `dropout(emb) * mask` at the tower input
+// Optional last step on the dx rows the LayerNorm backward writes: the gradient of `dropout(emb) * mask` at the tower input
 // (sasrec.py:58-62), so that block 0's backward kernel emits the embedding gradient directly.
 struct LnOutFx {
   const int* ids;  // row mask (ids[row] == 0 => 0), may be null
@@ -258,99 +108,6 @@ __device__ __forceinline__ LnOutFx ln_out_none() {
   return f;
 }
 
-template <int NWARP = FT / 32, bool COLS = true>
-__device__ __forceinline__ void f_ln_bwd_rows(const float* __restrict__ Gs, const float* __restrict__ Xr, int sxr,
-                                              int sxc, const float* __restrict__ Add,
-                                              const float* __restrict__ gamma,
-                                              const float* __restrict__ mean, const float* __restrict__ rstd,
-                                              float* __restrict__ rowstat /* smem [FR][4] */, long row0,
-                                              const FDims& d, float* __restrict__ dx, float& dgamma_acc,
-                                              float& dbeta_acc, const LnOutFx fx = ln_out_none()) {
-  const int t = threadIdx.x;
-  // (a) per-row scalars: one warp per row
-  {
-    const int lane = t & 31;
-    const int c0 = lane, c1 = lane + 32;
-    const float g0 = c0 < d.H ? gamma[c0] : 0.f, g1 = c1 < d.H ? gamma[c1] : 0.f;
-    for (int r = t >> 5; r < FR; r += NWARP) {
-      const long row = row0 + r;
-      float mu = 0.f, rs = 0.f;
-      if (row < d.N) { mu = mean[row]; rs = rstd[row]; }
-      const float x0 = c0 < d.H ? (Xr[r * sxr + c0 * sxc] - mu) * rs : 0.f;
-      const float x1 = c1 < d.H ? (Xr[r * sxr + c1 * sxc] - mu) * rs : 0.f;
-      const float a0 = c0 < d.H ? Gs[r * d.HS + c0] * g0 : 0.f;
-      const float a1 = c1 < d.H ? Gs[r * d.HS + c1] * g1 : 0.f;
-      const float s1 = warp_sum(a0 + a1) / (float)d.H;
-      const float s2 = warp_sum(a0 * x0 + a1 * x1) / (float)d.H;
-      if (lane == 0) {
-        rowstat[r * 4 + 0] = mu;
-        rowstat[r * 4 + 1] = rs;
-        rowstat[r * 4 + 2] = s1;
-        rowstat[r * 4 + 3] = s2;
-      }
-      if (row < d.N) {
-        const float fm = (fx.on && fx.ids && fx.ids[row] == 0) ? 0.f : 1.f;
-        if (c0 < d.H) {
-          float o = rs * (a0 - s1 - x0 * s2);
-          if (Add) o += Add[r * d.HS + c0];
-          if (fx.on) o = o * fm * drop_mul(fx.drop, (unsigned long long)(row * d.H + c0));
-          dx[row * d.H + c0] = o;
-        }
-        if (c1 < d.H) {
-          float o = rs * (a1 - s1 - x1 * s2);
-          if (Add) o += Add[r * d.HS + c1];
-          if (fx.on) o = o * fm * drop_mul(fx.drop, (unsigned long long)(row * d.H + c1));
-          dx[row * d.H + c1] = o;
-        }
-      }
-    }
-  }
-  __syncthreads();
-  // (b) column sums for dgamma / dbeta: threads 0..63 -> dgamma[c], 64..127 -> dbeta[c]
-  // (COLS == false: the caller spreads them over all its threads, fused_mma.cuh)
-  if (COLS && t < 128) {
-    const int c = t & 63;
-    if (c < d.H) {
-      float s = 0.f;
-      if (t < 64) {
-        for (int r = 0; r < FR; ++r)
-          s += Gs[r * d.HS + c] * ((Xr[r * sxr + c * sxc] - rowstat[r * 4]) * rowstat[r * 4 + 1]);
-        dgamma_acc += s;
-      } else {
-        for (int r = 0; r < FR; ++r) s += Gs[r * d.HS + c];
-        dbeta_acc += s;
-      }
-    }
-  }
-}
-
-// column sum of a row-major tile: thread (tid % 64) of group (tid / 64) == grp adds sum_r Ts[r][c] to acc
-__device__ __forceinline__ void f_colsum(const float* __restrict__ Ts, int grp, const FDims& d, float& acc) {
-  const int t = threadIdx.x;
-  if ((t >> 6) == grp) {
-    const int c = t & 63;
-    if (c < d.H) {
-      float s = 0.f;
-      for (int r = 0; r < FR; ++r) s += Ts[r * d.HS + c];
-      acc += s;
-    }
-  }
-}
-
-__device__ __forceinline__ void f_store_wpartial(float* __restrict__ P, const float (&acc)[4][4], int ty, int tx,
-                                                 const FDims& d) {
-#pragma unroll
-  for (int ii = 0; ii < 4; ++ii) {
-    const int k = ty * 4 + ii;
-    if (k >= d.H) continue;
-#pragma unroll
-    for (int cc = 0; cc < 4; ++cc) {
-      const int n = tx * 4 + cc;
-      if (n < d.H) P[k * d.H + n] = acc[ii][cc];
-    }
-  }
-}
-
 struct FfnBwdArgs {
   const float *dx, *zn, *h1d, *y, *mean, *rstd, *gamma, *W1, *W2;
   const int* ids;
@@ -362,104 +119,6 @@ struct FfnBwdArgs {
   float* partial;  // [gridDim.x][2H + 2(H*H + H)]
   long ntiles;
 };
-
-__global__ void __launch_bounds__(FT) ffn_bwd_kernel(FfnBwdArgs a, FDims d) {
-  CAST_DYN_SMEM(float, sm);
-  float* Gm = sm;                       // dx * mask                       [FR][HS]
-  float* Gd = Gm + FR * d.HS;           // dx * mask * dropout, later dzn  [FR][HS]
-  float* Dh = Gd + FR * d.HS;           // gradient at the FFN hidden pre-activation
-  float* Yr = Dh + FR * d.HS;           // LN input tile (y)
-  float* HdT = Yr + FR * d.HS;          // h1d^T  [HP4][FTS]
-  float* ZnT = HdT + d.HP4 * FTS;       // zn^T   [HP4][FTS]
-  float* W2T = ZnT + d.HP4 * FTS;       // [HP4][HS]
-  float* W1T = W2T + d.HP4 * d.HS;
-  float* rowstat = W1T + d.HP4 * d.HS;  // [FR][4]
-  const int t = threadIdx.x, tx = t & 15, ty = t >> 4;
-  const int col = tx * 4;
-  const bool active = col < d.HP4;
-  const float scale = a.rate > 0.f ? 1.0f / (1.0f - a.rate) : 1.0f;
-  const Drop dout = make_drop(a.rate, a.seed, a.step, a.site_o);
-  f_load_w_T(W2T, a.W2, d);
-  f_load_w_T(W1T, a.W1, d);
-  float gW1[4][4], gW2[4][4];
-  zero_acc(gW1);
-  zero_acc(gW2);
-  float vb = 0.f;      // thread-owned vector gradient: group 0 -> db2, 1 -> db1 (tid/64), column tid%64
-  float dgam = 0.f, dbet = 0.f;
-  for (long tile = blockIdx.x; tile < a.ntiles; tile += gridDim.x) {
-    const long row0 = tile * FR;
-    __syncthreads();
-    {  // masked / dropped upstream gradient
-      const int lane = t & 31;
-      for (int r = t >> 5; r < FR; r += FT / 32) {
-        const long row = row0 + r;
-        const bool ok = row < d.N;
-        const float m = (ok && (!a.ids || a.ids[row] != 0)) ? 1.f : 0.f;
-        for (int c = lane; c < d.HP4; c += 32) {
-          float g = 0.f, gd = 0.f;
-          if (ok && c < d.H) {
-            g = a.dx[row * d.H + c] * m;
-            gd = g * drop_mul(dout, (unsigned long long)(row * d.H + c));
-          }
-          Gm[r * d.HS + c] = g;
-          Gd[r * d.HS + c] = gd;
-        }
-      }
-    }
-    f_load_rows(Yr, a.y, row0, d);
-    f_load_rows_T(HdT, a.h1d, row0, d);
-    f_load_rows_T(ZnT, a.zn, row0, d);
-    __syncthreads();
-    // dW2 += h1d^T Gd ; db2 += colsum(Gd) ; dh = (Gd W2^T) * relu/dropout mask
-    if (active) {
-      if (ty * 4 < d.HP4) pv_tile<4, 0>(HdT, FTS, Gd, d.HS, FR, col, gW2, ty);
-      float acc[4][4];
-      zero_acc(acc);
-      pv_tile<4, 0>(Gd, d.HS, W2T, d.HS, d.HP4, col, acc, ty);
-#pragma unroll
-      for (int ii = 0; ii < 4; ++ii) {
-        const int r = ty * 4 + ii;
-#pragma unroll
-        for (int cc = 0; cc < 4; ++cc) {
-          const int c = col + cc;
-          Dh[r * d.HS + c] = (c < d.H && HdT[c * FTS + r] > 0.f) ? acc[ii][cc] * scale : 0.f;
-        }
-      }
-    }
-    f_colsum(Gd, 0, d, vb);
-    __syncthreads();
-    // dW1 += zn^T Dh ; db1 += colsum(Dh) ; dzn = Dh W1^T + Gm  (stored over Gd)
-    if (active) {
-      if (ty * 4 < d.HP4) pv_tile<4, 0>(ZnT, FTS, Dh, d.HS, FR, col, gW1, ty);
-      float acc[4][4];
-      zero_acc(acc);
-      pv_tile<4, 0>(Dh, d.HS, W1T, d.HS, d.HP4, col, acc, ty);
-#pragma unroll
-      for (int ii = 0; ii < 4; ++ii) {
-        const int r = ty * 4 + ii;
-#pragma unroll
-        for (int cc = 0; cc < 4; ++cc) {
-          const int c = col + cc;
-          Gd[r * d.HS + c] = c < d.H ? acc[ii][cc] + Gm[r * d.HS + c] : 0.f;
-        }
-      }
-    }
-    f_colsum(Dh, 1, d, vb);
-    __syncthreads();
-    f_ln_bwd_rows(Gd, Yr, d.HS, 1, nullptr, a.gamma, a.mean, a.rstd, rowstat, row0, d, a.dy, dgam, dbet);
-  }
-  // ---- per-CTA partials in the flat gradient layout [beta | gamma | W1 | b1 | W2 | b2]
-  const int H = d.H;
-  float* P = a.partial + (long)blockIdx.x * (2L * H + 2L * (H * H + H));
-  if (t < 64 && t < H) P[H + t] = dgam;
-  if (t >= 64 && t < 128 && (t & 63) < H) P[t & 63] = dbet;
-  if (ty * 4 < d.HP4 && active) {
-    f_store_wpartial(P + 2 * H, gW1, ty, tx, d);
-    f_store_wpartial(P + 2 * H + H * H + H, gW2, ty, tx, d);
-  }
-  if ((t >> 6) == 1 && (t & 63) < H) P[2 * H + H * H + (t & 63)] = vb;                  // db1
-  if ((t >> 6) == 0 && (t & 63) < H) P[2 * H + H * H + H + H * H + (t & 63)] = vb;      // db2
-}
 
 struct QkvBwdArgs {
   const float *dQ, *dK, *dV, *dres, *x, *qn, *mean, *rstd, *gamma, *Wq, *Wk, *Wv;
@@ -484,94 +143,14 @@ __device__ __forceinline__ LnOutFx qkv_out_fx(const QkvBwdArgs& a) {
   return f;
 }
 
-__global__ void __launch_bounds__(FT) qkv_bwd_kernel(QkvBwdArgs a, FDims d) {
-  CAST_DYN_SMEM(float, sm);
-  float* Gq = sm;                      // dQ tile, later dqn
-  float* Gk = Gq + FR * d.HS;          // dK tile, later d(x) through K and V
-  float* Gv = Gk + FR * d.HS;
-  float* XT = Gv + FR * d.HS;          // x^T   [HP4][FTS]  (LN input; also read as x-hat source)
-  float* QnT = XT + d.HP4 * FTS;       // LN(x)^T
-  float* WqT = QnT + d.HP4 * FTS;
-  float* WkT = WqT + d.HP4 * d.HS;
-  float* WvT = WkT + d.HP4 * d.HS;
-  float* rowstat = WvT + d.HP4 * d.HS;
-  const int t = threadIdx.x, tx = t & 15, ty = t >> 4;
-  const int col = tx * 4;
-  const bool active = col < d.HP4;
-  const LnOutFx ofx = qkv_out_fx(a);
-  f_load_w_T(WqT, a.Wq, d);
-  f_load_w_T(WkT, a.Wk, d);
-  f_load_w_T(WvT, a.Wv, d);
-  float gWq[4][4], gWk[4][4], gWv[4][4];
-  zero_acc(gWq);
-  zero_acc(gWk);
-  zero_acc(gWv);
-  float vb = 0.f;  // group 0 -> dbq, 1 -> dbk, 2 -> dbv
-  float dgam = 0.f, dbet = 0.f;
-  for (long tile = blockIdx.x; tile < a.ntiles; tile += gridDim.x) {
-    const long row0 = tile * FR;
-    __syncthreads();
-    f_load_rows(Gq, a.dQ, row0, d);
-    f_load_rows(Gk, a.dK, row0, d);
-    f_load_rows(Gv, a.dV, row0, d);
-    f_load_rows_T(XT, a.x, row0, d);
-    f_load_rows_T(QnT, a.qn, row0, d);
-    __syncthreads();
-    float accq[4][4], acck[4][4];
-    zero_acc(accq);
-    zero_acc(acck);
-    if (active) {
-      if (ty * 4 < d.HP4) {
-        pv_tile<4, 0>(QnT, FTS, Gq, d.HS, FR, col, gWq, ty);
-        pv_tile<4, 0>(XT, FTS, Gk, d.HS, FR, col, gWk, ty);
-        pv_tile<4, 0>(XT, FTS, Gv, d.HS, FR, col, gWv, ty);
-      }
-      pv_tile<4, 0>(Gq, d.HS, WqT, d.HS, d.HP4, col, accq, ty);   // dqn (without the residual)
-      pv_tile<4, 0>(Gk, d.HS, WkT, d.HS, d.HP4, col, acck, ty);   // dx through K ...
-      pv_tile<4, 0>(Gv, d.HS, WvT, d.HS, d.HP4, col, acck, ty);   // ... and V
-    }
-    f_colsum(Gq, 0, d, vb);
-    f_colsum(Gk, 1, d, vb);
-    f_colsum(Gv, 2, d, vb);
-    __syncthreads();
-    if (active) {
-#pragma unroll
-      for (int ii = 0; ii < 4; ++ii) {
-        const int r = ty * 4 + ii;
-        const long row = row0 + r;
-#pragma unroll
-        for (int cc = 0; cc < 4; ++cc) {
-          const int c = col + cc;
-          const bool ok = c < d.H && row < d.N;
-          Gq[r * d.HS + c] = ok ? accq[ii][cc] + a.dres[row * d.H + c] : 0.f;  // + gradient of `outputs += queries`
-          Gk[r * d.HS + c] = ok ? acck[ii][cc] : 0.f;
-        }
-      }
-    }
-    __syncthreads();
-    f_ln_bwd_rows(Gq, XT, 1, FTS, Gk, a.gamma, a.mean, a.rstd, rowstat, row0, d, a.dx, dgam, dbet, ofx);
-  }
-  const int H = d.H;
-  float* P = a.partial + (long)blockIdx.x * (2L * H + 3L * (H * H + H));
-  if (t < 64 && t < H) P[H + t] = dgam;
-  if (t >= 64 && t < 128 && (t & 63) < H) P[t & 63] = dbet;
-  if (ty * 4 < d.HP4 && active) {
-    f_store_wpartial(P + 2 * H, gWq, ty, tx, d);
-    f_store_wpartial(P + 2 * H + (H * H + H), gWk, ty, tx, d);
-    f_store_wpartial(P + 2 * H + 2 * (H * H + H), gWv, ty, tx, d);
-  }
-  const int grp = t >> 6;
-  if (grp < 3 && (t & 63) < H) P[2 * H + grp * (H * H + H) + H * H + (t & 63)] = vb;
-}
-
 }  // namespace cast
 #include "fused_mma.cuh"
 namespace cast {
 
-// persistent grids: one wave of resident CTAs on the 148 SMs of a B200 (ffn_bwd: 2 CTAs/SM; qkv_bwd: 1 CTA/SM — 160
-// registers x 256 threads), so no CTA waits for a slot and the number of weight-gradient partials stays minimal
+// persistent grids: one wave of resident CTAs on the 148 SMs of a B200 (the backward kernels run one 512-thread CTA
+// per SM), so no CTA waits for a slot and the number of weight-gradient partials stays minimal
 constexpr int NUM_SMS = 148;
-static int bwd_grid(long ntiles, int ctas_per_sm = 2) {
+static int bwd_grid(long ntiles, int ctas_per_sm) {
   const long cap = (long)NUM_SMS * ctas_per_sm;
   return (int)(ntiles < cap ? ntiles : cap);
 }
@@ -590,14 +169,6 @@ using namespace cast;
   }
 
 extern "C" int cast_fused_supported(int H) { return H > 0 && H <= 64; }
-
-// bit 0: backward row kernels on the tensor cores (fused_mma.cuh), bit 1: forward row kernels; 0: FP32 FFMA kernels
-static int g_fused_backend = 3;
-extern "C" int cast_fused_set_backend(int backend) {
-  if (backend < 0 || backend > 3) return set_error(CAST_ERR_BAD_ARG, "fused_set_backend");
-  g_fused_backend = backend;
-  return CAST_OK;
-}
 
 template <int KS>
 static void launch_qkv_bwd_mma(const QkvBwdArgs& a, FDims d, int grid, cudaStream_t stream) {
@@ -648,15 +219,9 @@ extern "C" int cast_ln_qkv_fwd(const float* x, const float* gamma, const float* 
   if (!cast_fused_supported(H)) return set_error(CAST_ERR_UNSUPPORTED, "ln_qkv_fwd: H > 64");
   const FDims d = fdims(N, H);
   LnQkvArgs a{x, gamma, beta, {Wq, Wk, Wv}, {bq, bk, bv}, eps, qn, {Q, K, V}, mean, rstd, kmask, qmask};
-  if (g_fused_backend & 2) {
 #define CAST_CALL(K) launch_ln_qkv_fwd_mma<K>(a, d, (cudaStream_t)stream)
-    CAST_KS_SWITCH(H, CAST_CALL)
+  CAST_KS_SWITCH(H, CAST_CALL)
 #undef CAST_CALL
-    return check_launch("ln_qkv_fwd");
-  }
-  const size_t smem = sizeof(float) * ((size_t)2 * FR * d.HS + (size_t)d.HP4 * d.HS);
-  CAST_FUSED_SMEM(ln_qkv_fwd_kernel, smem)
-  CAST_LAUNCH(ln_qkv_fwd_kernel, dim3((unsigned)cdiv(N, FR)), dim3(FT), smem, (cudaStream_t)stream, a, d);
   return check_launch("ln_qkv_fwd");
 }
 
@@ -672,26 +237,22 @@ extern "C" int cast_ln_ffn_fwd(const float* y, const float* gamma, const float* 
   const FDims d = fdims(N, H);
   LnFfnArgs a{y, gamma, beta, W1, b1, W2, b2, ids, eps, drop_rate, seed, step, site_hidden, site_out,
               zn, h1d, xout, mean, rstd};
-  if (g_fused_backend & 2) {
 #define CAST_CALL(K) launch_ln_ffn_fwd_mma<K>(a, d, (cudaStream_t)stream)
-    CAST_KS_SWITCH(H, CAST_CALL)
+  CAST_KS_SWITCH(H, CAST_CALL)
 #undef CAST_CALL
-    return check_launch("ln_ffn_fwd");
-  }
-  const size_t smem = sizeof(float) * ((size_t)2 * FR * d.HS + (size_t)d.HP4 * d.HS);
-  CAST_FUSED_SMEM(ln_ffn_fwd_kernel, smem)
-  CAST_LAUNCH(ln_ffn_fwd_kernel, dim3((unsigned)cdiv(N, FR)), dim3(FT), smem, (cudaStream_t)stream, a, d);
   return check_launch("ln_ffn_fwd");
 }
 
 /* number of per-CTA partial blocks cast_ffn_bwd / cast_qkv_bwd leave in their workspace for N rows */
 extern "C" int cast_block_bwd_parts(long N, int which) {  // which: 0 = cast_ffn_bwd, 1 = cast_qkv_bwd
-  return bwd_grid(cdiv(N, FR), (which == 1 || (g_fused_backend & 1)) ? 1 : 2);
+  (void)which;  // both kernels run the same grid
+  return bwd_grid(cdiv(N, FR), 1);
 }
 
+// sized for up to two CTAs per SM, twice what the kernels use: callers size their buffers with this value, so it stays
 extern "C" size_t cast_block_bwd_workspace_bytes(long N, int H) {
   const long ntiles = cdiv(N, FR);
-  return (size_t)bwd_grid(ntiles) * (size_t)(2L * H + 3L * ((long)H * H + H)) * sizeof(float);
+  return (size_t)bwd_grid(ntiles, 2) * (size_t)(2L * H + 3L * ((long)H * H + H)) * sizeof(float);
 }
 
 extern "C" int cast_ffn_bwd(const float* dx, const int* ids, const float* zn, const float* h1d, const float* y,
@@ -706,19 +267,12 @@ extern "C" int cast_ffn_bwd(const float* dx, const int* ids, const float* zn, co
     return set_error(CAST_ERR_WORKSPACE, "ffn_bwd: workspace too small");
   const FDims d = fdims(N, H);
   const long ntiles = cdiv(N, FR);
-  const int grid = bwd_grid(ntiles, (g_fused_backend & 1) ? 1 : 2);
+  const int grid = bwd_grid(ntiles, 1);
   FfnBwdArgs a{dx, zn, h1d, y, mean, rstd, gamma, W1, W2, ids, drop_rate, seed, step, site_out, dy,
                static_cast<float*>(workspace), ntiles};
-  if (g_fused_backend & 1) {
 #define CAST_CALL(K) launch_ffn_bwd_mma<K>(a, d, grid, (cudaStream_t)stream)
-    CAST_KS_SWITCH(H, CAST_CALL)
+  CAST_KS_SWITCH(H, CAST_CALL)
 #undef CAST_CALL
-  } else {
-    const size_t smem = sizeof(float) * ((size_t)4 * FR * d.HS + (size_t)2 * d.HP4 * FTS + (size_t)2 * d.HP4 * d.HS +
-                                         (size_t)FR * 4);
-    CAST_FUSED_SMEM(ffn_bwd_kernel, smem)
-    CAST_LAUNCH(ffn_bwd_kernel, dim3(grid), dim3(FT), smem, (cudaStream_t)stream, a, d);
-  }
   int rc = check_launch("ffn_bwd");
   if (rc || !grads_out) return rc;  // grads_out == null: partials stay in the workspace (cast_reduce_partials_batch)
   const long count = 2L * H + 2L * ((long)H * H + H);
@@ -743,16 +297,9 @@ static int qkv_bwd_impl(const float* dQ, const float* dK, const float* dV, const
   const int grid = bwd_grid(ntiles, 1);
   QkvBwdArgs a{dQ, dK, dV, dres, x, qn, mean, rstd, gamma, Wq, Wk, Wv, dx, static_cast<float*>(workspace), ntiles,
                out_ids, out_rate, seed, step, out_site, out_fx};
-  if (g_fused_backend & 1) {
 #define CAST_CALL(K) launch_qkv_bwd_mma<K>(a, d, grid, (cudaStream_t)stream)
-    CAST_KS_SWITCH(H, CAST_CALL)
+  CAST_KS_SWITCH(H, CAST_CALL)
 #undef CAST_CALL
-  } else {
-    const size_t smem = sizeof(float) * ((size_t)3 * FR * d.HS + (size_t)2 * d.HP4 * FTS + (size_t)3 * d.HP4 * d.HS +
-                                         (size_t)FR * 4);
-    CAST_FUSED_SMEM(qkv_bwd_kernel, smem)
-    CAST_LAUNCH(qkv_bwd_kernel, dim3(grid), dim3(FT), smem, (cudaStream_t)stream, a, d);
-  }
   int rc = check_launch("qkv_bwd");
   if (rc || !grads_out) return rc;
   const long count = 2L * H + 3L * ((long)H * H + H);

@@ -1,6 +1,6 @@
-// Tensor-core versions of the fused row-tile kernels of fused.cu (included from there, after its helpers): same
-// arithmetic and gradient layout, contractions as mma.sync m16n8k8 3xTF32 (mma_tf32.cuh), tiles streamed through a
-// two-stage cp.async pipeline so the next 64-row tile loads while the current one is multiplied.
+// The fused row-tile kernels of fused.cu (included from there, after its helpers and argument structs): contractions
+// as mma.sync m16n8k8 3xTF32 (mma_tf32.cuh), tiles streamed through a two-stage cp.async pipeline so the next 64-row
+// tile loads while the current one is multiplied.
 //
 //   CTA = 8 warps (forward) or 16 warps (backward) on one 64-row tile; warp w owns the 16-row block (w & 3) and the
 //   column group (w >> 2: 32 or 16 columns) of every 64 x H product, and the same block of every H x H weight gradient.

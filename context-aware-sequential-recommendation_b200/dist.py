@@ -1,13 +1,16 @@
-"""Data-parallel training over the GPUs of one box: one process per GPU, `torch.distributed` (NCCL over NVLink 5 /
-NVSwitch) for the gradient all-reduce; with a row-sharded item table (BASELINE config 5) the table traffic bypasses the
-collective library altogether: kernels read the owning rank's memory over NVLink peer mappings (PeerArena).
+"""Data-parallel training over the GPUs of one box: one process per GPU.  `torch.distributed` only sets things up
+(broadcast of the initial weights, exchange of the peer-memory handles, evaluation's final histogram sum); inside a
+training step the ranks exchange gradients with plain kernel launches over NVLink peer mappings (PeerArena,
+PeerExchange): a flag barrier, then every rank sums the ranks' buffers itself in rank order.  No collective call sits
+in the step, so the whole step stays one CUDA graph.  With a row-sharded item table (BASELINE config 5) the table
+traffic goes the same way: kernels read the owning rank's memory directly.
 
 The reference is single-device (SURVEY §2.1); the semantics kept here are those of its loss: the gradient is the
 derivative of  sum(loss terms) / sum(istarget)  over the WHOLE batch (models/sasrec.py:105-108).  Each rank therefore
-contributes un-normalised gradient numerators plus its local sum(istarget); one flat `all_reduce(SUM)` over
-[gradients | loss_sum, auc_sum, count] makes every rank hold the global numerators and the global denominator, and
-the Adam kernel divides.  N ranks with B/N sequences each reproduce the single-GPU step on B sequences up to fp32
-summation order.
+contributes un-normalised gradient numerators plus its local sum(istarget); the rank-ordered sum over
+[gradients | loss_sum, auc_sum, count] gives every rank the same global numerators and global denominator (the same
+bits on every rank), and the Adam kernel divides.  N ranks with B/N sequences each reproduce the single-GPU step on
+B sequences up to fp32 summation order.
 """
 from __future__ import annotations
 
@@ -186,16 +189,12 @@ def _quiesce_at_exit(engine, group):
     atexit.register(_at_exit)
 
 
-def use_peer_exchange(engine) -> bool:
-    """peer-memory exchange unless CAST_DP_EXCHANGE=nccl (the process-group all-reduce, kept for A/B runs)"""
-    return os.environ.get("CAST_DP_EXCHANGE", "peer") != "nccl"
-
-
 def attach(engine, group=None, arena=None):
     """Make `engine.launch_train_step` data parallel over `group` (default: the world group): replicated parameters;
-    per step the ranks' [gradient numerators | loss_sum, auc_sum, count] buffers are summed in rank order, either by
-    every rank reading its peers' buffers over NVLink between two flag barriers (default: no collective call, the step
-    stays one CUDA graph) or by one process-group all-reduce (CAST_DP_EXCHANGE=nccl)."""
+    per step the ranks' [gradient numerators | loss_sum, auc_sum, count] buffers are summed in rank order.  A flag
+    barrier over NVLink marks every rank's gradient buffer final; the Adam pass then reads the ranks' buffers over
+    their peer mappings and adds them in rank order itself.  A second barrier, between the next step's forward and
+    backward passes, keeps any rank from overwriting its buffer while a peer may still read it."""
     if not dist.is_initialized() or dist.get_world_size(group) == 1:
         return engine
     if engine.item_shard is not None:
@@ -208,46 +207,25 @@ def attach(engine, group=None, arena=None):
     # independent dropout streams per rank (one global batch, different positions)
     engine.seed = (engine.seed + 0x9E3779B1 * engine.rank) & 0xFFFFFFFFFFFF
 
-    if use_peer_exchange(engine):
-        arena = arena or PeerArena(engine.lib, engine.device, group)
-        engine.arena = arena
-        px = engine.peer_exchange = PeerExchange(engine, arena, group)
+    arena = arena or PeerArena(engine.lib, engine.device, group)
+    engine.arena = arena
+    px = engine.peer_exchange = PeerExchange(engine, arena, group)
 
-        ab = os.environ.get("CAST_DP_EXCHANGE", "peer")
-        if ab == "peer3":         # A/B: separate reduction launch between two barriers (the first form of this path)
-            def exchange(c):
-                px.barrier()      # every rank's gradient buffer is final
-                px.reduce()       # (Adam consumes the reduced copy)
-                px.barrier()      # everybody has read everybody
-        else:
-            # One barrier on the critical path: every rank's gradient buffer is final => Adam sums the ranks' buffers
-            # itself (cast_adam_tf_step_peers).  The second barrier ("everybody has read everybody: the buffers may be
-            # overwritten") is only needed before the NEXT backward pass writes gradients, so it sits between the next
-            # step's forward and backward, where no rank waits for it.
-            def exchange(c):
-                px.barrier()
+    # One barrier on the critical path: every rank's gradient buffer is final => Adam sums the ranks' buffers itself
+    # (cast_adam_tf_step_peers).  The second barrier ("everybody has read everybody: the buffers may be overwritten")
+    # is only needed before the NEXT backward pass writes gradients, so it sits between the next step's forward and
+    # backward, where no rank waits for it.
+    def exchange(c):
+        px.barrier()
 
-            engine.peer_adam = (px.g_ptrs, px.world, px.g_red)
-            engine.before_backward = px.barrier
-            _quiesce_at_exit(engine, group)
-        if ab in ("none", "barrier"):   # measurement hooks only (wrong gradients): where does a multi-rank step's time go?
-            engine.peer_adam = engine.before_backward = None
-
-            def exchange(c):
-                if ab == "barrier":
-                    px.barrier()
-                engine.adam_g.copy_(engine.gbuf)
-        engine.grad_allreduce = exchange
-        engine.exchange_capturable = True
-        if engine.device.type == "cuda":
-            torch.cuda.synchronize(engine.device)
-        dist.barrier(group=group)
-        return engine
-
-    def allreduce(c):
-        dist.all_reduce(engine.gbuf, op=dist.ReduceOp.SUM, group=group)
-
-    engine.grad_allreduce = allreduce
+    engine.peer_adam = (px.g_ptrs, px.world, px.g_red)
+    engine.before_backward = px.barrier
+    _quiesce_at_exit(engine, group)
+    engine.grad_allreduce = exchange
+    engine.exchange_capturable = True
+    if engine.device.type == "cuda":
+        torch.cuda.synchronize(engine.device)
+    dist.barrier(group=group)
     return engine
 
 
@@ -258,8 +236,9 @@ def attach_sharded(engine, group=None, arena: "PeerArena | None" = None):
       forward / backward   the embedding, positive and negative lookups read rows from the owning rank's shard over
                            NVLink (peer mappings; no exchange step, no staging buffers); every rank sorts its
                            (item id, entry) pairs by (owner, local row) on a side stream
-      all-reduce           [dense-weight gradients | loss_sum, auc_sum, count] — also the barrier after which every
-                           rank's sorted entries and source rows are final
+      exchange             a flag barrier (every rank's dense gradients, sorted entries and source rows are final),
+                           then the rank-ordered sum of [dense-weight gradients | loss_sum, auc_sum, count] read
+                           from the peers' buffers
       owner pull           each rank folds, rank by rank in rank order, the entries that hit ITS rows (read from the
                            peers' memory) into its dense gradient shard: fixed order, no atomics, no table collective
       TF-Adam              one launch over [own shard | dense weights]  (28 B/param of table traffic divided by world)
@@ -290,7 +269,6 @@ def attach_sharded(engine, group=None, arena: "PeerArena | None" = None):
     shards = arena.ptrs(engine.w)          # the shard is the first tensor of the flat parameter buffer
     engine.shard_ptrs = torch.tensor(shards, dtype=torch.int64, device=engine.device)
     R, H = engine.shard_R, engine.H
-    flag = torch.zeros(1, dtype=torch.float32, device=engine.device)
 
     def build_peer_view(c):
         """pointers to every rank's sorted entries and source rows for this batch size (collective, first step only)"""
@@ -314,17 +292,12 @@ def attach_sharded(engine, group=None, arena: "PeerArena | None" = None):
                             device=engine.device)
         c.peer = SimpleNamespace(view=view, scale=(C.c_float * nsrc)(*scale), nsrc=nsrc, stage=stage, spart=spart)
 
-    px = None
-    if use_peer_exchange(engine):
-        px = engine.peer_exchange = PeerExchange(engine, arena, group, first=region)
-        engine.exchange_capturable = True
+    px = engine.peer_exchange = PeerExchange(engine, arena, group, first=region)
+    engine.exchange_capturable = True
 
     def exchange(c):
-        if px is not None:
-            px.barrier()    # every rank's dense gradients, sorted entries and source rows are final
-            px.reduce()     # dense gradients + loss sums, rank order
-        else:
-            dist.all_reduce(engine.gbuf[region:], op=dist.ReduceOp.SUM, group=group)
+        px.barrier()    # every rank's dense gradients, sorted entries and source rows are final
+        px.reduce()     # dense gradients + loss sums, rank order
         if c.peer is None:
             build_peer_view(c)
         pv = c.peer
@@ -340,14 +313,8 @@ def attach_sharded(engine, group=None, arena: "PeerArena | None" = None):
                              pv.stage.numel() * 4, pv.spart.data_ptr(), pv.spart.numel() * 4, 1 if p else 0,
                              engine._stream())
 
-    def end_of_step():
-        if px is not None:
-            px.barrier()    # shards are updated; exported buffers may be overwritten
-        else:
-            dist.all_reduce(flag, op=dist.ReduceOp.SUM, group=group)
-
     engine.grad_allreduce = exchange
-    engine.after_adam = end_of_step
+    engine.after_adam = px.barrier   # shards are updated; exported buffers may be overwritten
     if engine.device.type == "cuda":
         torch.cuda.synchronize(engine.device)
     dist.barrier(group=group)      # every shard is initialised before anybody gathers from it

@@ -204,15 +204,13 @@ class Engine:
         self.world_size = 1
         self.grad_allreduce = None  # set by dist.attach(); called between backward and Adam
         self.adam_g = self.gbuf     # what Adam consumes: the local buffer, or the rank-ordered sum (dist.PeerExchange)
-        self.exchange_capturable = False   # the exchange is plain kernel launches => the step is one CUDA graph
+        self.exchange_capturable = False   # dist.attach*: the exchange is plain kernel launches (the step is one graph)
         self.after_adam = None      # set by dist.attach_sharded(): the barrier that ends a row-sharded step
         # the step's kernels form a chain whose operands obey include/cast_b200.h's cast_set_pdl contract (weights are
         # last written by the optimizer pass of the previous step, images on a joined side stream, activations of the
         # forward pass long before the backward kernels that re-read them): programmatic dependent launch is safe here
         if self.device.type == "cuda":
             self.lib.cast_set_pdl(0 if os.environ.get("CAST_PDL", "1") == "0" else 1)
-        self.fork_reduce = os.environ.get("CAST_FORK_REDUCE", "1") != "0"            # A/B switches (measurement)
-        self.fuse_embed_bwd = os.environ.get("CAST_FUSE_EMBED_BWD", "1") != "0"
         self.before_backward = None  # set by dist.attach(): the barrier that lets this step overwrite the gradient buffer
         self.peer_adam = None       # set by dist.attach(): (device pointer table, n_ranks, g_red) => Adam sums the ranks' buffers
         self.shard_ptrs = None      # ... device array of the ranks' item-table shard pointers (own + peer mappings)
@@ -762,8 +760,7 @@ class Engine:
         add_time, drop, mask = plan.embed
         pre_merge = bool(plan.merge and plan.merge[3] == "pre")
         # the tower's input is dropout(emb) * mask: block 0's fused backward kernel applies that gradient itself
-        fuse_embed = ((drop or mask) and not pre_merge and self.use_fused and self.fuse_embed_bwd
-                      and len(c.tw["main"].blocks) > 0
+        fuse_embed = ((drop or mask) and not pre_merge and self.use_fused and len(c.tw["main"].blocks) > 0
                       and bool(self.lib.cast_fused_supported(self.H)))
         d = self.tower_bwd(c, "main", d, ids, embed_fx=(ids if mask else None, self.rate if drop else 0.0, SITE_EMBED,
                                                         c.g0) if fuse_embed else None)
@@ -800,7 +797,7 @@ class Engine:
             ctx_scatter.append((j, dk, tname))
         # every deferred partial sum of the step is known now: its one reduction launch runs beside the embedding
         # gradient scatters (independent outputs; a parallel branch of the captured graph), joined before the exchange
-        forked = self.fork_reduce and self.device.type == "cuda" and self.timing is None and bool(c.reduce_jobs)
+        forked = self.device.type == "cuda" and self.timing is None and bool(c.reduce_jobs)
         if forked:
             main = torch.cuda.current_stream(self.device)
             if getattr(c, "side3", None) is None:
@@ -926,7 +923,7 @@ class Engine:
             c.reduce_jobs = []
 
     def launch_train_step(self, c):
-        """Enqueue one full training step (forward, loss, backward, [all-reduce], Adam) on the current stream."""
+        """Enqueue one full training step (forward, loss, backward, [gradient exchange], Adam) on the current stream."""
         self.launch_fwd_bwd(c)
         if self.grad_allreduce is not None:
             self.grad_allreduce(c)

@@ -109,8 +109,8 @@ class _Model:
             st["event"].record(torch.cuda.current_stream(eng.device))
 
     def _capture(self, c):
-        """Capture the step as CUDA graphs: [forward+loss+backward] and [Adam]; under data parallelism the NCCL
-        all-reduce runs between the two replays (3 host launches per step instead of ~70)."""
+        """Capture the whole step (forward, loss, backward, the data-parallel exchange, Adam) as one CUDA graph: one
+        host launch per step instead of ~70.  The exchange is plain kernel launches (dist.PeerExchange)."""
         eng = self.engine
         # one eager step first (lazy CUDA init, smem attributes), with parameters / optimizer state restored after
         saved = (eng.w.clone(), eng.m.clone(), eng.v.clone(), eng.adam_state.clone())
@@ -121,42 +121,22 @@ class _Model:
         eng.w.copy_(saved[0]); eng.m.copy_(saved[1]); eng.v.copy_(saved[2]); eng.adam_state.copy_(saved[3])
         s = torch.cuda.Stream(device=eng.device)
         s.wait_stream(torch.cuda.current_stream(eng.device))
-        g1, g2 = torch.cuda.CUDAGraph(), torch.cuda.CUDAGraph()
-        # one process, or an exchange made of kernel launches only (dist.PeerExchange): the whole step is one graph
-        single = (eng.grad_allreduce is None and eng.after_adam is None) or eng.exchange_capturable
+        g = torch.cuda.CUDAGraph()
         with torch.cuda.stream(s):
-            with torch.cuda.graph(g1, stream=s):
-                eng.launch_fwd_bwd(c)
-                if single:
-                    if eng.grad_allreduce is not None:
-                        eng.grad_allreduce(c)
-                    eng.adam(c)
-                    if eng.after_adam is not None:
-                        eng.after_adam()
-            if not single:
-                with torch.cuda.graph(g2, stream=s):
-                    eng.adam(c)
-            else:
-                g2 = None
+            with torch.cuda.graph(g, stream=s):
+                eng.launch_train_step(c)
         torch.cuda.current_stream(eng.device).wait_stream(s)
         eng.w.copy_(saved[0]); eng.m.copy_(saved[1]); eng.v.copy_(saved[2]); eng.adam_state.copy_(saved[3])
-        c.graph = (g1, g2)
+        c.graph = g
 
     def launch(self, c):
         """Enqueue one training step on the batch already resident in c.keys3 / c.cids."""
-        eng = self.engine
         if self.use_graph:
             if c.graph is None:
                 self._capture(c)
-            c.graph[0].replay()
-            if c.graph[1] is not None:
-                if eng.grad_allreduce is not None:
-                    eng.grad_allreduce(c)
-                c.graph[1].replay()
-                if eng.after_adam is not None:
-                    eng.after_adam()
+            c.graph.replay()
         else:
-            eng.launch_train_step(c)
+            self.engine.launch_train_step(c)
 
     def _score_cand(self, last, ld, B, cand, Cn, logits, cgt=None, ceq=None):
         """logits (+ rank counts) of per-user candidate lists; the item rows come from the local table or, with a

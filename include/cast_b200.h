@@ -195,9 +195,6 @@ int cast_rowk_status(int* timed_out);
 int cast_rowk_set_grid(int max_ctas);
 /* tuning hook: device buffer of 148*4*16 int64 filled with clock64() phase stamps by the row kernels (NULL: off) */
 int cast_rowk_set_trace(void* device_buffer);
-/* Row-kernel backend (A/B testing): bit 0 = backward kernels on the tensor cores (mma.sync 3xTF32), bit 1 = forward
- * kernels; default 3; 0 = FP32 FFMA kernels. */
-int cast_fused_set_backend(int backend);
 size_t cast_block_bwd_workspace_bytes(long N, int H);
 /* cast_ffn_bwd / cast_qkv_bwd sum their per-CTA gradient partials (workspace layout [parts][count], count =
  * 2H + 2(H*H+H) resp. 2H + 3(H*H+H)) into grads_out with a fixed-order reduction launch.  With grads_out == NULL the
@@ -243,7 +240,6 @@ int cast_attn_fwd(const float* Q, long ldq, const float* K, long ldk, const floa
                   const float* kmask, const float* qmask, int B, int T, int H, int h, float drop_rate,
                   unsigned long long seed, const unsigned long long* step, int site, const int* skip_ids, float* out,
                   float* attn_weights, float* row_max, float* row_linv, void* stream);
-/* Tuning hook: columns per streamed chunk of the tensor-core attention kernels (32 or 64; default 32). */
 /* Programmatic dependent launch of the training step's main-chain kernels.  Off (0, the default): ordinary
  * stream-ordered launches, any operand may come from the immediately preceding launch.  On (1, what engine.py sets):
  * the next kernel's CTAs may be scheduled while the previous kernel drains, and a kernel reads a few operands BEFORE it
@@ -254,10 +250,6 @@ int cast_attn_fwd(const float* Q, long ldq, const float* K, long ldk, const floa
  *   - cast_attn_bwd with out / queries: every input except dO (Q, K, V, out, queries, masks, row_max, row_linv, skip_ids).
  * Everything else is read, and everything is written, after the wait, so results do not change. */
 int cast_set_pdl(int on);
-int cast_attn_set_chunk(int columns);
-/* Tuning hook: warps that share one 16-row block of a 64-row attention tile, each taking a 32-key slice of every
- * streamed chunk (forward and dQ kernels): 2 = 8 warps, two CTAs per SM (default); 4 = 16 warps, one CTA per SM. */
-int cast_attn_set_kg(int key_groups);
 /* Gradient of the attention output (without the residual branch) w.r.t. Q, K, V.  rowD: scratch [B,h,T].
  * out / queries (optional, both or neither): the forward call's `out` and `queries`; with them (and d = H/h <= 64)
  * the tensor-core kernels run and D_i = sum_j P_ij dP_ij is taken as dO_i . (out_i - queries_i).

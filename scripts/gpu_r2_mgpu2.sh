@@ -1,5 +1,5 @@
 #!/bin/bash
-# 2-GPU: peer exchange vs nccl at C2, row-sharded C5, pull micro-benchmark, scatter tests
+# 2-GPU: peer exchange at C2, row-sharded C5, pull micro-benchmark, scatter tests
 cd "$(dirname "$0")/.."
 mkdir -p gpurun_out
 N=${1:-2}
@@ -14,6 +14,5 @@ PY
 }
 timeout 600 python -m pytest tests/test_scatter.py -m gpu -x -q 2>&1 | tail -2
 run c2peer --steps 20 --warmup 5 --no_profile --no_cpu_baseline --no_eval
-CAST_DP_EXCHANGE=nccl run c2nccl --steps 20 --warmup 5 --no_profile --no_cpu_baseline --no_eval
 run c5peer --config c5 --steps 10 --warmup 3 --no_profile --no_cpu_baseline --no_eval
 timeout 600 python -m torch.distributed.run --nnodes=1 --nproc-per-node $N --master-addr 127.0.0.1 --master-port 29531 scripts/bench_pull.py c5 2>&1 | grep "^rank"

@@ -142,29 +142,3 @@ GPU = [(8, 200, 50, 1, 0.2, True, "mma"), (8, 200, 50, 1, 0.2, False, "mma"), (5
 def test_attention_gpu(B, T, H, h, rate, use_ids, path):
     run_case("gpu", B, T, H, h, rate, use_ids, path)
 
-
-# the 16-warp / four-key-group configuration of the forward and dQ kernels (tuning hook cast_attn_set_kg; the
-# default is two key groups): same results within the same tolerance
-KG4 = [(8, 200, 50, 1, 0.2, True, "mma_ws"), (5, 200, 50, 2, 0.2, False, "mma_ws"), (3, 300, 40, 1, 0.2, False, "mma_ws"),
-       (3, 37, 50, 2, 0.5, True, "mma_ws")]
-
-
-def _with_kg4(kind, *case):
-    lib, _ = backend(kind)
-    assert lib.cast_attn_set_kg(3) != 0          # only 2 or 4
-    assert lib.cast_attn_set_kg(4) == 0
-    try:
-        run_case(kind, *case)
-    finally:
-        assert lib.cast_attn_set_kg(2) == 0
-
-
-@pytest.mark.emu
-def test_attention_four_key_groups_emulated():
-    _with_kg4("emu", 2, 150, 12, 1, 0.25, True, "mma_ws")
-
-
-@pytest.mark.gpu
-@pytest.mark.parametrize("B,T,H,h,rate,use_ids,path", KG4)
-def test_attention_four_key_groups_gpu(B, T, H, h, rate, use_ids, path):
-    _with_kg4("gpu", B, T, H, h, rate, use_ids, path)

@@ -1,7 +1,8 @@
 """Data-parallel path with world_size 2 on CPU (`gloo`), kernels host-emulated (tests/emu, test infrastructure):
 two ranks with B/2 sequences each must reproduce the single-process step on B sequences — the reference's loss is
 sum(terms)/sum(istarget) over the WHOLE batch (models/sasrec.py:105-108), so ranks exchange un-normalised numerators
-plus the target count in one all-reduce (dist.py) — and the evaluation histogram reduction must be exact."""
+plus the target count, summed in rank order over peer memory (dist.py) — and the evaluation histogram reduction must
+be exact."""
 import os
 import socket
 
@@ -30,9 +31,9 @@ def _load_batch(eng, gb, lo, hi):
     return c
 
 
-def _worker(rank, world, port, model, out, shard=False, exchange="peer"):
+def _worker(rank, world, port, model, out, shard=False):
     os.environ.update(MASTER_ADDR="127.0.0.1", MASTER_PORT=str(port), RANK=str(rank), WORLD_SIZE=str(world),
-                      LOCAL_RANK=str(rank), CAST_DP_EXCHANGE=exchange)
+                      LOCAL_RANK=str(rank))
     from cast_b200 import dist as cdist
     from cast_b200 import evaluation as cev
     cdist.init_from_env("gloo")
@@ -75,12 +76,12 @@ def _worker(rank, world, port, model, out, shard=False, exchange="peer"):
 
 
 @pytest.mark.emu
-@pytest.mark.parametrize("model,exchange", [("sasrec", "peer"), ("cast_1", "peer"), ("sasrec", "nccl")])
-def test_two_rank_step_equals_single_process(tmp_path, model, exchange):
-    """exchange = "peer": rank-ordered sum over peer memory between two flag barriers (dist.PeerExchange; shared memory
-    stands in for NVLink); "nccl": the process-group all-reduce (gloo here)."""
+@pytest.mark.parametrize("model", ["sasrec", "cast_1"])
+def test_two_rank_step_equals_single_process(tmp_path, model):
+    """rank-ordered sum over peer memory behind a flag barrier (dist.PeerExchange; shared memory stands in for
+    NVLink)"""
     out = str(tmp_path / "res.pt")
-    mp.spawn(_worker, args=(2, _free_port(), model, out, False, exchange), nprocs=2, join=True)
+    mp.spawn(_worker, args=(2, _free_port(), model, out, False), nprocs=2, join=True)
     r = torch.load(out, weights_only=False)
     g_dp, g_1 = r["g_dp"], r["g_1"]
     assert abs(g_dp[-2] - g_1[-2]) == 0            # sum(istarget): exact
@@ -109,7 +110,7 @@ def _unshard(flat_per_rank, R, H, V):
 def test_row_sharded_item_table_step_equals_single_process(tmp_path):
     """dist.attach_sharded (BASELINE config 5 path) on 2 ranks: each rank holds HALF of the item table (+ its gradient
     and Adam slots); lookups read the owning rank's shard (POSIX shared memory standing in for NVLink peer memory);
-    after the all-reduce of the dense gradients each owner folds both ranks' sorted entries into its gradient shard
+    after the exchange of the dense gradients each owner folds both ranks' sorted entries into its gradient shard
     in rank order and runs Adam on [own shard | dense weights].  No table collective.  Gradient and parameters of every
     table row must equal the single-process step on the whole batch."""
     out = str(tmp_path / "res.pt")
