@@ -130,13 +130,14 @@ class Engine:
     """Owns parameters, optimizer state, activations and launches.  One instance per process / GPU."""
 
     def __init__(self, model: str, usernum: int, itemnum: int, args, device=None, lib=None, seed: Optional[int] = None,
-                 item_shard: Optional[tuple] = None, alloc=None):
+                 item_shard: Optional[tuple] = None, alloc=None, fused: bool = True):
         """item_shard = (rank, world): this process owns one row shard of the item table (BASELINE config 5; the
         other shards are read over NVLink peer mappings once dist.attach has exchanged them).  alloc(numel, dtype) ->
-        tensor: allocator for the buffers peers read (CPU tests: POSIX shared memory; default torch)."""
+        tensor: allocator for the buffers peers read (CPU tests: POSIX shared memory; default torch).
+        fused=False runs every block on the generic LayerNorm + GEMM kernels even where the row kernels apply (the
+        reference the row kernels are tested against)."""
         self.lib = lib if lib is not None else _lib.load_library()
         self.timing = None
-        self.use_fused = True
         if device is None:
             if not torch.cuda.is_available():
                 raise _lib.CastError("no CUDA device: this package has no CPU fallback")
@@ -190,17 +191,28 @@ class Engine:
         self.sinus = torch.from_numpy(sinusoid_table(self.H, self.T)).to(self.device)
         self.init_parameters(self.seed or 42)
         self._call(self.lib.cast_adam_init_state, self.adam_state.data_ptr(), self.beta1, self.beta2, self._stream())
-        self._ctx: Dict[tuple, SimpleNamespace] = {}
-        # tcgen05 row kernels (csrc/row_umma.cu): per-block weight operand images, rebuilt once per forward pass
-        self.use_rowk = bool(self.lib.cast_rowk_supported(self.H))
-        self.rowk_block: Dict[str, int] = {}
-        if self.use_rowk:
-            names = [f"{tower}.{i}." for tower, nb in self.plan.towers.items() for i in range(nb)]
+        self._ctx: Dict[int, SimpleNamespace] = {}
+        # The kernels every transformer block runs on, fixed for the engine's lifetime (the row kernels take H <= 64):
+        #   "rowk"   forward on the tcgen05 row kernels (csrc/row_umma.cu), backward on the mma.sync row kernels
+        #   "fused"  the mma.sync row kernels both ways (csrc/fused.cu)
+        #   "gemm"   LayerNorm kernels + cast_gemm / cast_colsum
+        # Both row-kernel paths defer their gradient partial sums to one reduction launch per step.
+        names = [f"{tower}.{i}." for tower, nb in self.plan.towers.items() for i in range(nb)]
+        if fused and self.lib.cast_rowk_supported(self.H) and names:
+            self.block_path = "rowk"
+        elif fused and self.lib.cast_fused_supported(self.H):
+            self.block_path = "fused"
+        else:
+            self.block_path = "gemm"
+        if self.block_path == "rowk":   # per-block weight operand images, rebuilt once per forward pass
             self.rowk_block = {n: j for j, n in enumerate(names)}
             self.rowk_img_bytes = int(self.lib.cast_rowk_image_bytes(self.H))
-            self.rowk_img = torch.zeros(max(1, len(names)) * self.rowk_img_bytes, dtype=torch.uint8, device=self.device)
+            self.rowk_img = torch.zeros(len(names) * self.rowk_img_bytes, dtype=torch.uint8, device=self.device)
             ptrs = [self.P[n + w].data_ptr() for n in names for w in ("q.w", "k.w", "v.w", "ffn1.w", "ffn2.w")]
             self.rowk_wptrs = (C.c_void_p * len(ptrs))(*ptrs)
+        # final LayerNorm + loss + LayerNorm backward in one launch: the main tower's output must be seq_emb itself
+        self.fuse_tail = (self.block_path != "gemm" and self.item_shard is None
+                          and not (self.plan.merge and self.plan.merge[3] == "post"))
         self.world_size = 1
         self.grad_allreduce = None  # set by dist.attach(); called between backward and Adam
         self.adam_g = self.gbuf     # what Adam consumes: the local buffer, or the rank-ordered sum (dist.PeerExchange)
@@ -240,6 +252,29 @@ class Engine:
             rc = fn(*a)
         if rc != 0:
             _lib.check(self.lib, rc, fn.__name__)
+
+    def _fork(self, c, name: str, fn) -> bool:
+        """Runs fn() on the context's side stream `name` after the work enqueued so far on the current stream: a
+        parallel branch of the step (and of its captured graph) until _join(c, name).  Where the step runs in stream
+        order (no CUDA device, per-call timing) nothing is enqueued and it returns False."""
+        if self.device.type != "cuda" or self.timing is not None:
+            return False
+        s = c.streams.get(name)
+        if s is None:
+            s = c.streams[name] = torch.cuda.Stream(device=self.device)
+        s.wait_stream(torch.cuda.current_stream(self.device))
+        with torch.cuda.stream(s):
+            fn()
+        c.forked[name] = s
+        return True
+
+    def _join(self, c, name: str) -> bool:
+        """The current stream waits for the branch `name` if it is forked; returns whether it was."""
+        s = c.forked.pop(name, None)
+        if s is None:
+            return False
+        torch.cuda.current_stream(self.device).wait_stream(s)
+        return True
 
     @staticmethod
     def _p(t):
@@ -304,17 +339,22 @@ class Engine:
 
     # ------------------------------------------------------------------ buffers
     def ctx(self, B: int) -> SimpleNamespace:
-        key = (B, bool(self.use_fused))   # the per-block workspaces differ between the fused and the unfused path
-        c = self._ctx.get(key)
+        c = self._ctx.get(B)
         if c is not None:
             return c
         H, T, h, dev = self.H, self.T, self.h, self.device
         N = B * T
         lib = self.lib
+        fused = self.block_path != "gemm"
         f = lambda *s: torch.empty(*s, dtype=torch.float32, device=dev)  # noqa: E731
         # buffers the other ranks read during the row-sharded gradient exchange (dist.attach_sharded)
         fp = (lambda *s: self._peer_zeros(int(np.prod(s)), torch.float32).view(*s)) if self.item_shard else f
         c = SimpleNamespace(B=B, N=N)
+        c.streams = {}       # name -> side stream of this context (_fork), created on first use
+        # per step, left empty by launch_fwd_bwd: the side-stream branches forked and not yet joined (name -> stream)
+        # and the deferred gradient partial sums (flush_reduce_jobs)
+        c.forked = {}
+        c.reduce_jobs = []
         c.keys3 = torch.zeros(3, N, dtype=torch.int32, device=dev)   # input_seq | pos | neg
         c.cids = torch.zeros(3, N, dtype=torch.int32, device=dev)    # time_seq | hours | days
         c.tw = {}
@@ -328,14 +368,19 @@ class Engine:
                     setattr(b, nm, f(N))
                 for nm in ("rmax", "rlinv", "rowD"):
                     setattr(b, nm, f(B * h * T))
-                if self.use_fused and bool(self.lib.cast_fused_supported(H)):
+                if fused:
                     # own partial buffers per block: the fixed-order reduction of all blocks is one launch at the end
                     # of backward (cast_reduce_partials_batch) instead of one small launch per fused backward kernel
                     nws = self.lib.cast_block_bwd_workspace_bytes(N, H) // 4 + 16
                     b.ws_ffn, b.ws_qkv = f(nws), f(nws)
                 blocks.append(b)
+            # x_last: the main tower's last block output, normalised by cast_lnf_loss (fuse_tail);
+            # ws_lnf: the gamma/beta partials of the final LayerNorm's backward (row-kernel paths, unless fuse_tail)
+            lnf_partials = fused and not (tower == "main" and self.fuse_tail)
             c.tw[tower] = SimpleNamespace(blocks=blocks, out=(fp if tower == "main" else f)(N, H), muf=f(N), rsf=f(N),
-                                          dx_in=f(N, H), x_in=None)
+                                          dx_in=f(N, H), x_in=None, x_last=None,
+                                          ws_lnf=f(lib.cast_layernorm_bwd_workspace_bytes(N, H) // 4 + 16)
+                                          if lnf_partials else None)
         # attention backward scratch: P~ and dS of one block ([2][h*B,T,T]), shared by all blocks (d <= 64 only)
         c.attn_ws = None
         if H // h <= 64 and 2 * B * h * T * T * 4 <= (2 << 30):
@@ -361,6 +406,12 @@ class Engine:
                  lib.cast_logits_loss_workspace_bytes(N), lib.cast_block_bwd_workspace_bytes(N, H))
         c.ws = torch.empty(ws // 4 + 16, dtype=torch.float32, device=dev)
         c.ws_bytes = ws
+        # the training step's loss partial sums, reduced with the other deferred jobs: cast_lnf_loss's (fuse_tail,
+        # with the final LayerNorm's gamma/beta partials) or cast_logits_loss's
+        c.ws_tail = f(lib.cast_lnf_loss_workspace_bytes(N, H) // 4 + 16) if self.fuse_tail else None
+        c.ws_loss = None if self.fuse_tail else f(lib.cast_logits_loss_workspace_bytes(N) // 4 + 16)
+        c.seq_emb = None     # the forward pass's output (forward)
+        c.shard_src = None   # the item-table gradient's source rows for the sharded exchange (scatter)
         vmax = max(self.P[t].shape[0] for t in self.plan.tables)
         if self.item_shard:
             vmax = max(vmax, self.item_shard[1] * self.shard_R)   # owner-major key range of the sharded sort
@@ -374,7 +425,7 @@ class Engine:
         c.spart_bytes = spb
         c.attn = None
         c.graph = None
-        self._ctx[key] = c
+        self._ctx[B] = c
         return c
 
     # ------------------------------------------------------------------ op wrappers
@@ -438,19 +489,14 @@ class Engine:
         rs_a = (C.c_void_p * nsrc)(*[(r.data_ptr() if r is not None else None) for r in rowscale])
         sc_a = (C.c_float * nsrc)(*scale)
         if table_name == "item_emb" and self.item_shard is not None:
-            if getattr(c, "presorted", False):
-                torch.cuda.current_stream(self.device).wait_stream(c.side)
-                c.presorted = False
-            else:
+            if not self._join(c, "sort"):   # sorted on a side stream during the forward pass (launch_fwd_bwd)
                 self._call(self.lib.cast_scatter_sort_sharded, keys.data_ptr(), nsrc, N, self.V_items,
                            self.item_shard[1], self.shard_R, c.sws.data_ptr(), c.sws_bytes, self._stream())
             if rows[0] is not c.g0:    # peers read the input-sequence gradient from the exported buffer
                 c.g0.copy_(rows[0])
             c.shard_src = (nsrc, [c.g0] + list(rows[1:]), list(rowscale), list(scale))
             return
-        if table_name == "item_emb" and getattr(c, "presorted", False):
-            torch.cuda.current_stream(self.device).wait_stream(c.side)   # join the side-stream sort
-            c.presorted = False
+        if table_name == "item_emb" and self._join(c, "sort"):   # the ids are sorted already: only the sums remain
             self._call(self.lib.cast_scatter_apply, nsrc, N, rows_a, rs_a, sc_a, V, self.H,
                        self.G[table_name].data_ptr(), c.sws.data_ptr(), c.sws_bytes, c.spart.data_ptr(),
                        c.spart_bytes, 0, self._stream())
@@ -468,21 +514,18 @@ class Engine:
         H, B, T, h = self.H, c.B, self.T, self.h
         x = x_in
         nb = len(tb.blocks)
-        fused = self.use_fused and bool(self.lib.cast_fused_supported(H))
-        rowk = self.rowk_active()
-        if rowk and getattr(c, "presplit_pending", False):   # join the side-stream weight split (launch_fwd_bwd)
-            torch.cuda.current_stream(self.device).wait_stream(c.side2)
-            c.presplit_pending = False
+        path = self.block_path
+        self._join(c, "presplit")   # the rowk weight split, if launch_fwd_bwd forked it
         P = self.P
         for i, b in enumerate(tb.blocks):
             pre = f"{tower}.{i}."
-            if rowk:
+            if path == "rowk":
                 self._call(self.lib.cast_rowk_ln_qkv_fwd, x.data_ptr(), P[pre + "ln1.gamma"].data_ptr(),
                            P[pre + "ln1.beta"].data_ptr(), P[pre + "q.b"].data_ptr(), P[pre + "k.b"].data_ptr(),
                            P[pre + "v.b"].data_ptr(), self.rowk_image(pre), c.N, H, 1e-8, b.qn.data_ptr(),
                            b.Q.data_ptr(), b.K.data_ptr(), b.V.data_ptr(), b.mu1.data_ptr(), b.rs1.data_ptr(),
                            b.kmask.data_ptr(), b.qmask.data_ptr(), self._stream())
-            elif fused:
+            elif path == "fused":
                 self._call(self.lib.cast_ln_qkv_fwd, x.data_ptr(), P[pre + "ln1.gamma"].data_ptr(),
                            P[pre + "ln1.beta"].data_ptr(), P[pre + "q.w"].data_ptr(), P[pre + "q.b"].data_ptr(),
                            P[pre + "k.w"].data_ptr(), P[pre + "k.b"].data_ptr(), P[pre + "v.w"].data_ptr(),
@@ -503,13 +546,13 @@ class Engine:
                        b.qn.data_ptr(), b.kmask.data_ptr(), b.qmask.data_ptr(), B, T, H, h, rate, self.seed,
                        self.step_ptr, block_site(tower, i, 1), ids.data_ptr(), b.y.data_ptr(), self._p(attn),
                        b.rmax.data_ptr(), b.rlinv.data_ptr(), self._stream())
-            if rowk:
+            if path == "rowk":
                 self._call(self.lib.cast_rowk_ln_ffn_fwd, b.y.data_ptr(), P[pre + "ln2.gamma"].data_ptr(),
                            P[pre + "ln2.beta"].data_ptr(), P[pre + "ffn1.b"].data_ptr(), P[pre + "ffn2.b"].data_ptr(),
                            self.rowk_image(pre), ids.data_ptr(), rate, self.seed, self.step_ptr,
                            block_site(tower, i, 2), block_site(tower, i, 3), c.N, H, 1e-8, b.zn.data_ptr(),
                            b.h1d.data_ptr(), b.xout.data_ptr(), b.mu2.data_ptr(), b.rs2.data_ptr(), self._stream())
-            elif fused:
+            elif path == "fused":
                 self._call(self.lib.cast_ln_ffn_fwd, b.y.data_ptr(), P[pre + "ln2.gamma"].data_ptr(),
                            P[pre + "ln2.beta"].data_ptr(), P[pre + "ffn1.w"].data_ptr(), P[pre + "ffn1.b"].data_ptr(),
                            P[pre + "ffn2.w"].data_ptr(), P[pre + "ffn2.b"].data_ptr(), ids.data_ptr(), rate,
@@ -523,7 +566,7 @@ class Engine:
                 self.linear_fwd(c, b.h1d, self.P[pre + "ffn2.w"], self.P[pre + "ffn2.b"], b.xout, rate=rate,
                                 site=block_site(tower, i, 3), resid=b.zn, ldr=H, row_ids=ids)
             x = b.xout
-        if tower == "main" and train and getattr(c, "fuse_tail", False):
+        if tower == "main" and train and self.fuse_tail:
             tb.x_last = x       # cast_lnf_loss normalises it (and writes tb.out) together with the loss
             return tb.out
         self.ln_fwd(x, tower + ".lnf", tb.out, tb.muf, tb.rsf)
@@ -540,14 +583,11 @@ class Engine:
         t = c.t
         nb = len(tb.blocks)
         x_last = tb.blocks[-1].xout if nb else tb.x_in
-        fused = self.use_fused and bool(self.lib.cast_fused_supported(H))
+        fused = self.block_path != "gemm"
         dx = t[0]
-        if tower == "main" and getattr(c, "fuse_tail", False):
+        if tower == "main" and self.fuse_tail:
             pass                # dx (= t[0]) and the gamma/beta partials were produced by cast_lnf_loss
         elif fused:  # gamma/beta partials of the tower's final LayerNorm join the step's single reduction launch
-            if getattr(tb, "ws_lnf", None) is None:
-                nb_ = self.lib.cast_layernorm_bwd_workspace_bytes(c.N, H)
-                tb.ws_lnf = torch.empty(nb_ // 4 + 16, dtype=torch.float32, device=self.device)
             self._call(self.lib.cast_layernorm_bwd, d_out.data_ptr(), x_last.data_ptr(), tb.muf.data_ptr(),
                        tb.rsf.data_ptr(), self.P[tower + ".lnf.gamma"].data_ptr(), c.N, H, None, dx.data_ptr(), None,
                        None, tb.ws_lnf.data_ptr(), tb.ws_lnf.numel() * 4, self._stream())
@@ -556,13 +596,14 @@ class Engine:
             c.reduce_jobs.append((tb.ws_lnf.data_ptr() + 4 * H, parts, H, self.G[tower + ".lnf.beta"], 2 * H))
         else:
             self.ln_bwd(c, d_out, x_last, tb.muf, tb.rsf, tower + ".lnf", dx)
+        P = self.P
         for i in reversed(range(nb)):
             b = tb.blocks[i]
             pre = f"{tower}.{i}."
             x_i = tb.blocks[i - 1].xout if i > 0 else tb.x_in
             gm, gmd, dh, dzn, dy = t[1], t[2], t[3], t[4], t[5]
+            # x_out = (dropout(h1d W2 + b2) + zn) * mask                      modules.py:304-311, sasrec.py:83
             if fused:
-                P = self.P
                 self._call(self.lib.cast_ffn_bwd, dx.data_ptr(), ids.data_ptr(), b.zn.data_ptr(), b.h1d.data_ptr(),
                            b.y.data_ptr(), b.mu2.data_ptr(), b.rs2.data_ptr(), P[pre + "ln2.gamma"].data_ptr(),
                            P[pre + "ffn1.w"].data_ptr(), P[pre + "ffn2.w"].data_ptr(), rate, self.seed, self.step_ptr,
@@ -571,14 +612,22 @@ class Engine:
                 cnt = 2 * H + 2 * (H * H + H)
                 c.reduce_jobs.append((b.ws_ffn.data_ptr(), self.lib.cast_block_bwd_parts(c.N, 0), cnt,
                                       self.G[pre + "ln2.beta"], cnt))
-                dQ, dK, dV = t[1], t[2], t[3]
-                self._call(self.lib.cast_attn_bwd, b.Q.data_ptr(), H, b.K.data_ptr(), H, b.V.data_ptr(), H,
-                           dy.data_ptr(), b.kmask.data_ptr(), b.qmask.data_ptr(), b.rmax.data_ptr(),
-                           b.rlinv.data_ptr(), ids.data_ptr(), b.rowD.data_ptr(), B, T, H, h, rate, self.seed,
-                           self.step_ptr,
-                           block_site(tower, i, 1), dQ.data_ptr(), H, dK.data_ptr(), H, dV.data_ptr(), H,
-                           b.y.data_ptr(), b.qn.data_ptr(), self._p(c.attn_ws),
-                           c.attn_ws.numel() * 4 if c.attn_ws is not None else 0, self._stream())
+            else:
+                self.mask_dropout(dx, ids, rate, block_site(tower, i, 3), gm, gmd)
+                self.linear_wgrad(c, b.h1d, gmd, self.G[pre + "ffn2.w"], self.G[pre + "ffn2.b"])
+                self.linear_dgrad(c, gmd, self.P[pre + "ffn2.w"], dh, act=b.h1d, ld_act=H, act_scale=scale)
+                self.linear_wgrad(c, b.zn, dh, self.G[pre + "ffn1.w"], self.G[pre + "ffn1.b"])
+                self.linear_dgrad(c, dh, self.P[pre + "ffn1.w"], dzn, resid=gm, ldr=H)
+                self.ln_bwd(c, dzn, b.y, b.mu2, b.rs2, pre + "ln2", dy)
+            # y = attention(Q, K, V) + qn                                      modules.py:262-269
+            dQ, dK, dV = t[1], t[2], t[3]
+            self._call(self.lib.cast_attn_bwd, b.Q.data_ptr(), H, b.K.data_ptr(), H, b.V.data_ptr(), H,
+                       dy.data_ptr(), b.kmask.data_ptr(), b.qmask.data_ptr(), b.rmax.data_ptr(), b.rlinv.data_ptr(),
+                       ids.data_ptr(), b.rowD.data_ptr(), B, T, H, h, rate, self.seed, self.step_ptr,
+                       block_site(tower, i, 1),
+                       dQ.data_ptr(), H, dK.data_ptr(), H, dV.data_ptr(), H, b.y.data_ptr(), b.qn.data_ptr(),
+                       self._p(c.attn_ws), c.attn_ws.numel() * 4 if c.attn_ws is not None else 0, self._stream())
+            if fused:
                 dst = tb.dx_in if i == 0 else t[0]
                 if i == 0 and embed_fx is not None:
                     fx_ids, fx_rate, fx_site, dst = embed_fx
@@ -599,21 +648,6 @@ class Engine:
                                       self.G[pre + "ln1.beta"], cnt))
                 dx = dst
                 continue
-            # x_out = (dropout(h1d W2 + b2) + zn) * mask                      modules.py:304-311, sasrec.py:83
-            self.mask_dropout(dx, ids, rate, block_site(tower, i, 3), gm, gmd)
-            self.linear_wgrad(c, b.h1d, gmd, self.G[pre + "ffn2.w"], self.G[pre + "ffn2.b"])
-            self.linear_dgrad(c, gmd, self.P[pre + "ffn2.w"], dh, act=b.h1d, ld_act=H, act_scale=scale)
-            self.linear_wgrad(c, b.zn, dh, self.G[pre + "ffn1.w"], self.G[pre + "ffn1.b"])
-            self.linear_dgrad(c, dh, self.P[pre + "ffn1.w"], dzn, resid=gm, ldr=H)
-            self.ln_bwd(c, dzn, b.y, b.mu2, b.rs2, pre + "ln2", dy)
-            # y = attention(Q, K, V) + qn                                      modules.py:262-269
-            dQ, dK, dV = t[1], t[2], t[3]
-            self._call(self.lib.cast_attn_bwd, b.Q.data_ptr(), H, b.K.data_ptr(), H, b.V.data_ptr(), H,
-                       dy.data_ptr(), b.kmask.data_ptr(), b.qmask.data_ptr(), b.rmax.data_ptr(), b.rlinv.data_ptr(),
-                       ids.data_ptr(), b.rowD.data_ptr(), B, T, H, h, rate, self.seed, self.step_ptr,
-                       block_site(tower, i, 1),
-                       dQ.data_ptr(), H, dK.data_ptr(), H, dV.data_ptr(), H, b.y.data_ptr(), b.qn.data_ptr(),
-                       self._p(c.attn_ws), c.attn_ws.numel() * 4 if c.attn_ws is not None else 0, self._stream())
             self.linear_wgrad(c, b.qn, dQ, self.G[pre + "q.w"], self.G[pre + "q.b"])
             self.linear_wgrad(c, x_i, dK, self.G[pre + "k.w"], self.G[pre + "k.b"])
             self.linear_wgrad(c, x_i, dV, self.G[pre + "v.w"], self.G[pre + "v.b"])
@@ -666,9 +700,6 @@ class Engine:
         return c.dsrc
 
     # ------------------------------------------------------------------ whole model
-    def rowk_active(self):
-        return self.use_rowk and self.use_fused and bool(self.rowk_block)
-
     def rowk_presplit(self, stream):
         self._call(self.lib.cast_rowk_presplit, self.rowk_wptrs, len(self.rowk_block), self.H,
                    self.rowk_img.data_ptr(), self.rowk_img.numel(), stream)
@@ -680,7 +711,7 @@ class Engine:
         """Builds seq_emb [N,H] from the ids already resident in c.keys3 / c.cids; returns the buffer."""
         plan = self.plan
         ids = c.keys3[0]
-        if self.rowk_active() and not getattr(c, "presplit_pending", False):
+        if self.block_path == "rowk" and "presplit" not in c.forked:
             self.rowk_presplit(self._stream())   # weights moved since the last step: refresh the operand images
         streams: Dict[str, torch.Tensor] = {}
         for j, (tname, key) in enumerate((("time_emb", "time"), ("hours_emb", "hours"), ("days_emb", "days"))):
@@ -703,18 +734,9 @@ class Engine:
         c.seq_emb = x
         return x
 
-    def tail_fusable(self):
-        """final LayerNorm + loss + LayerNorm backward in one launch: the main tower's output must be seq_emb itself"""
-        plan = self.plan
-        return (self.use_fused and bool(self.lib.cast_fused_supported(self.H)) and self.item_shard is None
-                and not (plan.merge and plan.merge[3] == "post"))
-
     def loss_tail_fused(self, c):
         tb = c.tw["main"]
         H, N = self.H, c.N
-        if getattr(c, "ws_tail", None) is None:
-            c.ws_tail = torch.empty(self.lib.cast_lnf_loss_workspace_bytes(N, H) // 4 + 16, dtype=torch.float32,
-                                    device=self.device)
         parts = self.lib.cast_lnf_loss_parts(N)
         self._call(self.lib.cast_lnf_loss, tb.x_last.data_ptr(), self.P["main.lnf.gamma"].data_ptr(),
                    self.P["main.lnf.beta"].data_ptr(), 1e-8, self.P["item_emb"].data_ptr(),
@@ -729,9 +751,6 @@ class Engine:
     def loss_fwd_bwd(self, c, with_grad=True, defer_sums=False):
         ws, ws_bytes, sums = c.ws, c.ws_bytes, c.sums
         if defer_sums:  # the three loss sums join the step's single reduction launch (end of backward)
-            if getattr(c, "ws_loss", None) is None:
-                c.ws_loss = torch.empty(self.lib.cast_logits_loss_workspace_bytes(c.N) // 4 + 16, dtype=torch.float32,
-                                        device=self.device)
             ws, ws_bytes, sums = c.ws_loss, c.ws_loss.numel() * 4, None
             c.reduce_jobs.append((c.ws_loss.data_ptr(), self.lib.cast_logits_loss_parts(c.N), 3, c.sums, 3))
         tail = (c.keys3[1].data_ptr(), c.keys3[2].data_ptr(), c.pos_logits.data_ptr(), c.neg_logits.data_ptr(),
@@ -750,8 +769,6 @@ class Engine:
         plan = self.plan
         ids = c.keys3[0]
         d = c.dseq
-        if getattr(c, "reduce_jobs", None) is None:
-            c.reduce_jobs = []
         dstreams: Dict[str, torch.Tensor] = {}
         if plan.merge and plan.merge[3] == "post":
             ds = self.merge_bwd(c, d)
@@ -760,13 +777,13 @@ class Engine:
         add_time, drop, mask = plan.embed
         pre_merge = bool(plan.merge and plan.merge[3] == "pre")
         # the tower's input is dropout(emb) * mask: block 0's fused backward kernel applies that gradient itself
-        fuse_embed = ((drop or mask) and not pre_merge and self.use_fused and len(c.tw["main"].blocks) > 0
-                      and bool(self.lib.cast_fused_supported(self.H)))
+        fuse_embed = ((drop or mask) and not pre_merge and self.block_path != "gemm"
+                      and len(c.tw["main"].blocks) > 0)
         d = self.tower_bwd(c, "main", d, ids, embed_fx=(ids if mask else None, self.rate if drop else 0.0, SITE_EMBED,
                                                         c.g0) if fuse_embed else None)
         if pre_merge:
-            if plan.merge[4]:  # `seq *= mask` after the MLP (cast_9.py:174): mlp_out is already masked => relu_bwd
-                pass           # zeroes those rows (act == 0)
+            # cast_9's `seq *= mask` after the MLP (cast_9.py:174) needs no backward step: mlp_out is already masked,
+            # so relu_bwd zeroes those rows (act == 0)
             ds = self.merge_bwd(c, d)
             d = ds["seq"]
             dstreams.update({k: v for k, v in ds.items() if k != "seq"})
@@ -780,7 +797,7 @@ class Engine:
             dstreams["time"] = g0
         if plan.learned_pos:
             th = self.T * self.H
-            if self.use_fused and bool(self.lib.cast_fused_supported(self.H)):
+            if self.block_path != "gemm":
                 # d(pos_emb) = sum over the batch of g0 [B, T*H]: another job of the step's reduction launch
                 c.reduce_jobs.append((g0.data_ptr(), c.B, th, self.G["pos_emb"], th))
             else:
@@ -797,22 +814,13 @@ class Engine:
             ctx_scatter.append((j, dk, tname))
         # every deferred partial sum of the step is known now: its one reduction launch runs beside the embedding
         # gradient scatters (independent outputs; a parallel branch of the captured graph), joined before the exchange
-        forked = self.device.type == "cuda" and self.timing is None and bool(c.reduce_jobs)
-        if forked:
-            main = torch.cuda.current_stream(self.device)
-            if getattr(c, "side3", None) is None:
-                c.side3 = torch.cuda.Stream(device=self.device)
-            c.side3.wait_stream(main)
-            with torch.cuda.stream(c.side3):
-                self.flush_reduce_jobs(c)
-        try:
-            self.scatter(c, c.keys3, 3, [g0, c.seq_emb, c.seq_emb], [None, c.gpos, c.gneg], [sq, 1.0, 1.0], "item_emb")
-            for j, dk, tname in ctx_scatter:
-                self.scatter(c, c.cids[j], 1, [dk], [None], [sq], tname)
-        finally:
-            if forked:
-                torch.cuda.current_stream(self.device).wait_stream(c.side3)
-        self.flush_reduce_jobs(c)
+        if c.reduce_jobs:
+            self._fork(c, "reduce", lambda: self.flush_reduce_jobs(c))
+        self.scatter(c, c.keys3, 3, [g0, c.seq_emb, c.seq_emb], [None, c.gpos, c.gneg], [sq, 1.0, 1.0], "item_emb")
+        for j, dk, tname in ctx_scatter:
+            self.scatter(c, c.cids[j], 1, [dk], [None], [sq], tname)
+        self._join(c, "reduce")
+        self.flush_reduce_jobs(c)   # not forked: in stream order
 
     def rank_local(self):
         """context manager: steps launched inside touch no other rank (no barrier, exchange or peer reads) — for
@@ -834,7 +842,6 @@ class Engine:
         jobs = c.reduce_jobs
         if not jobs:
             return
-        import ctypes as C
         n = len(jobs)
         parts = (C.c_void_p * n)(*[int(j[0]) for j in jobs])
         nparts = (C.c_int * n)(*[int(j[1]) for j in jobs])
@@ -863,63 +870,34 @@ class Engine:
         # The sort of the (item id, entry) pairs for the embedding gradient depends on the ids only: it runs on a side
         # stream while the forward pass computes (a parallel branch of the captured CUDA graph) and is joined right
         # before the segment sums at the end of backward.
-        c.presorted = False
-        if self.device.type == "cuda" and self.timing is None:
-            main = torch.cuda.current_stream(self.device)
-            if getattr(c, "side", None) is None:
-                c.side = torch.cuda.Stream(device=self.device)
-            c.side.wait_stream(main)
-            with torch.cuda.stream(c.side):
-                if self.item_shard is not None:
-                    self._call(self.lib.cast_scatter_sort_sharded, c.keys3.data_ptr(), 3, c.N, self.V_items,
-                               self.item_shard[1], self.shard_R, c.sws.data_ptr(), c.sws_bytes, c.side.cuda_stream)
-                else:
-                    V = self.P["item_emb"].shape[0]
-                    self._call(self.lib.cast_scatter_sort, c.keys3.data_ptr(), 3, c.N, V, c.sws.data_ptr(),
-                               c.sws_bytes, c.side.cuda_stream)
-            c.presorted = True
-            if self.rowk_active():   # the weight operand images are needed by the first row kernel, not by the embedding
-                if getattr(c, "side2", None) is None:
-                    c.side2 = torch.cuda.Stream(device=self.device)
-                c.side2.wait_stream(main)
-                with torch.cuda.stream(c.side2):
-                    self.rowk_presplit(c.side2.cuda_stream)
-                c.presplit_pending = True
-        c.reduce_jobs = []
-        c.fuse_tail = self.tail_fusable()
-        bb_forked = False
-        if self.before_backward is not None and self.device.type == "cuda" and self.timing is None:
+        def sort():
+            if self.item_shard is not None:
+                self._call(self.lib.cast_scatter_sort_sharded, c.keys3.data_ptr(), 3, c.N, self.V_items,
+                           self.item_shard[1], self.shard_R, c.sws.data_ptr(), c.sws_bytes, self._stream())
+            else:
+                V = self.P["item_emb"].shape[0]
+                self._call(self.lib.cast_scatter_sort, c.keys3.data_ptr(), 3, c.N, V, c.sws.data_ptr(), c.sws_bytes,
+                           self._stream())
+
+        try:
+            if self._fork(c, "sort", sort) and self.block_path == "rowk":
+                # the weight operand images are needed by the first row kernel, not by the embedding
+                self._fork(c, "presplit", lambda: self.rowk_presplit(self._stream()))
             # "peers have finished reading the previous step's gradients": a flag round trip over NVLink that nothing in
             # the forward pass depends on => a parallel branch of the step, joined before the first gradient write
-            main = torch.cuda.current_stream(self.device)
-            if getattr(c, "side4", None) is None:
-                c.side4 = torch.cuda.Stream(device=self.device)
-            c.side4.wait_stream(main)
-            with torch.cuda.stream(c.side4):
+            if self.before_backward is not None:
+                self._fork(c, "barrier", self.before_backward)
+            self.forward(c, train=True)
+            if self.before_backward is not None and not self._join(c, "barrier"):
                 self.before_backward()
-            bb_forked = True
-        try:
-            try:
-                self.forward(c, train=True)
-            finally:
-                if bb_forked:
-                    torch.cuda.current_stream(self.device).wait_stream(c.side4)
-            if self.before_backward is not None and not bb_forked:
-                self.before_backward()
-            if c.fuse_tail:
+            if self.fuse_tail:
                 self.loss_tail_fused(c)
             else:
                 self.loss_fwd_bwd(c, with_grad=True, defer_sums=True)
             self.backward(c)
-        finally:   # a failed launch must not leave per-step flags (or un-joined side streams) behind: contexts are reused
-            c.fuse_tail = False
-            if getattr(c, "presorted", False) or getattr(c, "presplit_pending", False):
-                main = torch.cuda.current_stream(self.device)
-                if getattr(c, "presorted", False):
-                    main.wait_stream(c.side)
-                if getattr(c, "presplit_pending", False):
-                    main.wait_stream(c.side2)
-                c.presorted = c.presplit_pending = False
+        finally:   # contexts are reused: a failed launch must leave no side branch un-joined and no deferred job behind
+            for name in list(c.forked):
+                self._join(c, name)
             c.reduce_jobs = []
 
     def launch_train_step(self, c):

@@ -113,8 +113,7 @@ def test_fused_and_unfused_paths_agree_at_full_size():
     neg = np.where(seq > 0, rng.randint(1, 301, (B, T)), 0).astype(np.int32)
     outs = []
     for fused in (True, False):
-        eng = Engine("sasrec", 80, 300, args, device=dev, lib=lib, seed=3)
-        eng.use_fused = fused
+        eng = Engine("sasrec", 80, 300, args, device=dev, lib=lib, seed=3, fused=fused)
         g = torch.Generator().manual_seed(5)
         for k in eng.P:
             if k.endswith("beta") or k.endswith(".b"):
