@@ -157,6 +157,13 @@ class Engine:
         self.item_shard = tuple(item_shard) if item_shard is not None and item_shard[1] > 1 else None
         self.V_items = itemnum + 1
         self.shard_R = shard_rows(itemnum, self.item_shard[1]) if self.item_shard else None
+        # the shard map (local_rows / global_ids): row 0 of ranks > 0 is a pad; item_rows = rows of this process's item
+        # table that hold items, counting that pad
+        self.shard_pad = 1 if self.item_shard is not None and self.item_shard[0] > 0 else 0
+        self.item_rows = self.V_items
+        if self.item_shard is not None:
+            rank, world = self.item_shard
+            self.item_rows = (self.V_items - rank + world - 1) // world + self.shard_pad
         self.alloc = alloc
         self.arena = None
         if self.item_shard is not None and alloc is None:
@@ -304,9 +311,25 @@ class Engine:
         rank, world = self.item_shard
         out = torch.zeros((self.shard_R,) + tuple(full.shape[1:]), dtype=full.dtype)
         mine = full[rank::world]
-        off = 1 if rank else 0
-        out[off:off + mine.shape[0]] = mine
+        out[self.shard_pad:self.shard_pad + mine.shape[0]] = mine
         return out
+
+    def local_rows(self, ids: np.ndarray) -> np.ndarray:
+        """global item ids -> rows of this process's item table, 0 where the id is not on this shard (the identity
+        without a row-sharded table).  The map is increasing on the ids a shard holds."""
+        if self.item_shard is None:
+            return ids
+        rank, world = self.item_shard
+        mine = (ids % world == rank) & (ids > 0) & (ids < self.V_items)
+        return np.where(mine, ids // world + self.shard_pad, 0)
+
+    def global_ids(self, rows: torch.Tensor) -> torch.Tensor:
+        """rows of this process's item table -> global item ids, row 0 -> 0 (the inverse of local_rows; the identity
+        without a row-sharded table)"""
+        if self.item_shard is None:
+            return rows
+        rank, world = self.item_shard
+        return torch.where(rows > 0, (rows - self.shard_pad) * world + rank, rows)
 
     def rebind_gradients(self, gbuf: torch.Tensor):
         """move the flat gradient buffer (and every view of it) to `gbuf` — peer-visible memory for data parallelism"""

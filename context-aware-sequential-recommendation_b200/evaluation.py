@@ -143,34 +143,45 @@ def build_recommend_inputs(dataset, args):
             "hours": st(hrs, np.int32), "days": st(dys, np.int32), "tsraw": st(raws, np.int64), "rated": rated}
 
 
-def recommend_users(model, inputs, k: int, batch_users: int = 256, lo: int = 0, hi: Optional[int] = None,
-                    mode: int = 0):
-    """model.recommend over rows [lo, hi) of build_recommend_inputs' output, with each user's history excluded; fixed
-    batch shape (tail padded as in score_users).  Returns (ids [n,k] int32, scores [n,k] float32)."""
-    hi = len(inputs["u"]) if hi is None else hi
-    n_all = max(0, hi - lo)
-    ids = np.zeros((n_all, k), np.int32)
-    scores = np.zeros((n_all, k), np.float32)
-    B = max(1, min(batch_users, max(1, n_all)))
+def _batches(model, rows, batch_users: int, lo: int, hi: int):
+    """Fixed-shape batches over rows [lo, hi) of a build_candidates / build_recommend_inputs dict; the tail batch is
+    padded with zero rows and empty id lists.  Yields (out, pad, feats): the batch's slice of the [hi - lo] results,
+    pad(key) -> the batch of rows[key], and the time-feature keywords of the model call — the raw timestamps
+    (featurised on the device, util.py:276-289) when the model has use_device_time_features and the rows carry them,
+    else the time-bin / hour / weekday id sequences."""
+    B = max(1, min(batch_users, max(1, hi - lo)))
+    use_ts = getattr(model, "timefeat", None) is not None and "tsraw" in rows
     for s in range(lo, hi, B):
         e = min(hi, s + B)
         n = e - s
 
-        def pad(a):
+        def pad(key):
+            a = rows[key]
+            if key == "rated":     # one id collection per user
+                return list(a[s:e]) + [np.zeros(0, np.int32)] * (B - n)
             if n == B:
                 return a[s:e]
             out = np.zeros((B,) + a.shape[1:], a.dtype)
             out[:n] = a[s:e]
             return out
 
-        excl = list(inputs["rated"][s:e]) + [np.zeros(0, np.int32)] * (B - n)
-        if getattr(model, "timefeat", None) is not None:
-            i, sc = model.recommend(pad(inputs["seq"]), k, excl, timestamps=pad(inputs["tsraw"]), mode=mode)
-        else:
-            i, sc = model.recommend(pad(inputs["seq"]), k, excl, pad(inputs["timeseq"]), pad(inputs["hours"]),
-                                    pad(inputs["days"]), mode=mode)
-        ids[s - lo:e - lo] = i[:n]
-        scores[s - lo:e - lo] = sc[:n]
+        feats = ({"timestamps": pad("tsraw")} if use_ts else
+                 {"time_seq": pad("timeseq"), "hours": pad("hours"), "days": pad("days")})
+        yield slice(s - lo, e - lo), pad, feats
+
+
+def recommend_users(model, inputs, k: int, batch_users: int = 256, lo: int = 0, hi: Optional[int] = None,
+                    mode: int = 0):
+    """model.recommend over rows [lo, hi) of build_recommend_inputs' output, with each user's history excluded; fixed
+    batch shape (tail padded as in score_users).  Returns (ids [n,k] int32, scores [n,k] float32)."""
+    hi = len(inputs["u"]) if hi is None else hi
+    ids = np.zeros((max(0, hi - lo), k), np.int32)
+    scores = np.zeros((max(0, hi - lo), k), np.float32)
+    for out, pad, feats in _batches(model, inputs, batch_users, lo, hi):
+        n = out.stop - out.start
+        i, sc = model.recommend(pad("seq"), k, pad("rated"), mode=mode, **feats)
+        ids[out] = i[:n]
+        scores[out] = sc[:n]
     return ids, scores
 
 
@@ -218,35 +229,19 @@ def score_users(model, cand, batch_users: int = 256, lo: int = 0, hi: Optional[i
     user — what the reference collects per user in --test_model mode (util.py:329-336)."""
     hi = len(cand["u"]) if hi is None else hi
     ranks = np.zeros(max(0, hi - lo), np.int64)
-    B = max(1, min(batch_users, max(1, hi - lo)))
-    for s in range(lo, hi, B):
-        e = min(hi, s + B)
-        n = e - s
-
-        def pad(a):
-            if n == B:
-                return a[s:e]
-            out = np.zeros((B,) + a.shape[1:], a.dtype)
-            out[:n] = a[s:e]
-            return out
-
-        if mode == "full":
-            rated = list(cand["rated"][s:e]) + [np.zeros(0, np.int32)] * (B - n)
-            cgt, _ = model.score_full_catalog(pad(cand["seq"]), pad(cand["item_idx"])[:, 0], rated, pad(cand["timeseq"]),
-                                              pad(cand["hours"]), pad(cand["days"]))
-            ranks[s - lo:e - lo] = cgt[:n]
+    for out, pad, feats in _batches(model, cand, batch_users, lo, hi):
+        n = out.stop - out.start
+        seq = pad("seq")
+        if mode == "full":      # score_full_catalog takes the id sequences
+            cgt, _ = model.score_full_catalog(seq, pad("item_idx")[:, 0], pad("rated"), pad("timeseq"), pad("hours"),
+                                              pad("days"))
+            ranks[out] = cgt[:n]
             continue
         want = attn_sum is not None
-        if getattr(model, "timefeat", None) is not None and "tsraw" in cand:
-            # time bins / hours / weekdays derived on the device from the raw event times (util.py:276-289)
-            logits, cgt, ceq = model.score_candidates(pad(cand["seq"]), pad(cand["item_idx"]),
-                                                      timestamps=pad(cand["tsraw"]), want_attn=want)
-        else:
-            logits, cgt, ceq = model.score_candidates(pad(cand["seq"]), pad(cand["item_idx"]), pad(cand["timeseq"]),
-                                                      pad(cand["hours"]), pad(cand["days"]), want_attn=want)
+        logits, cgt, ceq = model.score_candidates(seq, pad("item_idx"), want_attn=want, **feats)
         if want:   # head 0 of user b is row b of the [h*B, T, T] stack (modules.py:208-213)
-            attn_sum += model.engine.ctx(B).attn[:n].sum(0, dtype=attn_sum.dtype)
-        ranks[s - lo:e - lo] = ranks_from_device(logits[:n], cgt[:n], ceq[:n])
+            attn_sum += model.engine.ctx(len(seq)).attn[:n].sum(0, dtype=attn_sum.dtype)
+        ranks[out] = ranks_from_device(logits[:n], cgt[:n], ceq[:n])
     return ranks
 
 

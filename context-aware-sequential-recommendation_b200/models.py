@@ -9,12 +9,28 @@ numpy int arrays as produced by the reference's sampler; results are host floats
 """
 from __future__ import annotations
 
+import ctypes
 from typing import Optional
 
 import numpy as np
 import torch
+import torch.distributed as dist
 
 from .engine import Engine, MODELS
+
+
+def _all_gather(t):
+    """every rank's t, concatenated along dim 0 in rank order"""
+    out = torch.empty((dist.get_world_size() * t.shape[0],) + tuple(t.shape[1:]), dtype=t.dtype, device=t.device)
+    dist.all_gather_into_tensor(out, t)
+    return out
+
+
+def _all_gather_lists(lists):
+    """every rank's per-user id collections, in rank order (None if this rank passes None)"""
+    parts = [None] * dist.get_world_size()
+    dist.all_gather_object(parts, None if lists is None else [sorted(set(int(i) for i in r)) for r in lists])
+    return None if lists is None else [r for p in parts for r in p]
 
 
 class _Model:
@@ -152,96 +168,125 @@ class _Model:
                       eng.P["item_emb"].shape[0], eng.H, B, cand.data_ptr(), Cn, logits.data_ptr(), p(cgt), p(ceq),
                       eng._stream())
 
-    def _id_csr(self, lists, n, local_rows=False):
-        """Per-user id collections -> CSR device tensors (ptr [n+1], idx), ids unique and ascending per user.
-        local_rows=True (row-sharded table): keeps the ids this rank's shard holds, as local rows (id // n_ranks, +1 on
-        ranks > 0) — the map is increasing, so each row stays ascending."""
+    def _id_csr(self, lists, n):
+        """Per-user id collections -> CSR device tensors (ptr [n+1], idx) of rows of this process's item table, unique
+        and ascending per user.  A row-sharded table keeps the ids its shard holds, as local rows (an increasing map,
+        so each row stays ascending)."""
         eng = self.engine
         ptr = np.zeros(n + 1, np.int32)
         flat = []
         for u, r in enumerate(lists):
             ids = np.unique(np.asarray(list(r), dtype=np.int64))
-            if local_rows:
-                rank, world = eng.item_shard
-                ids = ids[(ids % world == rank) & (ids > 0) & (ids < eng.V_items)] // world + (1 if rank else 0)
+            if eng.item_shard is not None:
+                ids = eng.local_rows(ids)
+                ids = ids[ids > 0]
             flat.append(ids)
             ptr[u + 1] = ptr[u] + len(ids)
         idx = np.concatenate(flat + [np.zeros(1, np.int64)]).astype(np.int32)
         return torch.from_numpy(ptr).to(eng.device), torch.from_numpy(idx).to(eng.device)
 
-    def _topk(self, last, ld, U, V, k, eptr, eidx, mode):
-        """cast_topk_full over the rows [0, V) of this process's item table; (ids, scores) [U, k] device tensors"""
-        import ctypes
+    # ------------------------------------------------------------------ full catalog
+    # With a row-sharded item table (SURVEY §8e row 3, config 5) score_full_catalog and recommend are collective calls:
+    # every rank passes its own users (the same count on every rank), the last-position rows of all ranks are
+    # all-gathered, each rank runs the kernel over the items of its own shard and the per-rank results are combined.
+    def _last_rows(self, c):
+        """(rows, ld) of the last position of each sequence of the batch c; with a row-sharded table, of every rank's
+        batch (all-gathered, rank-major)"""
+        eng = self.engine
+        B, T, H = c.B, eng.T, eng.H
+        last = c.seq_emb.view(B, T, H)[:, T - 1, :]
+        if eng.item_shard is None:
+            return last, T * H
+        return _all_gather(last.contiguous()), H
+
+    def _workspace(self, nbytes: int):
+        """device workspace of the full-catalog kernels: one buffer, grown on demand (the operand images of a large
+        catalog are GBs)"""
+        ws = self._pinned.get("catalog_ws")
+        if ws is None or ws.numel() * 4 < nbytes:
+            self._pinned["catalog_ws"] = None
+            ws = self._pinned["catalog_ws"] = torch.empty(nbytes // 4 + 16, dtype=torch.int32, device=self.engine.device)
+        return ws
+
+    def _check_watchdog(self, status, what, *args):
+        """status(*args, &flag, stream) reads the watchdog flag of a mode-0 call's tensor-core pass; raises if it fired"""
+        eng = self.engine
+        flag = ctypes.c_int(0)
+        eng._call(status, *args, ctypes.byref(flag), eng._stream())
+        if flag.value != 0:
+            raise RuntimeError(f"{what}: tensor-core pass watchdog fired")
+
+    def score_full_catalog(self, seq, target, rated=None, time_seq=None, hours=None, days=None, mode: int = 0):
+        """Full-catalog evaluation scoring: rank of target[u] among every item in [1, itemnum] the user has not
+        rated (rated: optional list of id collections, one per user).  mode 0 = tcgen05 tensor-core GEMM with exact
+        band re-scoring, mode 1 = exact brute force.  Returns (count_greater [U], count_equal [U]) int32 arrays.
+        With a row-sharded item table each rank counts the items of its own shard that beat the target (whose
+        canonical score is gathered from the owning shard) and one integer all-reduce adds the counts up."""
         eng = self.engine
         dev = eng.device
-        table = eng.P["item_emb"]
-        ids = torch.empty(U, k, dtype=torch.int32, device=dev)
-        scores = torch.empty(U, k, dtype=torch.float32, device=dev)
-        wsb = eng.lib.cast_topk_full_workspace_bytes(U, V, eng.H, k)
-        ws = self._pinned.get("tkws")     # one buffer, grown on demand (the operand images of a large catalog are GBs)
-        if ws is None or ws.numel() * 4 < wsb:
-            self._pinned["tkws"] = None
-            ws = self._pinned["tkws"] = torch.empty(wsb // 4 + 16, dtype=torch.int32, device=dev)
-        eng._call(eng.lib.cast_topk_full, last.data_ptr(), ld, table.data_ptr(), V, eng.H, U, k, eng._p(eptr),
-                  eng._p(eidx), mode, ids.data_ptr(), scores.data_ptr(), None, ws.data_ptr(), wsb, eng._stream())
-        if mode == 0:
-            flag = ctypes.c_int(0)
-            eng._call(eng.lib.cast_topk_full_status, ws.data_ptr(), U, V, eng.H, k, ctypes.byref(flag), eng._stream())
-            if flag.value != 0:
-                raise RuntimeError("topk_full: tensor-core pass watchdog fired")
-        return ids, scores
+        c = self.forward_eval(seq, time_seq, hours, days)
+        last, ld = self._last_rows(c)
+        U, V = last.shape[0], eng.item_rows
+        tgt = torch.from_numpy(np.ascontiguousarray(np.asarray(target, dtype=np.int32).reshape(-1))).to(dev)
+        tscore = None
+        if eng.item_shard is not None:
+            tgt = _all_gather(tgt)
+            rated = _all_gather_lists(rated)
+            tscore = torch.empty(U, 1, dtype=torch.float32, device=dev)
+            self._score_cand(last, ld, U, tgt.view(U, 1), 1, tscore)
+            tgt = torch.from_numpy(eng.local_rows(tgt.cpu().numpy().astype(np.int64)).astype(np.int32)).to(dev)
+        cgt = torch.zeros(U, dtype=torch.int32, device=dev)
+        ceq = torch.zeros(U, dtype=torch.int32, device=dev)
+        if V > 1:       # a shard of a catalog smaller than the world may hold no item
+            rptr, ridx = self._id_csr(rated, U) if rated is not None else (None, None)
+            wsb = eng.lib.cast_score_rank_full_workspace_bytes(U, V, eng.H)
+            ws = self._workspace(wsb)
+            eng._call(eng.lib.cast_score_rank_full, last.data_ptr(), ld, eng.P["item_emb"].data_ptr(), V, eng.H, U,
+                      tgt.data_ptr(), eng._p(tscore), eng._p(rptr), eng._p(ridx), mode, cgt.data_ptr(), ceq.data_ptr(),
+                      None, ws.data_ptr(), wsb, eng._stream())
+            if mode == 0:
+                self._check_watchdog(eng.lib.cast_score_rank_full_status, "score_rank_full", ws.data_ptr(), U, V)
+        if eng.item_shard is None:
+            return cgt.cpu().numpy(), ceq.cpu().numpy()
+        rank = eng.item_shard[0]
+        both = torch.stack([cgt, ceq])
+        dist.all_reduce(both, op=dist.ReduceOp.SUM)
+        mine = slice(rank * c.B, (rank + 1) * c.B)
+        return both[0, mine].cpu().numpy(), both[1, mine].cpu().numpy()
 
     def recommend(self, seq, k=10, exclude=None, time_seq=None, hours=None, days=None, timestamps=None, mode: int = 0):
         """Exact top-k recommendation from the last position of each sequence: the k items of [1, itemnum] not in
         exclude[u] (optional, one id collection per user) with the largest canonical fp32 logits (the logits of
         score_candidates / predict), ties broken by item id ascending.  mode 0 = tcgen05 tensor cores as an exact
         filter, mode 1 = exact brute force; both return the same bits.  Returns (ids [U,k] int32, scores [U,k] float32);
-        fewer than k eligible items pad the tail with id 0 and score -inf.  With a row-sharded item table this is a
-        collective call (every rank passes its own users, the same count on every rank)."""
+        fewer than k eligible items pad the tail with id 0 and score -inf.  With a row-sharded item table each rank
+        takes the top k of its own shard (local rows -> global ids, an increasing map, so the tie order holds) and the
+        ranks' lists are merged per user by (score desc, id asc)."""
         eng = self.engine
-        if eng.item_shard is not None:
-            return self._recommend_sharded(seq, k, exclude, time_seq, hours, days, timestamps, mode)
-        c = self.forward_eval(seq, time_seq, hours, days, timestamps=timestamps)
-        B, T, H = c.B, eng.T, eng.H
-        eptr, eidx = self._id_csr(exclude, B) if exclude is not None else (None, None)
-        last = c.seq_emb.view(B, T, H)[:, T - 1, :]
-        ids, scores = self._topk(last, T * H, B, eng.P["item_emb"].shape[0], k, eptr, eidx, mode)
-        return ids.cpu().numpy(), scores.cpu().numpy()
-
-    def _recommend_sharded(self, seq, k, exclude, time_seq, hours, days, timestamps, mode):
-        """Top-k with the item table sharded by row: the last-position vectors of all ranks are all-gathered, each rank
-        takes the top k of its own shard (local rows -> global ids, an increasing map, so the tie order holds), the
-        [U, k] lists are all-gathered and merged per user by (score desc, id asc)."""
-        import torch.distributed as dist
-        eng = self.engine
-        rank, world = eng.item_shard
         dev = eng.device
         c = self.forward_eval(seq, time_seq, hours, days, timestamps=timestamps)
-        B, T, H = c.B, eng.T, eng.H
-        last = c.seq_emb.view(B, T, H)[:, T - 1, :].contiguous()
-        U = B * world
-        last_all = torch.empty(U, H, dtype=torch.float32, device=dev)
-        dist.all_gather_into_tensor(last_all, last)
-        excl_all = [None] * world
-        dist.all_gather_object(excl_all, None if exclude is None else [sorted(set(int(i) for i in r)) for r in exclude])
-        off = 1 if rank else 0
-        v_loc = (eng.V_items - rank + world - 1) // world + off      # rows of this shard that hold items (+ the pad)
+        last, ld = self._last_rows(c)
+        U, V = last.shape[0], eng.item_rows
+        if eng.item_shard is not None:
+            exclude = _all_gather_lists(exclude)
         ids = torch.zeros(U, k, dtype=torch.int32, device=dev)
         scores = torch.full((U, k), float("-inf"), dtype=torch.float32, device=dev)
-        if v_loc > 1:
-            eptr = eidx = None
-            if excl_all[0] is not None:
-                eptr, eidx = self._id_csr([r for rl in excl_all for r in rl], U, local_rows=True)
-            rows, scores = self._topk(last_all, H, U, v_loc, k, eptr, eidx, mode)
-            ids = torch.where(rows > 0, (rows - off) * world + rank, rows)
-        parts_i = [torch.empty_like(ids) for _ in range(world)]
-        parts_s = [torch.empty_like(scores) for _ in range(world)]
-        dist.all_gather(parts_i, ids)
-        dist.all_gather(parts_s, scores)
-        all_i = np.concatenate([t.cpu().numpy() for t in parts_i], 1)
-        all_s = np.concatenate([t.cpu().numpy() for t in parts_s], 1)
+        if V > 1:       # a shard of a catalog smaller than the world may hold no item
+            eptr, eidx = self._id_csr(exclude, U) if exclude is not None else (None, None)
+            wsb = eng.lib.cast_topk_full_workspace_bytes(U, V, eng.H, k)
+            ws = self._workspace(wsb)
+            eng._call(eng.lib.cast_topk_full, last.data_ptr(), ld, eng.P["item_emb"].data_ptr(), V, eng.H, U, k,
+                      eng._p(eptr), eng._p(eidx), mode, ids.data_ptr(), scores.data_ptr(), None, ws.data_ptr(), wsb,
+                      eng._stream())
+            if mode == 0:
+                self._check_watchdog(eng.lib.cast_topk_full_status, "topk_full", ws.data_ptr(), U, V, eng.H, k)
+            ids = eng.global_ids(ids)
+        if eng.item_shard is None:
+            return ids.cpu().numpy(), scores.cpu().numpy()
+        rank, world = eng.item_shard
+        all_i, all_s = (np.hstack(np.split(_all_gather(t).cpu().numpy(), world)) for t in (ids, scores))
         order = np.lexsort((all_i, -all_s), axis=-1)[:, :k]
-        mine = slice(rank * B, (rank + 1) * B)
+        mine = slice(rank * c.B, (rank + 1) * c.B)
         return np.take_along_axis(all_i, order, 1)[mine], np.take_along_axis(all_s, order, 1)[mine]
 
     # ------------------------------------------------------------------ reference protocol
@@ -342,90 +387,6 @@ class _Model:
         last = c.seq_emb.view(B, T, H)[:, T - 1, :]
         self._score_cand(last, T * H, B, cand_t, Cn, logits, cgt, ceq)
         return logits.cpu().numpy(), cgt.cpu().numpy(), ceq.cpu().numpy()
-
-    def score_full_catalog(self, seq, target, rated=None, time_seq=None, hours=None, days=None, mode: int = 0):
-        """Full-catalog evaluation scoring: rank of target[u] among every item in [1, itemnum] the user has not
-        rated (rated: optional list of id collections, one per user).  mode 0 = tcgen05 tensor-core GEMM with exact
-        band re-scoring, mode 1 = exact brute force.  Returns (count_greater [U], count_equal [U]) int32 arrays."""
-        eng = self.engine
-        if eng.item_shard is not None:
-            return self._score_full_catalog_sharded(seq, target, rated, time_seq, hours, days, mode)
-        c = self.forward_eval(seq, time_seq, hours, days)
-        B, T, H = c.B, eng.T, eng.H
-        dev = eng.device
-        V = eng.P["item_emb"].shape[0]
-        tgt = torch.from_numpy(np.ascontiguousarray(np.asarray(target, dtype=np.int32).reshape(-1))).to(dev)
-        rptr, ridx = self._id_csr(rated, B) if rated is not None else (None, None)
-        cgt = torch.empty(B, dtype=torch.int32, device=dev)
-        ceq = torch.empty(B, dtype=torch.int32, device=dev)
-        wsb = eng.lib.cast_score_rank_full_workspace_bytes(B, V, H)
-        ws = self._pinned.get(("sfws", B))
-        if ws is None:
-            ws = self._pinned[("sfws", B)] = torch.empty(wsb // 4 + 16, dtype=torch.int32, device=dev)
-        last = c.seq_emb.view(B, T, H)[:, T - 1, :]
-        eng._call(eng.lib.cast_score_rank_full, last.data_ptr(), T * H, eng.P["item_emb"].data_ptr(), V, H, B,
-                  tgt.data_ptr(), None, eng._p(rptr), eng._p(ridx), mode, cgt.data_ptr(), ceq.data_ptr(), None,
-                  ws.data_ptr(), wsb, eng._stream())
-        if mode == 0:
-            import ctypes
-            flag = ctypes.c_int(0)
-            eng._call(eng.lib.cast_score_rank_full_status, ws.data_ptr(), B, V, ctypes.byref(flag), eng._stream())
-            if flag.value != 0:
-                raise RuntimeError("score_rank_full: tensor-core pass watchdog fired")
-        return cgt.cpu().numpy(), ceq.cpu().numpy()
-
-    def _score_full_catalog_sharded(self, seq, target, rated, time_seq, hours, days, mode):
-        """Full-catalog ranks with the item table sharded by row (SURVEY §8e row 3, config 5): every rank runs the
-        forward pass for ITS users, the last-position vectors of all ranks are all-gathered, each rank counts — on the
-        tensor cores — the items of its own shard that beat the target (whose canonical score is gathered from the
-        owning shard), and ONE integer all-reduce adds the per-shard counts up.  Collective: all ranks call it with
-        their own users (same count on every rank)."""
-        import torch.distributed as dist
-        eng = self.engine
-        rank, world = eng.item_shard
-        dev = eng.device
-        c = self.forward_eval(seq, time_seq, hours, days)
-        B, T, H = c.B, eng.T, eng.H
-        last = c.seq_emb.view(B, T, H)[:, T - 1, :].contiguous()
-        tgt_loc = torch.from_numpy(np.ascontiguousarray(np.asarray(target, dtype=np.int32).reshape(-1))).to(dev)
-        U = B * world
-        last_all = torch.empty(U, H, dtype=torch.float32, device=dev)
-        tgt_all = torch.empty(U, dtype=torch.int32, device=dev)
-        dist.all_gather_into_tensor(last_all, last)
-        dist.all_gather_into_tensor(tgt_all, tgt_loc)
-        rated_all = [None] * world
-        dist.all_gather_object(rated_all, None if rated is None else [sorted(set(int(i) for i in r)) for r in rated])
-        # canonical target scores: one gather from the owning shards
-        tscore = torch.empty(U, 1, dtype=torch.float32, device=dev)
-        self._score_cand(last_all, H, U, tgt_all.view(U, 1), 1, tscore)
-        # this shard's view: local row of the target (0 = not here), local rows of the rated items
-        tg = tgt_all.cpu().numpy().astype(np.int64)
-        off = 1 if rank else 0
-        tl = np.where((tg % world == rank) & (tg > 0) & (tg < eng.V_items), tg // world + off, 0).astype(np.int32)
-        rptr = ridx = None
-        if rated is not None:
-            rptr, ridx = self._id_csr([r for rl in rated_all for r in rl], U, local_rows=True)
-        v_loc = (eng.V_items - rank + world - 1) // world + off      # rows of this shard that hold items (+ the pad)
-        cgt = torch.zeros(U, dtype=torch.int32, device=dev)
-        ceq = torch.zeros(U, dtype=torch.int32, device=dev)
-        if v_loc > 1:
-            wsb = eng.lib.cast_score_rank_full_workspace_bytes(U, v_loc, H)
-            ws = self._pinned.get(("sfws", U))
-            if ws is None:
-                ws = self._pinned[("sfws", U)] = torch.empty(wsb // 4 + 16, dtype=torch.int32, device=dev)
-            eng._call(eng.lib.cast_score_rank_full, last_all.data_ptr(), H, eng.P["item_emb"].data_ptr(), v_loc, H, U,
-                      torch.from_numpy(tl).to(dev).data_ptr(), tscore.data_ptr(), eng._p(rptr), eng._p(ridx), mode,
-                      cgt.data_ptr(), ceq.data_ptr(), None, ws.data_ptr(), wsb, eng._stream())
-            if mode == 0 and dev.type == "cuda":
-                import ctypes
-                flag = ctypes.c_int(0)
-                eng._call(eng.lib.cast_score_rank_full_status, ws.data_ptr(), U, v_loc, ctypes.byref(flag), eng._stream())
-                if flag.value != 0:
-                    raise RuntimeError("score_rank_full: tensor-core pass watchdog fired")
-        both = torch.stack([cgt, ceq])
-        dist.all_reduce(both, op=dist.ReduceOp.SUM)
-        mine = slice(rank * B, (rank + 1) * B)
-        return both[0, mine].cpu().numpy(), both[1, mine].cpu().numpy()
 
     # parameter access by role name
     def state_dict(self):
