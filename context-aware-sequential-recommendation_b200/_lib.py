@@ -78,6 +78,13 @@ SIGNATURES = {
     "cast_adam_tf_step": (I, [P, P, P, P, L, F, F, F, F, P, F, L, L, P, P]),
     "cast_adam_tf_range": (I, [P, P, P, P, L, F, F, F, F, P, F, L, L, P, I, P]),
     "cast_adam_tf_step_peers": (I, [P, P, I, P, P, P, L, L, F, F, F, F, F, L, L, P, P]),
+    "cast_grad_epoch_advance": (I, [P, P]),
+    "cast_adam_tf_rows": (I, [P, P, P, P, L, I, F, F, F, F, P, P, P, P, P]),
+    "cast_adam_tf_rows_peers": (I, [P, P, P, P, I, P, P, L, I, L, F, F, F, F, P, P]),
+    "cast_adam_tf_range_peers": (I, [P, P, I, P, P, P, L, L, L, F, F, F, F, P, P]),
+    "cast_scatter_apply_lazy": (I, [I, L, P, P, P, I, I, P, P, SZ, P, SZ, P, P, P]),
+    "cast_scatter_apply_range_lazy": (I, [I, L, P, P, P, I, P, P, P, C.c_uint, C.c_uint, P, SZ, P, P, P]),
+    "cast_scatter_pull_range_lazy": (I, [I, L, P, P, P, I, P, P, P, C.c_uint, C.c_uint, P, SZ, P, SZ, P, P, P]),
     "cast_score_rank_cand": (I, [P, L, P, I, I, L, P, I, P, P, P, P]),
     "cast_score_rank_full_workspace_bytes": (SZ, [L, I, I]),
     "cast_score_rank_full": (I, [P, L, P, I, I, L, P, P, P, P, I, P, P, P, P, SZ, P]),

@@ -81,7 +81,7 @@ __global__ void adam_step_vec4_kernel(float4* __restrict__ w, const float4* __re
 constexpr int ADAM_PEER_BATCH = 8;
 __global__ void adam_step_peers_kernel(float* __restrict__ w, const float* const* __restrict__ g, int n,
                                        float* __restrict__ g_red, float* __restrict__ m, float* __restrict__ v,
-                                       long np, long tail, float lr, float b1, float b2, float eps, float l2,
+                                       long lo, long np, long tail, float lr, float b1, float b2, float eps, float l2,
                                        long l2_lo, long l2_hi, const AdamState* __restrict__ st) {
   __shared__ float s_count;
   cast_pdl_wait();
@@ -96,10 +96,14 @@ __global__ void adam_step_peers_kernel(float* __restrict__ w, const float* const
   const float lr_t = lr * sqrtf(1.0f - st->b2p) / (1.0f - st->b1p);
   const float omb1 = 1.0f - b1, omb2 = 1.0f - b2;
   const long total = np + tail;
-  for (long i0 = 4 * ((long)blockIdx.x * blockDim.x + threadIdx.x); i0 < total; i0 += 4 * (long)gridDim.x * blockDim.x) {
+  // elements below `lo` are neither reduced nor updated (lo = 0 but for the lazy optimizer, whose row pass owns them);
+  // groups of 4 stay aligned to the buffers, the one that straddles `lo` goes element by element
+  for (long i0 = (lo & ~3L) + 4 * ((long)blockIdx.x * blockDim.x + threadIdx.x); i0 < total;
+       i0 += 4 * (long)gridDim.x * blockDim.x) {
     float gv[4] = {0.f, 0.f, 0.f, 0.f};
     const int cnt = total - i0 < 4 ? (int)(total - i0) : 4;
-    if (cnt == 4) {
+    const int e0 = i0 < lo ? (int)(lo - i0) : 0;
+    if (cnt == 4 && e0 == 0) {
       for (int r0 = 0; r0 < n; r0 += ADAM_PEER_BATCH) {
         float4 q[ADAM_PEER_BATCH];
 #pragma unroll
@@ -117,7 +121,7 @@ __global__ void adam_step_peers_kernel(float* __restrict__ w, const float* const
       }
       *reinterpret_cast<float4*>(g_red + i0) = make_float4(gv[0], gv[1], gv[2], gv[3]);
     } else {
-      for (int e = 0; e < cnt; ++e) {
+      for (int e = e0; e < cnt; ++e) {
         float sacc = g[0][i0 + e];
         for (int r = 1; r < n; ++r) sacc += g[r][i0 + e];
         gv[e] = sacc;
@@ -125,7 +129,7 @@ __global__ void adam_step_peers_kernel(float* __restrict__ w, const float* const
       }
     }
     const int na = np - i0 >= 4 ? 4 : (np - i0 > 0 ? (int)(np - i0) : 0);  // elements of this group that are parameters
-    if (na == 4) {
+    if (na == 4 && e0 == 0) {
       const float4 wi = *reinterpret_cast<const float4*>(w + i0), mi = *reinterpret_cast<const float4*>(m + i0),
                    vi = *reinterpret_cast<const float4*>(v + i0);
       float wv[4] = {wi.x, wi.y, wi.z, wi.w}, mv[4] = {mi.x, mi.y, mi.z, mi.w}, vv[4] = {vi.x, vi.y, vi.z, vi.w};
@@ -138,7 +142,7 @@ __global__ void adam_step_peers_kernel(float* __restrict__ w, const float* const
       *reinterpret_cast<float4*>(v + i0) = make_float4(vv[0], vv[1], vv[2], vv[3]);
       *reinterpret_cast<float4*>(w + i0) = make_float4(wv[0], wv[1], wv[2], wv[3]);
     } else {
-      for (int e = 0; e < na; ++e) {
+      for (int e = e0; e < na; ++e) {
         const long idx = i0 + e;
         float wi = w[idx], mi = m[idx], vi = v[idx];
         adam_elem(wi, mi, vi, gv[e] * gs, idx >= l2_lo && idx < l2_hi, l2, b1, omb1, b2, omb2, lr_t, eps);
@@ -148,6 +152,125 @@ __global__ void adam_step_peers_kernel(float* __restrict__ w, const float* const
       }
     }
   }
+}
+
+// ---- lazy TF-Adam (optimizer "lazy_adam", tf.contrib.opt.LazyAdamOptimizer on the item table)
+// A table row is updated iff this backward pass wrote its gradient (stamp[r] == *epoch, see cast_scatter_apply_lazy);
+// every other row keeps w, m and v bit for bit.  The element arithmetic is adam_elem with the dense pass's lr_t and
+// 1/count, so a touched row gets exactly the bits the dense kernel would give it.  One warp per `rpw` <= 32 consecutive
+// rows: the lanes read the rpw stamps at once, then the warp updates the touched rows one by one, lanes over columns.
+// rpw is 32 for a large table (one coalesced stamp read per 32 rows) and shrinks until a small table still gives every
+// SM warps to run (rows_per_warp).
+__global__ void grad_epoch_advance_kernel(unsigned* epoch) {
+  cast_pdl_wait();
+  cast_pdl_trigger();
+  if (threadIdx.x == 0 && blockIdx.x == 0) *epoch += 1u;
+}
+
+__device__ __forceinline__ void adam_row(float* __restrict__ w, float* __restrict__ m, float* __restrict__ v,
+                                         const float* __restrict__ g, int H, bool vec, float gs, float b1, float omb1,
+                                         float b2, float omb2, float lr_t, float eps, int lane) {
+  if (vec) {
+    for (int c = 4 * lane; c < H; c += 128) {
+      const float4 wi = *reinterpret_cast<const float4*>(w + c), gi = *reinterpret_cast<const float4*>(g + c),
+                   mi = *reinterpret_cast<const float4*>(m + c), vi = *reinterpret_cast<const float4*>(v + c);
+      float wv[4] = {wi.x, wi.y, wi.z, wi.w}, gv[4] = {gi.x, gi.y, gi.z, gi.w};
+      float mv[4] = {mi.x, mi.y, mi.z, mi.w}, vv[4] = {vi.x, vi.y, vi.z, vi.w};
+#pragma unroll
+      for (int e = 0; e < 4; ++e) adam_elem(wv[e], mv[e], vv[e], gv[e] * gs, false, 0.f, b1, omb1, b2, omb2, lr_t, eps);
+      *reinterpret_cast<float4*>(m + c) = make_float4(mv[0], mv[1], mv[2], mv[3]);
+      *reinterpret_cast<float4*>(v + c) = make_float4(vv[0], vv[1], vv[2], vv[3]);
+      *reinterpret_cast<float4*>(w + c) = make_float4(wv[0], wv[1], wv[2], wv[3]);
+    }
+  } else {
+    for (int c = lane; c < H; c += 32) {
+      float wi = w[c], mi = m[c], vi = v[c];
+      adam_elem(wi, mi, vi, g[c] * gs, false, 0.f, b1, omb1, b2, omb2, lr_t, eps);
+      m[c] = mi;
+      v[c] = vi;
+      w[c] = wi;
+    }
+  }
+}
+
+__global__ void adam_rows_kernel(float* __restrict__ w, const float* __restrict__ grad, float* __restrict__ m,
+                                 float* __restrict__ v, long rows, int rpw, int H, int vec, float lr, float b1, float b2,
+                                 float eps, const float* __restrict__ gdenom, const unsigned* __restrict__ stamp,
+                                 const unsigned* __restrict__ epoch, const AdamState* __restrict__ st) {
+  cast_pdl_wait();
+  cast_pdl_trigger();
+  const float gs = gdenom ? 1.0f / *gdenom : 1.0f;
+  const float lr_t = lr * sqrtf(1.0f - st->b2p) / (1.0f - st->b1p);
+  const float omb1 = 1.0f - b1, omb2 = 1.0f - b2;
+  const unsigned ep = *epoch;
+  const int lane = threadIdx.x & 31;
+  const long nwarps = (long)gridDim.x * (blockDim.x >> 5);
+  for (long r0 = rpw * ((long)blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5)); r0 < rows; r0 += rpw * nwarps) {
+    const long r = r0 + lane;
+    unsigned todo = __ballot_sync(0xffffffffu, lane < rpw && r > 0 && r < rows && stamp[r] == ep);
+    while (todo) {
+      const long q = r0 + __ffs((int)todo) - 1;
+      todo &= todo - 1u;
+      const long o = q * H;
+      adam_row(w + o, m + o, v + o, grad + o, H, vec, gs, b1, omb1, b2, omb2, lr_t, eps, lane);
+    }
+  }
+}
+
+// replicated data parallelism: row r's gradient is the rank-ordered sum over the ranks that touched it (stamps[q][r] ==
+// *epochs[q], each rank against its own counter) with +0 for the others — what the dense peer pass reads from a rank
+// whose zeroed row the batch missed — and the denominator is the rank-ordered sum of the ranks' counts (grads[q][np+2])
+constexpr int ADAM_MAX_RANKS = 32;
+__global__ void adam_rows_peers_kernel(float* __restrict__ w, const float* const* __restrict__ g,
+                                       const unsigned* const* __restrict__ stamps,
+                                       const unsigned* const* __restrict__ epochs, int n, float* __restrict__ m,
+                                       float* __restrict__ v, long rows, int rpw, int H, long np, float lr, float b1,
+                                       float b2,
+                                       float eps, const AdamState* __restrict__ st) {
+  __shared__ float s_count;
+  cast_pdl_wait();
+  cast_pdl_trigger();
+  if (threadIdx.x == 0) {
+    float c = g[0][np + 2];
+    for (int q = 1; q < n; ++q) c += g[q][np + 2];
+    s_count = c;
+  }
+  __syncthreads();
+  const float gs = 1.0f / s_count;
+  const float lr_t = lr * sqrtf(1.0f - st->b2p) / (1.0f - st->b1p);
+  const float omb1 = 1.0f - b1, omb2 = 1.0f - b2;
+  const int lane = threadIdx.x & 31;
+  const long nwarps = (long)gridDim.x * (blockDim.x >> 5);
+  for (long r0 = rpw * ((long)blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5)); r0 < rows; r0 += rpw * nwarps) {
+    const long r = r0 + lane;
+    unsigned mine = 0u;        // ranks that touched row r (bit q)
+    if (lane < rpw && r > 0 && r < rows)
+      for (int q = 0; q < n; ++q) mine |= (stamps[q][r] == *epochs[q] ? 1u : 0u) << q;
+    unsigned todo = __ballot_sync(0xffffffffu, mine != 0u);
+    while (todo) {
+      const int l = __ffs((int)todo) - 1;
+      todo &= todo - 1u;
+      const long o = (r0 + l) * H;
+      const unsigned who = __shfl_sync(0xffffffffu, mine, l);
+      for (int c = lane; c < H; c += 32) {
+        float gsum = (who & 1u) ? g[0][o + c] : 0.f;
+        for (int q = 1; q < n; ++q) gsum += ((who >> q) & 1u) ? g[q][o + c] : 0.f;
+        float wi = w[o + c], mi = m[o + c], vi = v[o + c];
+        adam_elem(wi, mi, vi, gsum * gs, false, 0.f, b1, omb1, b2, omb2, lr_t, eps);
+        m[o + c] = mi;
+        v[o + c] = vi;
+        w[o + c] = wi;
+      }
+    }
+  }
+}
+
+// rows scanned per warp of the lazy row pass: 32 unless that leaves fewer than 32 warps per SM (148 SMs)
+static inline int rows_per_warp(long rows) {
+  const long per = rows / (148L * 32);
+  int rpw = 1;
+  while (rpw < 32 && rpw < per) rpw <<= 1;
+  return rpw;
 }
 
 __global__ void adam_advance_kernel(AdamState* st, float b1, float b2) {
@@ -221,11 +344,78 @@ extern "C" int cast_adam_tf_step_peers(float* w, const void* const* grads, int n
   long g = cdiv(cdiv(n + tail, 4), 256);
   if (g > 148 * 8) g = 148 * 8;
   CAST_LAUNCH_DEP(adam_step_peers_kernel, dim3((unsigned)g), dim3(256), 0, (cudaStream_t)stream, w,
-              reinterpret_cast<const float* const*>(grads), n_ranks, g_red, m, v, n, tail, lr, beta1, beta2, eps, l2,
-              l2_lo, l2_hi, static_cast<const AdamState*>(state));
+              reinterpret_cast<const float* const*>(grads), n_ranks, g_red, m, v, 0L, n, tail, lr, beta1, beta2, eps,
+              l2, l2_lo, l2_hi, static_cast<const AdamState*>(state));
   int rc;
   if ((rc = check_launch("adam_step_peers"))) return rc;
   CAST_LAUNCH_DEP(adam_advance_kernel, dim3(1), dim3(32), 0, (cudaStream_t)stream, static_cast<AdamState*>(state), beta1,
               beta2);
+  return check_launch("adam_advance");
+}
+
+/* One-thread kernel: the next backward pass's gradient epoch (*epoch += 1).  The counter is never rewound, so a
+ * stamp left by any earlier pass (an eager warm-up, a rewound optimizer state) can never look current. */
+extern "C" int cast_grad_epoch_advance(unsigned* epoch, void* stream) {
+  if (!epoch) return set_error(CAST_ERR_BAD_ARG, "grad_epoch_advance");
+  CAST_LAUNCH_DEP(grad_epoch_advance_kernel, dim3(1), dim3(32), 0, (cudaStream_t)stream, epoch);
+  return check_launch("grad_epoch_advance");
+}
+
+/* Lazy TF-Adam over a row table [rows, H] (the item table or this rank's shard of it): updates row r only if
+ * stamp[r] == *epoch (its gradient was written in this backward pass); row 0 never.  Does not advance the beta
+ * powers: the caller's cast_adam_tf_range over the dense remainder does, once. */
+extern "C" int cast_adam_tf_rows(float* w, const float* grad, float* m, float* v, long rows, int H, float lr,
+                                 float beta1, float beta2, float eps, const float* gdenom, const unsigned* stamp,
+                                 const unsigned* epoch, void* state, void* stream) {
+  if (!w || !grad || !m || !v || !stamp || !epoch || !state || rows <= 0 || H <= 0)
+    return set_error(CAST_ERR_BAD_ARG, "adam_tf_rows");
+  const int vec = (H % 4 == 0) && ((((uintptr_t)w | (uintptr_t)grad | (uintptr_t)m | (uintptr_t)v) & 15) == 0);
+  const int rpw = rows_per_warp(rows);
+  long g = cdiv(cdiv(rows, rpw), 8);
+  if (g > 148 * 8) g = 148 * 8;
+  CAST_LAUNCH_DEP(adam_rows_kernel, dim3((unsigned)g), dim3(256), 0, (cudaStream_t)stream, w, grad, m, v, rows, rpw, H,
+                  vec,
+                  lr, beta1, beta2, eps, gdenom, stamp, epoch, static_cast<const AdamState*>(state));
+  return check_launch("adam_rows");
+}
+
+/* cast_adam_tf_rows under replicated data parallelism: grads / stamps / epochs are DEVICE arrays of n_ranks pointers
+ * (own buffer + peer mappings; grads as for cast_adam_tf_step_peers, np = parameter count before the tail sums).  Row
+ * r is updated if any rank touched it, with the rank-ordered sum of the touching ranks' rows.  No advance. */
+extern "C" int cast_adam_tf_rows_peers(float* w, const void* const* grads, const void* const* stamps,
+                                       const void* const* epochs, int n_ranks, float* m, float* v, long rows, int H,
+                                       long np, float lr, float beta1, float beta2, float eps, void* state,
+                                       void* stream) {
+  if (!w || !grads || !stamps || !epochs || !m || !v || !state || rows <= 0 || H <= 0 || np < rows * H ||
+      n_ranks < 1 || n_ranks > ADAM_MAX_RANKS)
+    return set_error(CAST_ERR_BAD_ARG, "adam_tf_rows_peers");
+  const int rpw = rows_per_warp(rows);
+  long g = cdiv(cdiv(rows, rpw), 8);
+  if (g > 148 * 8) g = 148 * 8;
+  CAST_LAUNCH_DEP(adam_rows_peers_kernel, dim3((unsigned)g), dim3(256), 0, (cudaStream_t)stream, w,
+                  reinterpret_cast<const float* const*>(grads), reinterpret_cast<const unsigned* const*>(stamps),
+                  reinterpret_cast<const unsigned* const*>(epochs), n_ranks, m, v, rows, rpw, H, np, lr, beta1, beta2, eps,
+                  static_cast<const AdamState*>(state));
+  return check_launch("adam_rows_peers");
+}
+
+/* cast_adam_tf_step_peers over the elements [lo, n) only (elements below lo are neither reduced into g_red nor
+ * updated): the dense remainder behind the lazy row pass of cast_adam_tf_rows_peers.  Advances the beta powers. */
+extern "C" int cast_adam_tf_range_peers(float* w, const void* const* grads, int n_ranks, float* g_red, float* m,
+                                        float* v, long lo, long n, long tail, float lr, float beta1, float beta2,
+                                        float eps, void* state, void* stream) {
+  if (!w || !grads || !g_red || !m || !v || !state || lo < 0 || n <= lo || tail < 3 || n_ranks < 1)
+    return set_error(CAST_ERR_BAD_ARG, "adam_tf_range_peers");
+  if ((((uintptr_t)w | (uintptr_t)g_red | (uintptr_t)m | (uintptr_t)v) & 15) != 0)
+    return set_error(CAST_ERR_BAD_ARG, "adam_tf_range_peers: buffers must be 16-byte aligned");
+  long g = cdiv(cdiv(n + tail - (lo & ~3L), 4), 256);
+  if (g > 148 * 8) g = 148 * 8;
+  CAST_LAUNCH_DEP(adam_step_peers_kernel, dim3((unsigned)g), dim3(256), 0, (cudaStream_t)stream, w,
+                  reinterpret_cast<const float* const*>(grads), n_ranks, g_red, m, v, lo, n, tail, lr, beta1, beta2,
+                  eps, 0.f, 0L, 0L, static_cast<const AdamState*>(state));
+  int rc;
+  if ((rc = check_launch("adam_step_peers"))) return rc;
+  CAST_LAUNCH_DEP(adam_advance_kernel, dim3(1), dim3(32), 0, (cudaStream_t)stream, static_cast<AdamState*>(state), beta1,
+                  beta2);
   return check_launch("adam_advance");
 }

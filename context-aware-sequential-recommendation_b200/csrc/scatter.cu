@@ -118,11 +118,27 @@ static int g_seg_chunk = 0;
 // ("head": the run began in an earlier chunk) and/or part[w][1] ("tail": the run begins here and continues).  Stage 2
 // stitches the pieces of each crossing run in chunk order.  Work per warp is bounded by the chunk size however
 // skewed the id distribution is (popular items own thousands of entries).
-template <int NV, int SEG_CHUNK>
+// Lazy form (LAZY = true; the dense form compiles without it): stamp[r] == *epoch marks a table row that already holds a gradient of the current backward
+// pass.  The first segment sum that reaches row r in a pass writes it and stamps it, later ones (the other sources of
+// the owner pull) add to it, so the table needs no zeroing pass and rows no batch touches are never written.  Each
+// row is written by one warp per call and calls are stream-ordered: every lane reads the stamp before lane 0 moves it.
+template <bool LAZY>
+__device__ __forceinline__ bool row_adds(const unsigned* stamp, unsigned row, unsigned ep, int accumulate) {
+  if (LAZY) return stamp[row] == ep;
+  return accumulate != 0;
+}
+template <bool LAZY>
+__device__ __forceinline__ void stamp_row(unsigned* stamp, unsigned row, unsigned ep, int lane) {
+  if (!LAZY) return;
+  __syncwarp();
+  if (lane == 0) stamp[row] = ep;
+}
+
+template <int NV, int SEG_CHUNK, bool LAZY>
 __global__ void segment_partial_kernel(const unsigned* __restrict__ skeys, const unsigned* __restrict__ spay,
                                        long total, long N, ScatterSrc src, unsigned klo, unsigned khi, int H,
                                        float* __restrict__ dtable, float* __restrict__ part, int* __restrict__ pkey,
-                                       int accumulate) {
+                                       int accumulate, unsigned* __restrict__ stamp, const unsigned* __restrict__ epoch) {
   constexpr int SEG_Q = SEG_CHUNK / 32;
   cast_pdl_wait();
   cast_pdl_trigger();
@@ -132,6 +148,7 @@ __global__ void segment_partial_kernel(const unsigned* __restrict__ skeys, const
   if (beg >= total) return;
   const long end = beg + SEG_CHUNK < total ? beg + SEG_CHUNK : total;
   const int cnt = (int)(end - beg);
+  const unsigned ep = LAZY ? *epoch : 0u;
   constexpr int SEG_U = NV <= 2 ? 16 : (NV <= 8 ? 8 : (NV <= 16 ? 4 : 2));
   // ---- this lane's two entries
   unsigned mk[SEG_Q];
@@ -197,12 +214,14 @@ __global__ void segment_partial_kernel(const unsigned* __restrict__ skeys, const
             if (c < H) part[(w * 2 + 0) * H + c] = acc[i];
           }
         } else if (cur != 0u && cur >= klo && cur < khi) {
+          const bool add = row_adds<LAZY>(stamp, cur - klo, ep, accumulate);
 #pragma unroll
           for (int i = 0; i < NV; ++i) {
             const int c = lane + 32 * i;
             const long o = (long)(cur - klo) * H + c;
-            if (c < H) dtable[o] = accumulate ? dtable[o] + acc[i] : acc[i];
+            if (c < H) dtable[o] = add ? dtable[o] + acc[i] : acc[i];
           }
+          stamp_row<LAZY>(stamp, cur - klo, ep, lane);
         }
 #pragma unroll
         for (int i = 0; i < NV; ++i) acc[i] = 0.f;
@@ -229,12 +248,14 @@ __global__ void segment_partial_kernel(const unsigned* __restrict__ skeys, const
       if (c < H) part[(w * 2 + 1) * H + c] = acc[i];
     }
   } else if (cur != 0u && cur >= klo && cur < khi) {
+    const bool add = row_adds<LAZY>(stamp, cur - klo, ep, accumulate);
 #pragma unroll
     for (int i = 0; i < NV; ++i) {
       const int c = lane + 32 * i;
       const long o = (long)(cur - klo) * H + c;
-      if (c < H) dtable[o] = accumulate ? dtable[o] + acc[i] : acc[i];
+      if (c < H) dtable[o] = add ? dtable[o] + acc[i] : acc[i];
     }
+    stamp_row<LAZY>(stamp, cur - klo, ep, lane);
   }
   if (lane == 0) {
     pkey[w * 2 + 0] = head_key;
@@ -245,9 +266,10 @@ __global__ void segment_partial_kernel(const unsigned* __restrict__ skeys, const
 // Stage 2: the chunk where a crossing run begins adds the following chunks' heads.  The run length is found 32 chunks
 // per ballot; the sum uses ST_U interleaved accumulators (chunk j goes to accumulator j mod ST_U, each in ascending
 // chunk order) folded in a fixed order at the end => still a fixed summation tree, with ST_U loads in flight.
-template <int NV>
+template <int NV, bool LAZY>
 __global__ void segment_stitch_kernel(const float* __restrict__ part, const int* __restrict__ pkey, long nchunks,
-                                      unsigned klo, unsigned khi, int H, float* __restrict__ dtable, int accumulate) {
+                                      unsigned klo, unsigned khi, int H, float* __restrict__ dtable, int accumulate,
+                                      unsigned* __restrict__ stamp, const unsigned* __restrict__ epoch) {
   cast_pdl_wait();
   cast_pdl_trigger();
   const int lane = threadIdx.x & 31;
@@ -256,6 +278,7 @@ __global__ void segment_stitch_kernel(const float* __restrict__ part, const int*
   const int key = pkey[w * 2 + 1];
   if (key <= 0 || (unsigned)key < klo || (unsigned)key >= khi) return;
   constexpr int ST_U = NV <= 2 ? 16 : (NV <= 4 ? 8 : (NV <= 8 ? 4 : 2));
+  const unsigned ep = LAZY ? *epoch : 0u;
   long L = 0;  // chunks w+1 .. w+L continue the run
   for (;;) {
     const long w2 = w + 1 + L + lane;
@@ -289,6 +312,7 @@ __global__ void segment_stitch_kernel(const float* __restrict__ part, const int*
 #pragma unroll
       for (int i = 0; i < NV; ++i) acc[u][i] += val[u][i];
   }
+  const bool add = row_adds<LAZY>(stamp, (unsigned)key - klo, ep, accumulate);
 #pragma unroll
   for (int i = 0; i < NV; ++i) {
     const int c = lane + 32 * i;
@@ -297,9 +321,10 @@ __global__ void segment_stitch_kernel(const float* __restrict__ part, const int*
 #pragma unroll
       for (int u = 0; u < ST_U; ++u) s += acc[u][i];
       const long o = (long)((unsigned)key - klo) * H + c;
-      dtable[o] = accumulate ? dtable[o] + s : s;
+      dtable[o] = add ? dtable[o] + s : s;
     }
   }
+  stamp_row<LAZY>(stamp, (unsigned)key - klo, ep, lane);
 }
 
 // row-sharded table (TableRef, cast_rt.cuh): id -> owner-major key  (id % n) * R + id / n (+ 1 on shards 1..n-1), so
@@ -449,8 +474,9 @@ extern "C" int cast_scatter_sorted_offsets(long N, int nsrc, int Vkeys, size_t* 
 static int scatter_apply_impl(int nsrc, long N, const float* const* rows, const float* const* rowscale,
                               const float* scale, int H, float* dtable, long dtable_rows, const unsigned* kin,
                               const unsigned* pin, unsigned klo, unsigned khi, void* partial, size_t partial_bytes,
-                              int accumulate, void* stream) {
-  if (!rows || !scale || !dtable || !kin || nsrc < 1 || nsrc > 4 || N <= 0 || H <= 0 || H > 1024 || khi <= klo)
+                              int accumulate, unsigned* stamp, const unsigned* epoch, void* stream) {
+  if (!rows || !scale || !dtable || !kin || nsrc < 1 || nsrc > 4 || N <= 0 || H <= 0 || H > 1024 || khi <= klo ||
+      (stamp && !epoch))
     return set_error(CAST_ERR_BAD_ARG, "scatter_apply");
   const long total = N * nsrc;
   if (!partial || partial_bytes < cast_scatter_partial_bytes(N, nsrc, H))
@@ -466,31 +492,39 @@ static int scatter_apply_impl(int nsrc, long N, const float* const* rows, const 
   // rows nobody touches (and row 0) must read as zero: dense-gradient semantics of the reference
   // (accumulate: dtable already holds the sum of an earlier call over other sources; every row is written at most
   // once per call, so adding to it is race-free and keeps a fixed summation order)
-  if (!accumulate) cudaMemsetAsync(dtable, 0, (size_t)dtable_rows * H * sizeof(float), st);
+  // (lazy form: no zeroing; the stamps tell which rows hold this pass's gradient)
+  if (!accumulate && !stamp) cudaMemsetAsync(dtable, 0, (size_t)dtable_rows * H * sizeof(float), st);
   const int chunk = g_seg_chunk ? g_seg_chunk : (total >= 8 * ((long)khi - (long)klo) ? 64 : 32);
   const long nseg = cdiv(total, chunk);
   float* part = static_cast<float*>(partial);
   int* pkey = reinterpret_cast<int*>(part + (size_t)nseg * 2 * H);
   const int wpb = 4;
   const dim3 grid((unsigned)cdiv(nseg, wpb)), block(32 * wpb);
-#define CAST_SEG(NV)                                                                                            \
+#define CAST_SEG(NV, LZ)                                                                                        \
   {                                                                                                             \
     if (chunk == 32) {                                                                                          \
-      CAST_LAUNCH_DEP((segment_partial_kernel<NV, 32>), grid, block, 0, st, kin, pin, total, N, src, klo, khi, H,   \
-                  dtable, part, pkey, accumulate);                                                              \
+      CAST_LAUNCH_DEP((segment_partial_kernel<NV, 32, LZ>), grid, block, 0, st, kin, pin, total, N, src, klo, khi, \
+                  H, dtable, part, pkey, accumulate, stamp, epoch);                                             \
     } else {                                                                                                    \
-      CAST_LAUNCH_DEP((segment_partial_kernel<NV, 64>), grid, block, 0, st, kin, pin, total, N, src, klo, khi, H,   \
-                  dtable, part, pkey, accumulate);                                                              \
+      CAST_LAUNCH_DEP((segment_partial_kernel<NV, 64, LZ>), grid, block, 0, st, kin, pin, total, N, src, klo, khi, \
+                  H, dtable, part, pkey, accumulate, stamp, epoch);                                             \
     }                                                                                                           \
     if ((rc = check_launch("segment_partial"))) return rc;                                                      \
-    CAST_LAUNCH_DEP(segment_stitch_kernel<NV>, grid, block, 0, st, (const float*)part, (const int*)pkey, nseg, klo, \
-                khi, H, dtable, accumulate);                                                                    \
+    CAST_LAUNCH_DEP((segment_stitch_kernel<NV, LZ>), grid, block, 0, st, (const float*)part, (const int*)pkey,  \
+                nseg, klo, khi, H, dtable, accumulate, stamp, epoch);                                           \
   }
-  if (H <= 64) CAST_SEG(2)
-  else if (H <= 128) CAST_SEG(4)
-  else if (H <= 256) CAST_SEG(8)
-  else if (H <= 512) CAST_SEG(16)
-  else CAST_SEG(32)
+#define CAST_SEG_H(LZ)                                                                                          \
+  if (H <= 64) CAST_SEG(2, LZ)                                                                                  \
+  else if (H <= 128) CAST_SEG(4, LZ)                                                                            \
+  else if (H <= 256) CAST_SEG(8, LZ)                                                                            \
+  else if (H <= 512) CAST_SEG(16, LZ)                                                                           \
+  else CAST_SEG(32, LZ)
+  if (stamp) {
+    CAST_SEG_H(true)
+  } else {
+    CAST_SEG_H(false)
+  }
+#undef CAST_SEG_H
 #undef CAST_SEG
   return check_launch("segment_stitch");
 }
@@ -508,7 +542,25 @@ extern "C" int cast_scatter_apply(int nsrc, long N, const float* const* rows, co
   const unsigned char* w = static_cast<const unsigned char*>(workspace);
   return scatter_apply_impl(nsrc, N, rows, rowscale, scale, H, dtable, V, reinterpret_cast<const unsigned*>(w + ko),
                             reinterpret_cast<const unsigned*>(w + po), 0u, (unsigned)V, partial, partial_bytes,
-                            accumulate, stream);
+                            accumulate, nullptr, nullptr, stream);
+}
+
+/* cast_scatter_apply's lazy form (optimizer "lazy_adam"): no zeroing pass over the table; a row the batch touches is
+ * written (stamp[row] != *epoch) or added to (== *epoch) and then stamped, a row it does not touch keeps stale data
+ * and its old stamp.  stamp [V] and epoch are device memory; the epoch advances once per backward pass. */
+extern "C" int cast_scatter_apply_lazy(int nsrc, long N, const float* const* rows, const float* const* rowscale,
+                                       const float* scale, int V, int H, float* dtable, void* workspace,
+                                       size_t workspace_bytes, void* partial, size_t partial_bytes, unsigned* stamp,
+                                       const unsigned* epoch, void* stream) {
+  if (N <= 0 || nsrc < 1 || V <= 0 || !stamp || !epoch) return set_error(CAST_ERR_BAD_ARG, "scatter_apply_lazy");
+  if (!workspace || workspace_bytes < cast_scatter_workspace_bytes(N, nsrc, V))
+    return set_error(CAST_ERR_WORKSPACE, "scatter_apply_lazy: workspace too small");
+  size_t ko, po;
+  cast_scatter_sorted_offsets(N, nsrc, V, &ko, &po);
+  const unsigned char* w = static_cast<const unsigned char*>(workspace);
+  return scatter_apply_impl(nsrc, N, rows, rowscale, scale, H, dtable, V, reinterpret_cast<const unsigned*>(w + ko),
+                            reinterpret_cast<const unsigned*>(w + po), 0u, (unsigned)V, partial, partial_bytes, 0,
+                            stamp, epoch, stream);
 }
 
 /* Owner side of the row-sharded embedding gradient (SURVEY §8e): fold the entries of ONE rank's sorted arrays
@@ -522,7 +574,20 @@ extern "C" int cast_scatter_apply_range(int nsrc, long N, const float* const* ro
                                         size_t partial_bytes, int accumulate, void* stream) {
   return scatter_apply_impl(nsrc, N, rows, rowscale, scale, H, dtable, (long)key_hi - (long)key_lo,
                             static_cast<const unsigned*>(sorted_keys), static_cast<const unsigned*>(sorted_payload),
-                            key_lo, key_hi, partial, partial_bytes, accumulate, stream);
+                            key_lo, key_hi, partial, partial_bytes, accumulate, nullptr, nullptr, stream);
+}
+
+/* lazy form of cast_scatter_apply_range (stamps of dtable's rows, see cast_scatter_apply_lazy): every rank's call
+ * writes or adds by the stamps, so the rank-ordered calls need no accumulate flag and no zeroing pass */
+extern "C" int cast_scatter_apply_range_lazy(int nsrc, long N, const float* const* rows, const float* const* rowscale,
+                                             const float* scale, int H, float* dtable, const void* sorted_keys,
+                                             const void* sorted_payload, unsigned key_lo, unsigned key_hi,
+                                             void* partial, size_t partial_bytes, unsigned* stamp,
+                                             const unsigned* epoch, void* stream) {
+  if (!stamp || !epoch) return set_error(CAST_ERR_BAD_ARG, "scatter_apply_range_lazy");
+  return scatter_apply_impl(nsrc, N, rows, rowscale, scale, H, dtable, (long)key_hi - (long)key_lo,
+                            static_cast<const unsigned*>(sorted_keys), static_cast<const unsigned*>(sorted_payload),
+                            key_lo, key_hi, partial, partial_bytes, 0, stamp, epoch, stream);
 }
 
 /* cast_scatter_apply_range for a PEER's entries: its in-range rows are first gathered into `stage`
@@ -532,11 +597,11 @@ extern "C" size_t cast_scatter_stage_bytes(long N, int nsrc, int H) {
   return (size_t)N * nsrc * ((size_t)H + 1) * sizeof(float) + 256;
 }
 
-extern "C" int cast_scatter_pull_range(int nsrc, long N, const float* const* rows, const float* const* rowscale,
-                                       const float* scale, int H, float* dtable, const void* sorted_keys,
-                                       const void* sorted_payload, unsigned key_lo, unsigned key_hi, void* stage,
-                                       size_t stage_bytes, void* partial, size_t partial_bytes, int accumulate,
-                                       void* stream) {
+static int scatter_pull_range_impl(int nsrc, long N, const float* const* rows, const float* const* rowscale,
+                                   const float* scale, int H, float* dtable, const void* sorted_keys,
+                                   const void* sorted_payload, unsigned key_lo, unsigned key_hi, void* stage,
+                                   size_t stage_bytes, void* partial, size_t partial_bytes, int accumulate,
+                                   unsigned* stamp, const unsigned* epoch, void* stream) {
   if (!rows || !scale || !sorted_keys || !sorted_payload || nsrc < 1 || nsrc > 4 || N <= 0 || H <= 0)
     return set_error(CAST_ERR_BAD_ARG, "scatter_pull_range");
   if (!stage || stage_bytes < cast_scatter_stage_bytes(N, nsrc, H))
@@ -561,7 +626,28 @@ extern "C" int cast_scatter_pull_range(int nsrc, long N, const float* const* row
   const float one[1] = {1.0f};
   return scatter_apply_impl(1, total, lrows, lscale_rows, one, H, dtable, (long)key_hi - (long)key_lo,
                             static_cast<const unsigned*>(sorted_keys), nullptr, key_lo, key_hi, partial, partial_bytes,
-                            accumulate, stream);
+                            accumulate, stamp, epoch, stream);
+}
+
+extern "C" int cast_scatter_pull_range(int nsrc, long N, const float* const* rows, const float* const* rowscale,
+                                       const float* scale, int H, float* dtable, const void* sorted_keys,
+                                       const void* sorted_payload, unsigned key_lo, unsigned key_hi, void* stage,
+                                       size_t stage_bytes, void* partial, size_t partial_bytes, int accumulate,
+                                       void* stream) {
+  return scatter_pull_range_impl(nsrc, N, rows, rowscale, scale, H, dtable, sorted_keys, sorted_payload, key_lo,
+                                 key_hi, stage, stage_bytes, partial, partial_bytes, accumulate, nullptr, nullptr,
+                                 stream);
+}
+
+/* lazy form of cast_scatter_pull_range (stamps of dtable's rows, see cast_scatter_apply_lazy) */
+extern "C" int cast_scatter_pull_range_lazy(int nsrc, long N, const float* const* rows, const float* const* rowscale,
+                                            const float* scale, int H, float* dtable, const void* sorted_keys,
+                                            const void* sorted_payload, unsigned key_lo, unsigned key_hi, void* stage,
+                                            size_t stage_bytes, void* partial, size_t partial_bytes, unsigned* stamp,
+                                            const unsigned* epoch, void* stream) {
+  if (!stamp || !epoch) return set_error(CAST_ERR_BAD_ARG, "scatter_pull_range_lazy");
+  return scatter_pull_range_impl(nsrc, N, rows, rowscale, scale, H, dtable, sorted_keys, sorted_payload, key_lo,
+                                 key_hi, stage, stage_bytes, partial, partial_bytes, 0, stamp, epoch, stream);
 }
 
 extern "C" int cast_scatter_rows(const int* keys, int nsrc, long N, const float* const* rows,

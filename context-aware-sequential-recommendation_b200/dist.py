@@ -219,6 +219,15 @@ def attach(engine, group=None, arena=None):
         px.barrier()
 
     engine.peer_adam = (px.g_ptrs, px.world, px.g_red)
+    if engine.stamp is not None:
+        # lazy_adam: every rank's Adam reads the ranks' row stamps and gradient epochs next to their gradient rows
+        for name in ("stamp", "grad_epoch"):
+            t = getattr(engine, name)
+            shared = arena.alloc(t.numel(), t.dtype)
+            shared.copy_(t)
+            setattr(engine, name, shared)
+        engine.peer_stamps = tuple(torch.tensor(arena.ptrs(t), dtype=torch.int64, device=engine.device)
+                                   for t in (engine.stamp, engine.grad_epoch))
     engine.before_backward = px.barrier
     _quiesce_at_exit(engine, group)
     engine.grad_allreduce = exchange
@@ -301,9 +310,19 @@ def attach_sharded(engine, group=None, arena: "PeerArena | None" = None):
         if c.peer is None:
             build_peer_view(c)
         pv = c.peer
+        # lazy_adam: the owner's stamps decide write or add per row (no zeroing pass, no accumulate flag)
+        lazy = (engine.stamp.data_ptr(), engine.grad_epoch.data_ptr()) if engine.stamp is not None else None
         for p in range(world):
             rows_a, rs_a, keys_p, pay_p = pv.view[p]
-            if p == rank:   # own entries: summed straight from the source rows
+            if lazy and p == rank:
+                engine._call(engine.lib.cast_scatter_apply_range_lazy, pv.nsrc, c.N, rows_a, rs_a, pv.scale, H,
+                             engine.adam_g.data_ptr(), keys_p, pay_p, rank * R, (rank + 1) * R, c.spart.data_ptr(),
+                             c.spart_bytes, *lazy, engine._stream())
+            elif lazy:
+                engine._call(engine.lib.cast_scatter_pull_range_lazy, pv.nsrc, c.N, rows_a, rs_a, pv.scale, H,
+                             engine.adam_g.data_ptr(), keys_p, pay_p, rank * R, (rank + 1) * R, pv.stage.data_ptr(),
+                             pv.stage.numel() * 4, pv.spart.data_ptr(), pv.spart.numel() * 4, *lazy, engine._stream())
+            elif p == rank:   # own entries: summed straight from the source rows
                 engine._call(engine.lib.cast_scatter_apply_range, pv.nsrc, c.N, rows_a, rs_a, pv.scale, H,
                              engine.adam_g.data_ptr(), keys_p, pay_p, rank * R, (rank + 1) * R, c.spart.data_ptr(),
                              c.spart_bytes, 1 if p else 0, engine._stream())

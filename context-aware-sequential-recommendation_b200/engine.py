@@ -26,6 +26,7 @@ SITE_EMBED, SITE_CONCAT_A, SITE_CONCAT_B = 9000, 9001, 9002
 MODELS = ["cast_1", "cast_2", "cast_3", "cast_4", "cast_5", "cast_6", "cast_7", "cast_8", "cast_9", "sasrec",
           "sasrec_static"]  # reference main.py:28
 TABLE_ROWS = {"hours_emb": 25, "days_emb": 8}  # reference cast_3.py:34,45 ("24 hours / 7 days + zero padding")
+OPTIMIZERS = ["adam", "lazy_adam"]
 
 
 def block_site(tower: str, block: int, k: int) -> int:
@@ -135,7 +136,15 @@ class Engine:
         other shards are read over NVLink peer mappings once dist.attach has exchanged them).  alloc(numel, dtype) ->
         tensor: allocator for the buffers peers read (CPU tests: POSIX shared memory; default torch).
         fused=False runs every block on the generic LayerNorm + GEMM kernels even where the row kernels apply (the
-        reference the row kernels are tested against)."""
+        reference the row kernels are tested against).
+
+        args.optimizer (default "adam"): "adam" is the reference's dense TF-Adam on every parameter.  "lazy_adam" is
+        tf.contrib.opt.LazyAdamOptimizer on the item table: a step updates w, m and v of the table rows its batch touches
+        (the distinct nonzero ids of seq, pos and neg, over all ranks) with the dense update's arithmetic and bias
+        correction, and leaves every other row bit for bit as it was (row 0 and a shard's pad row never move); all other
+        parameters keep dense TF-Adam.  The step's table cost then follows the batch instead of the catalog.  It is a
+        different optimizer (m and v of a row decay only when the row is touched), so it is opt-in; it refuses
+        l2_emb != 0, whose table-wide decay cannot be lazy."""
         self.lib = lib if lib is not None else _lib.load_library()
         self.timing = None
         if device is None:
@@ -152,6 +161,11 @@ class Engine:
         self.rate = float(args.dropout_rate)
         self.lr = float(args.lr)
         self.l2 = float(getattr(args, "l2_emb", 0.0))
+        self.optimizer = getattr(args, "optimizer", "adam")
+        if self.optimizer not in OPTIMIZERS:
+            raise ValueError(f"optimizer must be one of {OPTIMIZERS}, got {self.optimizer!r}")
+        if self.optimizer == "lazy_adam" and self.l2:
+            raise ValueError("optimizer 'lazy_adam' cannot apply l2_emb: a table-wide decay would touch every row")
         self.seed = int(seed if seed is not None else (getattr(args, "seed", 0) or 0))
         self.beta1, self.beta2, self.eps = 0.9, 0.98, 1e-8  # models/sasrec.py:120 (beta2=0.98), TF defaults else
         self.item_shard = tuple(item_shard) if item_shard is not None and item_shard[1] > 1 else None
@@ -195,6 +209,14 @@ class Engine:
         self.n_params = total
         self.adam_state = torch.zeros(2, dtype=torch.int64, device=self.device)  # {f32 b1p, f32 b2p, u64 step}
         self.step_ptr = self.adam_state.data_ptr() + 8
+        # lazy_adam: the gradient epoch (advanced once per backward pass, never rewound) and each item-table row's stamp
+        # = the epoch of the last backward pass that wrote its gradient (csrc/scatter.cu, csrc/adam.cu).  Data
+        # parallelism moves both into peer-visible memory (dist.attach).
+        self.grad_epoch = self.stamp = None
+        self.peer_stamps = None     # set by dist.attach(): device arrays of the ranks' stamp / epoch pointers
+        if self.optimizer == "lazy_adam":
+            self.grad_epoch = torch.zeros(1, dtype=torch.int32, device=self.device)
+            self.stamp = torch.zeros(self.P["item_emb"].shape[0], dtype=torch.int32, device=self.device)
         self.sinus = torch.from_numpy(sinusoid_table(self.H, self.T)).to(self.device)
         self.init_parameters(self.seed or 42)
         self._call(self.lib.cast_adam_init_state, self.adam_state.data_ptr(), self.beta1, self.beta2, self._stream())
@@ -518,6 +540,14 @@ class Engine:
             if rows[0] is not c.g0:    # peers read the input-sequence gradient from the exported buffer
                 c.g0.copy_(rows[0])
             c.shard_src = (nsrc, [c.g0] + list(rows[1:]), list(rowscale), list(scale))
+            return
+        if table_name == "item_emb" and self.stamp is not None:   # lazy: no zeroing pass, touched rows get stamped
+            if not self._join(c, "sort"):
+                self._call(self.lib.cast_scatter_sort, keys.data_ptr(), nsrc, N, V, c.sws.data_ptr(), c.sws_bytes,
+                           self._stream())
+            self._call(self.lib.cast_scatter_apply_lazy, nsrc, N, rows_a, rs_a, sc_a, V, self.H,
+                       self.G[table_name].data_ptr(), c.sws.data_ptr(), c.sws_bytes, c.spart.data_ptr(),
+                       c.spart_bytes, self.stamp.data_ptr(), self.grad_epoch.data_ptr(), self._stream())
             return
         if table_name == "item_emb" and self._join(c, "sort"):   # the ids are sorted already: only the sums remain
             self._call(self.lib.cast_scatter_apply, nsrc, N, rows_a, rs_a, sc_a, V, self.H,
@@ -877,6 +907,9 @@ class Engine:
     def adam(self, c):
         # gradients are divided by sums[2] = sum(istarget) (global under data parallelism) inside the kernel; with a
         # row-sharded item table the flat buffers hold this rank's shard first, so the same launch updates it
+        if self.stamp is not None:
+            self.adam_lazy()
+            return
         if self.peer_adam is not None:
             ptrs, n_ranks, g_red = self.peer_adam
             self._call(self.lib.cast_adam_tf_step_peers, self.w.data_ptr(), ptrs.data_ptr(), n_ranks, g_red.data_ptr(),
@@ -888,6 +921,28 @@ class Engine:
                    self.v.data_ptr(), self.n_params, self.lr, self.beta1, self.beta2, self.eps,
                    self.adam_g[self.n_params + 2:].data_ptr(), self.l2, 0, self.l2_hi if self.l2 else 0,
                    self.adam_state.data_ptr(), self._stream())
+
+    def adam_lazy(self):
+        """lazy_adam: the touched rows of the item table (or of this rank's shard), then dense TF-Adam over the rest of
+        the flat buffer, which advances the beta powers once"""
+        rows, region, n = self.P["item_emb"].shape[0], self.P["item_emb"].numel(), self.n_params
+        if self.peer_adam is not None:
+            ptrs, n_ranks, g_red = self.peer_adam
+            sp, ep = self.peer_stamps
+            self._call(self.lib.cast_adam_tf_rows_peers, self.w.data_ptr(), ptrs.data_ptr(), sp.data_ptr(),
+                       ep.data_ptr(), n_ranks, self.m.data_ptr(), self.v.data_ptr(), rows, self.H, n, self.lr,
+                       self.beta1, self.beta2, self.eps, self.adam_state.data_ptr(), self._stream())
+            self._call(self.lib.cast_adam_tf_range_peers, self.w.data_ptr(), ptrs.data_ptr(), n_ranks, g_red.data_ptr(),
+                       self.m.data_ptr(), self.v.data_ptr(), region, n, g_red.numel() - n, self.lr, self.beta1,
+                       self.beta2, self.eps, self.adam_state.data_ptr(), self._stream())
+            return
+        g, gden = self.adam_g, self.adam_g[n + 2:].data_ptr()
+        self._call(self.lib.cast_adam_tf_rows, self.w.data_ptr(), g.data_ptr(), self.m.data_ptr(), self.v.data_ptr(),
+                   rows, self.H, self.lr, self.beta1, self.beta2, self.eps, gden, self.stamp.data_ptr(),
+                   self.grad_epoch.data_ptr(), self.adam_state.data_ptr(), self._stream())
+        self._call(self.lib.cast_adam_tf_range, self.w[region:].data_ptr(), g[region:].data_ptr(),
+                   self.m[region:].data_ptr(), self.v[region:].data_ptr(), n - region, self.lr, self.beta1, self.beta2,
+                   self.eps, gden, 0.0, 0, 0, self.adam_state.data_ptr(), 1, self._stream())
 
     def launch_fwd_bwd(self, c):
         # The sort of the (item id, entry) pairs for the embedding gradient depends on the ids only: it runs on a side
@@ -913,6 +968,8 @@ class Engine:
             self.forward(c, train=True)
             if self.before_backward is not None and not self._join(c, "barrier"):
                 self.before_backward()
+            if self.grad_epoch is not None:   # lazy_adam: the gradient rows this pass writes get a fresh stamp
+                self._call(self.lib.cast_grad_epoch_advance, self.grad_epoch.data_ptr(), self._stream())
             if self.fuse_tail:
                 self.loss_tail_fused(c)
             else:

@@ -352,6 +352,43 @@ int cast_adam_tf_step_peers(float* w, const void* const* grads, int n_ranks, flo
                             long tail, float lr, float beta1, float beta2, float eps, float l2, long l2_lo, long l2_hi,
                             void* state, void* stream);
 
+/* Lazy TF-Adam (tf.contrib.opt.LazyAdamOptimizer) for a row table: only the rows whose gradient the current backward
+ * pass wrote are updated; every other row keeps w, m and v bit for bit.  "Written" is tracked per row by a device
+ * stamp array and a device epoch counter (uint32 each):
+ *   cast_grad_epoch_advance        *epoch += 1 (one thread), once at the start of every backward pass; never rewound.
+ *   cast_scatter_*_lazy            the segment sums write a row whose stamp != *epoch (and stamp it), add to a row whose
+ *                                  stamp == *epoch, and skip the zeroing pass of the dense forms.
+ *   cast_adam_tf_rows              rows [1, rows) of a [rows, H] table with stamp == *epoch: the update of
+ *                                  cast_adam_tf_step (same lr_t, same 1/gdenom, same bits per element); no advance.
+ *   cast_adam_tf_rows_peers        the same with replicated data parallelism: grads / stamps / epochs are DEVICE arrays
+ *                                  of n_ranks pointers; row r's gradient is the rank-ordered sum over the ranks that
+ *                                  touched it (each rank's stamps against that rank's epoch), the denominator the
+ *                                  rank-ordered sum of grads[q][np + 2]; no advance (n_ranks <= 32).
+ *   cast_adam_tf_range_peers       cast_adam_tf_step_peers restricted to the elements [lo, n) (lo = the table's
+ *                                  rows * H): neither reduces nor updates below lo; advances the state. */
+int cast_grad_epoch_advance(unsigned* epoch, void* stream);
+int cast_adam_tf_rows(float* w, const float* grad, float* m, float* v, long rows, int H, float lr, float beta1,
+                      float beta2, float eps, const float* gdenom, const unsigned* stamp, const unsigned* epoch,
+                      void* state, void* stream);
+int cast_adam_tf_rows_peers(float* w, const void* const* grads, const void* const* stamps, const void* const* epochs,
+                            int n_ranks, float* m, float* v, long rows, int H, long np, float lr, float beta1,
+                            float beta2, float eps, void* state, void* stream);
+int cast_adam_tf_range_peers(float* w, const void* const* grads, int n_ranks, float* g_red, float* m, float* v, long lo,
+                             long n, long tail, float lr, float beta1, float beta2, float eps, void* state,
+                             void* stream);
+int cast_scatter_apply_lazy(int nsrc, long N, const float* const* rows, const float* const* rowscale,
+                            const float* scale, int V, int H, float* dtable, void* workspace, size_t workspace_bytes,
+                            void* partial, size_t partial_bytes, unsigned* stamp, const unsigned* epoch, void* stream);
+int cast_scatter_apply_range_lazy(int nsrc, long N, const float* const* rows, const float* const* rowscale,
+                                  const float* scale, int H, float* dtable, const void* sorted_keys,
+                                  const void* sorted_payload, unsigned key_lo, unsigned key_hi, void* partial,
+                                  size_t partial_bytes, unsigned* stamp, const unsigned* epoch, void* stream);
+int cast_scatter_pull_range_lazy(int nsrc, long N, const float* const* rows, const float* const* rowscale,
+                                 const float* scale, int H, float* dtable, const void* sorted_keys,
+                                 const void* sorted_payload, unsigned key_lo, unsigned key_hi, void* stage,
+                                 size_t stage_bytes, void* partial, size_t partial_bytes, unsigned* stamp,
+                                 const unsigned* epoch, void* stream);
+
 /* sasrec.py:93-97 + util.py:318-321: logits[u,c] = seq_last[u,:] . table0[cand[u,c],:] (sequential-k, unfused
  * multiply/add so the order is reproducible), and for candidate 0 the pair (count_greater, count_equal_excl_self)
  * from which the reference rank follows (SURVEY A-12). */

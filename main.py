@@ -68,6 +68,9 @@ def build_parser():
                    "hand raw timestamps to the device, which derives time bins / hours / weekdays there")
     p.add_argument("--recommend", default=0, type=int, help="with --test_model: after the evaluation, write the top K "
                    "items of every user (whole history excluded) to recommendations_top{K}.npz next to the checkpoint")
+    p.add_argument("--optimizer", default="adam", choices=["adam", "lazy_adam"],
+                   help="adam = the reference's dense TF-Adam; lazy_adam = LazyAdam on the item table (only the rows a "
+                   "batch touches are updated; step cost no longer grows with the catalog), dense TF-Adam elsewhere")
     return p
 
 
