@@ -33,9 +33,6 @@ SIGNATURES = {
     "cast_gemm_tensor_status": (I, [P, P]),
     "cast_gemm_workspace_bytes": (SZ, [L, I, L, I]),
     "cast_gemm": (I, [P, L, L, P, L, L, P, L, L, I, L, P, I, F, U64, P, I, P, L, F, P, L, P, I, P, SZ, P]),
-    "cast_fused_supported": (I, [I]),
-    "cast_ln_qkv_fwd": (I, [P, P, P, P, P, P, P, P, P, L, I, F, P, P, P, P, P, P, P, P, P]),
-    "cast_ln_ffn_fwd": (I, [P, P, P, P, P, P, P, P, F, U64, P, I, I, L, I, F, P, P, P, P, P, P]),
     "cast_rowk_supported": (I, [I]),
     "cast_rowk_image_bytes": (SZ, [I]),
     "cast_rowk_presplit": (I, [P, I, I, P, SZ, P]),

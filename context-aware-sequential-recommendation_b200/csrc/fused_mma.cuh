@@ -1,12 +1,12 @@
-// The fused row-tile kernels of fused.cu (included from there, after its helpers and argument structs): contractions
-// as mma.sync m16n8k8 3xTF32 (mma_tf32.cuh), tiles streamed through a two-stage cp.async pipeline so the next 64-row
-// tile loads while the current one is multiplied.
+// The backward row-tile kernels of fused.cu (included from there, after its helpers and argument structs):
+// contractions as mma.sync m16n8k8 3xTF32 (mma_tf32.cuh), tiles streamed through a two-stage cp.async pipeline so the
+// next 64-row tile loads while the current one is multiplied.
 //
-//   CTA = 8 warps (forward) or 16 warps (backward) on one 64-row tile; warp w owns the 16-row block (w & 3) and the
-//   column group (w >> 2: 32 or 16 columns) of every 64 x H product, and the same block of every H x H weight gradient.
+//   CTA = 16 warps (RM_BWD_NG = 4 column groups x 4 row blocks) on one 64-row tile; warp w owns the 16-row block
+//   (w & 3) and the 16-column group (w >> 2) of every 64 x H product, and the same block of every H x H weight
+//   gradient.
 //   Tiles are row-major with stride S = 8*ceil(H/8) + 4 floats (16-byte rows, S/4 odd: ldmatrix conflict-free);
 //   weights sit in shared memory in their natural [in][out] layout:
-//     forward  C = A W      : B[k][n] = W[k][n]            -> per-lane LDS.32 fragments
 //     dgrad    dX = dY W^T  : B^T[n'][k] = W[n'][k]        -> ldmatrix fragments (contraction along a weight row)
 //     wgrad    dW = X^T dY  : A^T and B straight from the two row-major tiles (contraction over the 64 rows)
 #pragma once
@@ -15,8 +15,8 @@
 namespace cast {
 
 // asynchronous copy of the 64-row tile starting at row0 of a row-major [N, H] tensor into dst (stride S); rows >= N
-// are zero-filled, columns >= H untouched (zeroed once at kernel start).  Warp w copies rows w, w+8, ...
-template <int S, int NW = FT / 32>
+// are zero-filled, columns >= H untouched (zeroed once at kernel start).  Warp w of NW copies rows w, w+NW, ...
+template <int S, int NW>
 __device__ __forceinline__ void rm_load_tile_async(float* __restrict__ dst, const float* __restrict__ src, long row0,
                                                    long N, int H, bool vec2) {
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
@@ -55,16 +55,8 @@ __device__ __forceinline__ void rm_zero_pad(float* __restrict__ buf, int rows, i
     for (int c = H; c < HP8; ++c) buf[r * S + c] = 0.f;
 }
 
-// W[H][H] row-major (global) -> Ws[k][n] stride S; the caller zeroed the buffer (64 rows) beforehand
-template <int S>
-__device__ __forceinline__ void rm_load_w(float* __restrict__ Ws, const float* __restrict__ W, int H) {
-  for (int idx = threadIdx.x; idx < H * H; idx += (int)blockDim.x) {
-    const int k = idx / H, n = idx - k * H;
-    Ws[k * S + n] = W[idx];
-  }
-}
-
-// the same through cp.async (joins the caller's next commit group: the weights arrive with the first row tile)
+// W[H][H] row-major (global) -> Ws[k][n] stride S through cp.async (joins the caller's next commit group: the weights
+// arrive with the first row tile)
 template <int S>
 __device__ __forceinline__ void rm_load_w_async(float* __restrict__ Ws, const float* __restrict__ W, int H) {
   for (int idx = threadIdx.x; idx < H * H; idx += (int)blockDim.x) {
@@ -200,37 +192,6 @@ __device__ __forceinline__ void rm_mm_bt(float (&acc)[NTW][4], const float* __re
       if (nt < nact) mma_tf32(acc[nt], ah, bl[nt][0], bl[nt][1]);
 #pragma unroll
     for (int nt = 0; nt < NTW; ++nt)
-      if (nt < nact) mma_tf32(acc[nt], ah, bh[nt][0], bh[nt][1]);
-  }
-}
-
-// acc[nt] += A[16 x 8KS] * B, B[k][n] row-major (n contiguous; column block starts at Bn), n-tiles nt < nact
-template <int KS, int S>
-__device__ __forceinline__ void rm_mm_b(float (&acc)[4][4], const float* __restrict__ As, const float* __restrict__ Bn,
-                                        int nact, int lane) {
-  const int g = lane >> 2, tig = lane & 3;
-#pragma unroll
-  for (int ks = 0; ks < KS; ++ks) {
-    unsigned af[4], ah[4], al[4];
-    ldsm_a<S>(af, As, ks * 8, lane);
-    tf32_split_n(af, ah, al);
-    const float* b0 = Bn + (ks * 8 + tig) * S + g;
-    unsigned bh[4][2], bl[4][2];
-#pragma unroll
-    for (int nt = 0; nt < 4; ++nt) {
-      if (nt < nact) {
-        tf32_split(b0[nt * 8], bh[nt][0], bl[nt][0]);
-        tf32_split(b0[4 * S + nt * 8], bh[nt][1], bl[nt][1]);
-      }
-    }
-#pragma unroll
-    for (int nt = 0; nt < 4; ++nt)
-      if (nt < nact) mma_tf32(acc[nt], al, bh[nt][0], bh[nt][1]);
-#pragma unroll
-    for (int nt = 0; nt < 4; ++nt)
-      if (nt < nact) mma_tf32(acc[nt], ah, bl[nt][0], bl[nt][1]);
-#pragma unroll
-    for (int nt = 0; nt < 4; ++nt)
       if (nt < nact) mma_tf32(acc[nt], ah, bh[nt][0], bh[nt][1]);
   }
 }
@@ -623,218 +584,6 @@ __global__ void __launch_bounds__(128 * NG, 1) ffn_bwd_mma_kernel(FfnBwdArgs a, 
   rm_fold_cols<SL>(vb2, sm, P + 2 * H + H * H + H + H * H, H);
   rm_store_wpartial(P + 2 * H, gW1[0], m0, n0, nact, H, lane);
   rm_store_wpartial(P + 2 * H + H * H + H, gW2[0], m0, n0, nact, H, lane);
-}
-
-// ------------------------------------------------------------------------------------------------ forward kernels
-// One 64-row tile per CTA, ~70 KB of shared memory => 3 CTAs per SM overlap each other's load / LayerNorm / product /
-// store phases.  Weights are staged transposed, Wt[n][k] (stride S), so that B fragments come from ldmatrix.
-
-// Wt[n][k] = W[k][n] for k, n < H, zeros for the padding up to [HP8][HP8]; warp per weight row, lanes along n
-template <int HP8, int S>
-__device__ __forceinline__ void rm_load_w_t(float* __restrict__ Wt, const float* __restrict__ W, int H) {
-  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-  constexpr int RW = HP8 / 8;  // weight rows per warp
-  float v[RW][2];
-#pragma unroll
-  for (int i = 0; i < RW; ++i) {  // all loads first (independent, in flight together), then the transposing stores
-    const int k = warp + 8 * i;
-#pragma unroll
-    for (int j = 0; j < 2; ++j) {
-      const int n = lane + 32 * j;
-      v[i][j] = (k < H && n < H) ? W[k * H + n] : 0.f;
-    }
-  }
-#pragma unroll
-  for (int i = 0; i < RW; ++i) {
-    const int k = warp + 8 * i;
-#pragma unroll
-    for (int j = 0; j < 2; ++j) {
-      const int n = lane + 32 * j;
-      if (n < HP8) Wt[n * S + k] = v[i][j];
-    }
-  }
-}
-
-// rm_mm_bt for a Bt buffer that ends after the last real n-tile: when nact is odd the ldmatrix rows of the missing
-// n-tile are redirected to the previous one (loaded twice, used once)
-template <int KS, int S>
-__device__ __forceinline__ void rm_mm_bt_tight(float (&acc)[4][4], const float* __restrict__ As,
-                                               const float* __restrict__ Bt, int nact, int lane) {
-  const int blk = lane >> 3, rr = lane & 7;
-#pragma unroll
-  for (int ks = 0; ks < KS; ++ks) {
-    unsigned af[4], ah[4], al[4];
-    ldsm_a<S>(af, As, ks * 8, lane);
-    tf32_split_n(af, ah, al);
-    unsigned bh[4][2], bl[4][2];
-#pragma unroll
-    for (int np = 0; np < 2; ++np) {
-      if (2 * np < nact) {
-        unsigned bf[4];
-        const int second = (2 * np + 1 < nact) ? (blk >> 1) : 0;
-        ldsm4(bf, Bt + (np * 16 + second * 8 + rr) * S + ks * 8 + (blk & 1) * 4);
-        tf32_split(__uint_as_float(bf[0]), bh[2 * np][0], bl[2 * np][0]);
-        tf32_split(__uint_as_float(bf[1]), bh[2 * np][1], bl[2 * np][1]);
-        tf32_split(__uint_as_float(bf[2]), bh[2 * np + 1][0], bl[2 * np + 1][0]);
-        tf32_split(__uint_as_float(bf[3]), bh[2 * np + 1][1], bl[2 * np + 1][1]);
-      }
-    }
-#pragma unroll
-    for (int nt = 0; nt < 4; ++nt)
-      if (nt < nact) mma_tf32(acc[nt], al, bh[nt][0], bh[nt][1]);
-#pragma unroll
-    for (int nt = 0; nt < 4; ++nt)
-      if (nt < nact) mma_tf32(acc[nt], ah, bl[nt][0], bl[nt][1]);
-#pragma unroll
-    for (int nt = 0; nt < 4; ++nt)
-      if (nt < nact) mma_tf32(acc[nt], ah, bh[nt][0], bh[nt][1]);
-  }
-}
-
-template <int KS>
-__global__ void __launch_bounds__(FT, 3) ln_qkv_fwd_mma_kernel(LnQkvArgs a, FDims d) {
-  constexpr int HP8 = 8 * KS, S = HP8 + 4, TILE = FR * S, WT = HP8 * S;
-  CAST_DYN_SMEM(float, sm);
-  float* Xs = sm;
-  float* Ns = Xs + TILE;   // LN(x) tile
-  float* Wsm = Ns + TILE;  // Wq^T | Wk^T | Wv^T, [HP8][S]
-  const int t = threadIdx.x, lane = t & 31, warp = t >> 5, g = lane >> 2, tig = lane & 3;
-  const int mt = warp & 3, nh = warp >> 2;
-  const int H = d.H;
-  int nact = KS - 4 * nh;
-  nact = nact < 0 ? 0 : (nact > 4 ? 4 : nact);
-  const int m0 = mt * 16, n0 = nh * 32;
-  const long row0 = (long)blockIdx.x * FR;
-  rm_load_tile_async<S>(Xs, a.x, row0, d.N, H, rm_vec2_ok(a.x, H));
-  cp_async_commit();
-  rm_zero_pad<HP8, S>(sm, 2 * FR, H);
-  for (int m = 0; m < 3; ++m) rm_load_w_t<HP8, S>(Wsm + m * WT, a.W[m], H);
-  cp_async_wait<0>();
-  __syncthreads();
-  f_layernorm_rows(Xs, Ns, a.gamma, a.beta, a.eps, row0, d, a.qn, a.mean, a.rstd, a.kmask, a.qmask);
-  __syncthreads();
-#pragma unroll
-  for (int m = 0; m < 3; ++m) {
-    float acc[4][4];
-    rm_zero(acc);
-    rm_mm_bt_tight<KS, S>(acc, (m == 0 ? Ns : Xs) + m0 * S, Wsm + m * WT + n0 * S, nact, lane);
-    const float* bias = a.b[m];
-    float* out = a.out[m];
-    const bool pair_ok = (H & 1) == 0 && (reinterpret_cast<uintptr_t>(out) & 7) == 0;
-#pragma unroll
-    for (int nt = 0; nt < 4; ++nt) {
-      if (nt >= nact) continue;
-      const int c = n0 + nt * 8 + 2 * tig;  // this thread's column pair (c, c+1) of the fragment
-      if (c >= H) continue;
-      const float bc0 = bias[c], bc1 = c + 1 < H ? bias[c + 1] : 0.f;
-#pragma unroll
-      for (int hf = 0; hf < 2; ++hf) {
-        const long row = row0 + m0 + g + hf * 8;
-        if (row >= d.N) continue;
-        const float v0 = acc[nt][2 * hf] + bc0, v1 = acc[nt][2 * hf + 1] + bc1;
-        if (pair_ok && c + 1 < H) {
-          *reinterpret_cast<float2*>(out + row * H + c) = make_float2(v0, v1);
-        } else {
-          out[row * H + c] = v0;
-          if (c + 1 < H) out[row * H + c + 1] = v1;
-        }
-      }
-    }
-  }
-}
-
-template <int KS>
-__global__ void __launch_bounds__(FT, 3) ln_ffn_fwd_mma_kernel(LnFfnArgs a, FDims d) {
-  constexpr int HP8 = 8 * KS, S = HP8 + 4, TILE = FR * S, WT = HP8 * S;
-  CAST_DYN_SMEM(float, sm);
-  float* Ys = sm;          // y tile, later the hidden activation
-  float* Ns = Ys + TILE;   // LN(y) tile
-  float* Wsm = Ns + TILE;  // W1^T | W2^T
-  const int t = threadIdx.x, lane = t & 31, warp = t >> 5, g = lane >> 2, tig = lane & 3;
-  const int mt = warp & 3, nh = warp >> 2;
-  const int H = d.H;
-  int nact = KS - 4 * nh;
-  nact = nact < 0 ? 0 : (nact > 4 ? 4 : nact);
-  const int m0 = mt * 16, n0 = nh * 32;
-  const long row0 = (long)blockIdx.x * FR;
-  rm_load_tile_async<S>(Ys, a.y, row0, d.N, H, rm_vec2_ok(a.y, H));
-  cp_async_commit();
-  rm_zero_pad<HP8, S>(sm, 2 * FR, H);
-  rm_load_w_t<HP8, S>(Wsm, a.W1, H);
-  rm_load_w_t<HP8, S>(Wsm + WT, a.W2, H);
-  const Drop dh = make_drop(a.rate, a.seed, a.step, a.site_h);
-  const Drop dout = make_drop(a.rate, a.seed, a.step, a.site_o);
-  const bool pair_ok = (H & 1) == 0 && ((reinterpret_cast<uintptr_t>(a.h1d) | reinterpret_cast<uintptr_t>(a.xout)) & 7) == 0;
-  cp_async_wait<0>();
-  __syncthreads();
-  f_layernorm_rows(Ys, Ns, a.gamma, a.beta, a.eps, row0, d, a.zn, a.mean, a.rstd, nullptr, nullptr);
-  __syncthreads();  // everybody is done with Ys (LN input): it becomes the hidden tile
-  float acc[4][4];
-  rm_zero(acc);
-  rm_mm_bt_tight<KS, S>(acc, Ns + m0 * S, Wsm + n0 * S, nact, lane);
-#pragma unroll
-  for (int nt = 0; nt < 4; ++nt) {
-    if (nt >= nact) continue;
-#pragma unroll
-    for (int hf = 0; hf < 2; ++hf) {
-      const int r = m0 + g + hf * 8, c0 = n0 + nt * 8 + 2 * tig;
-      const long row = row0 + r;
-      float dm2[2], hv[2];
-      drop_mul2(dh, (unsigned long long)(row * H + c0), dm2[0], dm2[1]);
-#pragma unroll
-      for (int cc = 0; cc < 2; ++cc) {
-        const int c = c0 + cc;
-        hv[cc] = (c < H && row < d.N) ? fmaxf(acc[nt][hf * 2 + cc] + a.b1[c], 0.f) * dm2[cc] : 0.f;
-        Ys[r * S + c] = hv[cc];
-      }
-      if (row < d.N && c0 < H) {
-        if (pair_ok && c0 + 1 < H) {
-          *reinterpret_cast<float2*>(a.h1d + row * H + c0) = make_float2(hv[0], hv[1]);
-        } else {
-          a.h1d[row * H + c0] = hv[0];
-          if (c0 + 1 < H) a.h1d[row * H + c0 + 1] = hv[1];
-        }
-      }
-    }
-  }
-  __syncthreads();
-  rm_zero(acc);
-  rm_mm_bt_tight<KS, S>(acc, Ys + m0 * S, Wsm + WT + n0 * S, nact, lane);
-#pragma unroll
-  for (int nt = 0; nt < 4; ++nt) {
-    if (nt >= nact) continue;
-#pragma unroll
-    for (int hf = 0; hf < 2; ++hf) {
-      const int r = m0 + g + hf * 8, c0 = n0 + nt * 8 + 2 * tig;
-      const long row = row0 + r;
-      if (row >= d.N) continue;
-      const float m = a.ids ? (a.ids[row] != 0 ? 1.f : 0.f) : 1.f;
-      float dm2[2], ov[2];
-      drop_mul2(dout, (unsigned long long)(row * H + c0), dm2[0], dm2[1]);
-#pragma unroll
-      for (int cc = 0; cc < 2; ++cc) {
-        const int c = c0 + cc;
-        ov[cc] = c < H ? ((acc[nt][hf * 2 + cc] + a.b2[c]) * dm2[cc] + Ns[r * S + c]) * m : 0.f;
-      }
-      if (c0 < H) {
-        if (pair_ok && c0 + 1 < H) {
-          *reinterpret_cast<float2*>(a.xout + row * H + c0) = make_float2(ov[0], ov[1]);
-        } else {
-          a.xout[row * H + c0] = ov[0];
-          if (c0 + 1 < H) a.xout[row * H + c0 + 1] = ov[1];
-        }
-      }
-    }
-  }
-}
-
-template <int KS>
-static size_t ln_qkv_fwd_mma_smem() {
-  return sizeof(float) * ((size_t)2 * FR * (8 * KS + 4) + (size_t)3 * 8 * KS * (8 * KS + 4));
-}
-template <int KS>
-static size_t ln_ffn_fwd_mma_smem() {
-  return sizeof(float) * ((size_t)2 * FR * (8 * KS + 4) + (size_t)2 * 8 * KS * (8 * KS + 4));
 }
 
 constexpr int RM_BWD_NG = 4;  // column groups (x4 row blocks = 16 warps) of the backward row kernels

@@ -1,7 +1,8 @@
 // Dense projections on the 5th-generation tensor cores: the strided GEMM of cast_gemm (tf.layers.dense / conv1d(k=1)
 // of modules.py:203-205, :298-306, :333-334 and their gradients) as tcgen05.mma kind::tf32 with the 3xTF32 operand
 // split (hi*hi + hi*lo + lo*hi => ~2^-22 relative to sum|a||b|: fp32-grade results, parity tolerance 1e-4 holds).
-// Used for the wide models (hidden_units > 64: BASELINE configs 4 and 5); H <= 64 runs the fused row kernels.
+// Used for the blocks of the wide models (hidden_units > 64: BASELINE configs 4 and 5) and of any width outside the
+// row kernels' 8 <= H <= 52; the blocks of configs 1-3 (H = 50) run the row kernels.
 //
 // Persistent, warp-specialised CTAs (one per SM) over work units = (128-row tile, <=256-column tile, K range):
 //   warps 0-3  producers : split the fp32 A chunk (and, for weight gradients, the B chunk) into tf32 hi/lo and store it

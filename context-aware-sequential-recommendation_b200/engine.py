@@ -136,7 +136,7 @@ class Engine:
         other shards are read over NVLink peer mappings once dist.attach has exchanged them).  alloc(numel, dtype) ->
         tensor: allocator for the buffers peers read (CPU tests: POSIX shared memory; default torch).
         fused=False runs every block on the generic LayerNorm + GEMM kernels even where the row kernels apply (the
-        reference the row kernels are tested against).
+        reference the row kernels are tested against); widths the row kernels do not take run there too.
 
         args.optimizer (default "adam"): "adam" is the reference's dense TF-Adam on every parameter.  "lazy_adam" is
         tf.contrib.opt.LazyAdamOptimizer on the item table: a step updates w, m and v of the table rows its batch touches
@@ -221,26 +221,22 @@ class Engine:
         self.init_parameters(self.seed or 42)
         self._call(self.lib.cast_adam_init_state, self.adam_state.data_ptr(), self.beta1, self.beta2, self._stream())
         self._ctx: Dict[int, SimpleNamespace] = {}
-        # The kernels every transformer block runs on, fixed for the engine's lifetime (the row kernels take H <= 64):
-        #   "rowk"   forward on the tcgen05 row kernels (csrc/row_umma.cu), backward on the mma.sync row kernels
-        #   "fused"  the mma.sync row kernels both ways (csrc/fused.cu)
-        #   "gemm"   LayerNorm kernels + cast_gemm / cast_colsum
-        # Both row-kernel paths defer their gradient partial sums to one reduction launch per step.
+        # The kernels every transformer block runs on, fixed for the engine's lifetime: with row_kernels the forward
+        # runs on the tcgen05 row kernels (csrc/row_umma.cu, cast_rowk_supported(H)), the backward on the mma.sync row
+        # kernels (csrc/fused.cu), and the gradient partial sums wait for one reduction launch per step; otherwise
+        # LayerNorm kernels + cast_gemm / cast_colsum.
+        self.row_kernels = bool(fused and self.lib.cast_rowk_supported(self.H))
         names = [f"{tower}.{i}." for tower, nb in self.plan.towers.items() for i in range(nb)]
-        if fused and self.lib.cast_rowk_supported(self.H) and names:
-            self.block_path = "rowk"
-        elif fused and self.lib.cast_fused_supported(self.H):
-            self.block_path = "fused"
-        else:
-            self.block_path = "gemm"
-        if self.block_path == "rowk":   # per-block weight operand images, rebuilt once per forward pass
+        # per-block weight operand images, rebuilt once per forward pass (cast_rowk_presplit); none without blocks
+        self.rowk_img = None
+        if self.row_kernels and names:
             self.rowk_block = {n: j for j, n in enumerate(names)}
             self.rowk_img_bytes = int(self.lib.cast_rowk_image_bytes(self.H))
             self.rowk_img = torch.zeros(len(names) * self.rowk_img_bytes, dtype=torch.uint8, device=self.device)
             ptrs = [self.P[n + w].data_ptr() for n in names for w in ("q.w", "k.w", "v.w", "ffn1.w", "ffn2.w")]
             self.rowk_wptrs = (C.c_void_p * len(ptrs))(*ptrs)
         # final LayerNorm + loss + LayerNorm backward in one launch: the main tower's output must be seq_emb itself
-        self.fuse_tail = (self.block_path != "gemm" and self.item_shard is None
+        self.fuse_tail = (self.row_kernels and self.item_shard is None
                           and not (self.plan.merge and self.plan.merge[3] == "post"))
         self.world_size = 1
         self.grad_allreduce = None  # set by dist.attach(); called between backward and Adam
@@ -390,7 +386,6 @@ class Engine:
         H, T, h, dev = self.H, self.T, self.h, self.device
         N = B * T
         lib = self.lib
-        fused = self.block_path != "gemm"
         f = lambda *s: torch.empty(*s, dtype=torch.float32, device=dev)  # noqa: E731
         # buffers the other ranks read during the row-sharded gradient exchange (dist.attach_sharded)
         fp = (lambda *s: self._peer_zeros(int(np.prod(s)), torch.float32).view(*s)) if self.item_shard else f
@@ -413,7 +408,7 @@ class Engine:
                     setattr(b, nm, f(N))
                 for nm in ("rmax", "rlinv", "rowD"):
                     setattr(b, nm, f(B * h * T))
-                if fused:
+                if self.row_kernels:
                     # own partial buffers per block: the fixed-order reduction of all blocks is one launch at the end
                     # of backward (cast_reduce_partials_batch) instead of one small launch per fused backward kernel
                     nws = self.lib.cast_block_bwd_workspace_bytes(N, H) // 4 + 16
@@ -421,7 +416,7 @@ class Engine:
                 blocks.append(b)
             # x_last: the main tower's last block output, normalised by cast_lnf_loss (fuse_tail);
             # ws_lnf: the gamma/beta partials of the final LayerNorm's backward (row-kernel paths, unless fuse_tail)
-            lnf_partials = fused and not (tower == "main" and self.fuse_tail)
+            lnf_partials = self.row_kernels and not (tower == "main" and self.fuse_tail)
             c.tw[tower] = SimpleNamespace(blocks=blocks, out=(fp if tower == "main" else f)(N, H), muf=f(N), rsf=f(N),
                                           dx_in=f(N, H), x_in=None, x_last=None,
                                           ws_lnf=f(lib.cast_layernorm_bwd_workspace_bytes(N, H) // 4 + 16)
@@ -567,24 +562,16 @@ class Engine:
         H, B, T, h = self.H, c.B, self.T, self.h
         x = x_in
         nb = len(tb.blocks)
-        path = self.block_path
         self._join(c, "presplit")   # the rowk weight split, if launch_fwd_bwd forked it
         P = self.P
         for i, b in enumerate(tb.blocks):
             pre = f"{tower}.{i}."
-            if path == "rowk":
+            if self.row_kernels:
                 self._call(self.lib.cast_rowk_ln_qkv_fwd, x.data_ptr(), P[pre + "ln1.gamma"].data_ptr(),
                            P[pre + "ln1.beta"].data_ptr(), P[pre + "q.b"].data_ptr(), P[pre + "k.b"].data_ptr(),
                            P[pre + "v.b"].data_ptr(), self.rowk_image(pre), c.N, H, 1e-8, b.qn.data_ptr(),
                            b.Q.data_ptr(), b.K.data_ptr(), b.V.data_ptr(), b.mu1.data_ptr(), b.rs1.data_ptr(),
                            b.kmask.data_ptr(), b.qmask.data_ptr(), self._stream())
-            elif path == "fused":
-                self._call(self.lib.cast_ln_qkv_fwd, x.data_ptr(), P[pre + "ln1.gamma"].data_ptr(),
-                           P[pre + "ln1.beta"].data_ptr(), P[pre + "q.w"].data_ptr(), P[pre + "q.b"].data_ptr(),
-                           P[pre + "k.w"].data_ptr(), P[pre + "k.b"].data_ptr(), P[pre + "v.w"].data_ptr(),
-                           P[pre + "v.b"].data_ptr(), c.N, H, 1e-8, b.qn.data_ptr(), b.Q.data_ptr(), b.K.data_ptr(),
-                           b.V.data_ptr(), b.mu1.data_ptr(), b.rs1.data_ptr(), b.kmask.data_ptr(),
-                           b.qmask.data_ptr(), self._stream())
             else:
                 self.ln_fwd(x, pre + "ln1", b.qn, b.mu1, b.rs1, b.kmask, b.qmask)
                 self.linear_fwd(c, b.qn, self.P[pre + "q.w"], self.P[pre + "q.b"], b.Q)
@@ -599,19 +586,12 @@ class Engine:
                        b.qn.data_ptr(), b.kmask.data_ptr(), b.qmask.data_ptr(), B, T, H, h, rate, self.seed,
                        self.step_ptr, block_site(tower, i, 1), ids.data_ptr(), b.y.data_ptr(), self._p(attn),
                        b.rmax.data_ptr(), b.rlinv.data_ptr(), self._stream())
-            if path == "rowk":
+            if self.row_kernels:
                 self._call(self.lib.cast_rowk_ln_ffn_fwd, b.y.data_ptr(), P[pre + "ln2.gamma"].data_ptr(),
                            P[pre + "ln2.beta"].data_ptr(), P[pre + "ffn1.b"].data_ptr(), P[pre + "ffn2.b"].data_ptr(),
                            self.rowk_image(pre), ids.data_ptr(), rate, self.seed, self.step_ptr,
                            block_site(tower, i, 2), block_site(tower, i, 3), c.N, H, 1e-8, b.zn.data_ptr(),
                            b.h1d.data_ptr(), b.xout.data_ptr(), b.mu2.data_ptr(), b.rs2.data_ptr(), self._stream())
-            elif path == "fused":
-                self._call(self.lib.cast_ln_ffn_fwd, b.y.data_ptr(), P[pre + "ln2.gamma"].data_ptr(),
-                           P[pre + "ln2.beta"].data_ptr(), P[pre + "ffn1.w"].data_ptr(), P[pre + "ffn1.b"].data_ptr(),
-                           P[pre + "ffn2.w"].data_ptr(), P[pre + "ffn2.b"].data_ptr(), ids.data_ptr(), rate,
-                           self.seed, self.step_ptr, block_site(tower, i, 2), block_site(tower, i, 3), c.N, H, 1e-8,
-                           b.zn.data_ptr(), b.h1d.data_ptr(), b.xout.data_ptr(), b.mu2.data_ptr(), b.rs2.data_ptr(),
-                           self._stream())
             else:
                 self.ln_fwd(b.y, pre + "ln2", b.zn, b.mu2, b.rs2)
                 self.linear_fwd(c, b.zn, self.P[pre + "ffn1.w"], self.P[pre + "ffn1.b"], b.h1d, relu=1, rate=rate,
@@ -627,7 +607,7 @@ class Engine:
 
     def tower_bwd(self, c, tower, d_out, ids, embed_fx=None):
         """Backward of tower_fwd; parameter gradients land in self.G, returns d(loss)/d(x_in) (tb.dx_in).
-        embed_fx = (mask ids or None, dropout rate, site, out): on the fused path block 0's kernel also applies the
+        embed_fx = (mask ids or None, dropout rate, site, out): on the row-kernel path block 0's kernel also applies the
         backward of `dropout(emb) * mask` (sasrec.py:58-62) and writes the result to `out` (returned instead)."""
         tb = c.tw[tower]
         H, B, T, h = self.H, c.B, self.T, self.h
@@ -636,11 +616,10 @@ class Engine:
         t = c.t
         nb = len(tb.blocks)
         x_last = tb.blocks[-1].xout if nb else tb.x_in
-        fused = self.block_path != "gemm"
         dx = t[0]
         if tower == "main" and self.fuse_tail:
             pass                # dx (= t[0]) and the gamma/beta partials were produced by cast_lnf_loss
-        elif fused:  # gamma/beta partials of the tower's final LayerNorm join the step's single reduction launch
+        elif self.row_kernels:  # final LayerNorm's gamma/beta partials join the step's single reduction launch
             self._call(self.lib.cast_layernorm_bwd, d_out.data_ptr(), x_last.data_ptr(), tb.muf.data_ptr(),
                        tb.rsf.data_ptr(), self.P[tower + ".lnf.gamma"].data_ptr(), c.N, H, None, dx.data_ptr(), None,
                        None, tb.ws_lnf.data_ptr(), tb.ws_lnf.numel() * 4, self._stream())
@@ -656,7 +635,7 @@ class Engine:
             x_i = tb.blocks[i - 1].xout if i > 0 else tb.x_in
             gm, gmd, dh, dzn, dy = t[1], t[2], t[3], t[4], t[5]
             # x_out = (dropout(h1d W2 + b2) + zn) * mask                      modules.py:304-311, sasrec.py:83
-            if fused:
+            if self.row_kernels:
                 self._call(self.lib.cast_ffn_bwd, dx.data_ptr(), ids.data_ptr(), b.zn.data_ptr(), b.h1d.data_ptr(),
                            b.y.data_ptr(), b.mu2.data_ptr(), b.rs2.data_ptr(), P[pre + "ln2.gamma"].data_ptr(),
                            P[pre + "ffn1.w"].data_ptr(), P[pre + "ffn2.w"].data_ptr(), rate, self.seed, self.step_ptr,
@@ -680,7 +659,7 @@ class Engine:
                        block_site(tower, i, 1),
                        dQ.data_ptr(), H, dK.data_ptr(), H, dV.data_ptr(), H, b.y.data_ptr(), b.qn.data_ptr(),
                        self._p(c.attn_ws), c.attn_ws.numel() * 4 if c.attn_ws is not None else 0, self._stream())
-            if fused:
+            if self.row_kernels:
                 dst = tb.dx_in if i == 0 else t[0]
                 if i == 0 and embed_fx is not None:
                     fx_ids, fx_rate, fx_site, dst = embed_fx
@@ -764,7 +743,7 @@ class Engine:
         """Builds seq_emb [N,H] from the ids already resident in c.keys3 / c.cids; returns the buffer."""
         plan = self.plan
         ids = c.keys3[0]
-        if self.block_path == "rowk" and "presplit" not in c.forked:
+        if self.rowk_img is not None and "presplit" not in c.forked:
             self.rowk_presplit(self._stream())   # weights moved since the last step: refresh the operand images
         streams: Dict[str, torch.Tensor] = {}
         for j, (tname, key) in enumerate((("time_emb", "time"), ("hours_emb", "hours"), ("days_emb", "days"))):
@@ -830,7 +809,7 @@ class Engine:
         add_time, drop, mask = plan.embed
         pre_merge = bool(plan.merge and plan.merge[3] == "pre")
         # the tower's input is dropout(emb) * mask: block 0's fused backward kernel applies that gradient itself
-        fuse_embed = ((drop or mask) and not pre_merge and self.block_path != "gemm"
+        fuse_embed = ((drop or mask) and not pre_merge and self.row_kernels
                       and len(c.tw["main"].blocks) > 0)
         d = self.tower_bwd(c, "main", d, ids, embed_fx=(ids if mask else None, self.rate if drop else 0.0, SITE_EMBED,
                                                         c.g0) if fuse_embed else None)
@@ -850,7 +829,7 @@ class Engine:
             dstreams["time"] = g0
         if plan.learned_pos:
             th = self.T * self.H
-            if self.block_path != "gemm":
+            if self.row_kernels:
                 # d(pos_emb) = sum over the batch of g0 [B, T*H]: another job of the step's reduction launch
                 c.reduce_jobs.append((g0.data_ptr(), c.B, th, self.G["pos_emb"], th))
             else:
@@ -958,7 +937,7 @@ class Engine:
                            self._stream())
 
         try:
-            if self._fork(c, "sort", sort) and self.block_path == "rowk":
+            if self._fork(c, "sort", sort) and self.rowk_img is not None:
                 # the weight operand images are needed by the first row kernel, not by the embedding
                 self._fork(c, "presplit", lambda: self.rowk_presplit(self._stream()))
             # "peers have finished reading the previous step's gradients": a flag round trip over NVLink that nothing in

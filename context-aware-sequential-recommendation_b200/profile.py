@@ -20,13 +20,9 @@ def _work(name, a, B, T, H, h):
         return 4.0 * B * T * T * H, 4.0 * 5 * B * T * H
     if name == "cast_attn_bwd":   # dP, dQ, dK, dV = 2x forward (algorithmic; recomputation of S not counted)
         return 8.0 * B * T * T * H, 4.0 * 8 * B * T * H
-    if name == "cast_ln_qkv_fwd":   # 3 projections  (a[9]=N, a[10]=H)
-        return 6.0 * a[9] * a[10] * a[10], 4.0 * 5 * a[9] * a[10]
-    if name == "cast_ln_ffn_fwd":   # 2 GEMMs        (a[13]=N, a[14]=H)
-        return 4.0 * a[13] * a[14] * a[14], 4.0 * 4 * a[13] * a[14]
-    if name == "cast_rowk_ln_qkv_fwd":  # tcgen05 version (a[7]=N, a[8]=H)
+    if name == "cast_rowk_ln_qkv_fwd":  # 3 projections  (a[7]=N, a[8]=H)
         return 6.0 * a[7] * a[8] * a[8], 4.0 * 5 * a[7] * a[8]
-    if name == "cast_rowk_ln_ffn_fwd":  # tcgen05 version (a[12]=N, a[13]=H)
+    if name == "cast_rowk_ln_ffn_fwd":  # 2 GEMMs        (a[12]=N, a[13]=H)
         return 4.0 * a[12] * a[13] * a[13], 4.0 * 4 * a[12] * a[13]
     if name == "cast_ffn_bwd":      # 2 dgrad + 2 wgrad  (a[14]=N, a[15]=H)
         return 8.0 * a[14] * a[15] * a[15], 4.0 * 5 * a[14] * a[15]
@@ -101,8 +97,8 @@ def load_peaks(root):
     return d
 
 
-COMPUTE_BOUND = ("cast_attn_fwd", "cast_attn_bwd", "cast_gemm", "cast_qkv_bwd", "cast_qkv_bwd_embed", "cast_ffn_bwd", "cast_ln_qkv_fwd",
-                 "cast_ln_ffn_fwd", "cast_rowk_ln_qkv_fwd", "cast_rowk_ln_ffn_fwd")
+COMPUTE_BOUND = ("cast_attn_fwd", "cast_attn_bwd", "cast_gemm", "cast_qkv_bwd", "cast_qkv_bwd_embed", "cast_ffn_bwd",
+                 "cast_rowk_ln_qkv_fwd", "cast_rowk_ln_ffn_fwd")
 
 
 def ncu_traffic(root, name):

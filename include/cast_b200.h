@@ -154,32 +154,18 @@ int cast_gemm(const float* A, long sam, long sak, const float* B, long sbk, long
               const float* resid, long ldr, const int* row_ids, int splits, void* workspace, size_t workspace_bytes,
               void* stream);
 
-/* ---- fused row-tile kernels of one transformer block, hidden_units <= 64 (cast_fused_supported) -------------------
- * ln_qkv_fwd  = normalize (modules.py:74-78) + the three tf.layers.dense of multihead_attention (:203-205) + the key /
- *               query zero-sum flags (:222, :248).
- * ln_ffn_fwd  = normalize + feedforward (modules.py:298-313) + `*= mask` (sasrec.py:83); saves LN output zn, the
- *               post-dropout hidden activation h1d, LN stats.
- * ffn_bwd / qkv_bwd = their backward passes.  Parameter gradients are written to `grads_out`, which must be the
- *               contiguous flat block  [ln.beta H | ln.gamma H | W H*H | b H | ...]  in the order
- *               (ffn_bwd) ln2.beta, ln2.gamma, ffn1.w, ffn1.b, ffn2.w, ffn2.b
- *               (qkv_bwd) ln1.beta, ln1.gamma, q.w, q.b, k.w, k.b, v.w, v.b          (all W stored [in,out]).
- *               qkv_bwd adds `dres` (gradient of the `outputs += queries` residual, modules.py:269) to d(LN(x)). */
-int cast_fused_supported(int H);
-int cast_ln_qkv_fwd(const float* x, const float* gamma, const float* beta, const float* Wq, const float* bq,
-                    const float* Wk, const float* bk, const float* Wv, const float* bv, long N, int H, float eps,
-                    float* qn, float* Q, float* K, float* V, float* mean, float* rstd, float* kmask, float* qmask,
-                    void* stream);
-int cast_ln_ffn_fwd(const float* y, const float* gamma, const float* beta, const float* W1, const float* b1,
-                    const float* W2, const float* b2, const int* ids, float drop_rate, unsigned long long seed,
-                    const unsigned long long* step, int site_hidden, int site_out, long N, int H, float eps, float* zn,
-                    float* h1d, float* xout, float* mean, float* rstd, void* stream);
-/* ---- the same forward row kernels on the 5th-generation tensor cores (tcgen05.mma kind::tf32, TMEM accumulators) -----
+/* ---- forward row kernels of one transformer block on the 5th-generation tensor cores (tcgen05.mma kind::tf32,
+ * TMEM accumulators) ----------------------------------------------------------------------------------------------
+ * cast_rowk_ln_qkv_fwd = normalize (modules.py:74-78) + the three tf.layers.dense of multihead_attention (:203-205) +
+ *               the key / query zero-sum flags (:222, :248).
+ * cast_rowk_ln_ffn_fwd = normalize + feedforward (modules.py:298-313) + `*= mask` (sasrec.py:83); saves LN output zn,
+ *               the post-dropout hidden activation h1d, LN stats.
+ * Both take their weights from the block's images.
  * cast_rowk_supported(H): hidden_units the tcgen05 row kernels accept (their shared-memory plan must fit 227 KB).
  * cast_rowk_presplit: once per step (weights change with every Adam update), splits the five [H,H] matrices of each
  *   block {Wq, Wk, Wv, W1, W2} (`weights` = HOST array of nblocks*5 device pointers) into tf32 hi/lo operand images
  *   (K-major UMMA layout; transposed and plain forms) at images + b * cast_rowk_image_bytes(H).
- * cast_rowk_ln_qkv_fwd / cast_rowk_ln_ffn_fwd: same contract as cast_ln_qkv_fwd / cast_ln_ffn_fwd, weights taken from
- *   the block's images.  cast_rowk_status reports (and clears) the kernels' barrier watchdog; it synchronises. */
+ * cast_rowk_status reports (and clears) the kernels' barrier watchdog; it synchronises. */
 int cast_rowk_supported(int H);
 size_t cast_rowk_image_bytes(int H);
 int cast_rowk_presplit(const float* const* weights, int nblocks, int H, void* images, size_t image_bytes, void* stream);
@@ -195,6 +181,13 @@ int cast_rowk_status(int* timed_out);
 int cast_rowk_set_grid(int max_ctas);
 /* tuning hook: device buffer of 148*4*16 int64 filled with clock64() phase stamps by the row kernels (NULL: off) */
 int cast_rowk_set_trace(void* device_buffer);
+/* ---- backward row kernels of one transformer block (mma.sync), hidden_units <= 64 ---------------------------------
+ * cast_ffn_bwd / cast_qkv_bwd = the backward passes of cast_rowk_ln_ffn_fwd / cast_rowk_ln_qkv_fwd.  Parameter
+ *               gradients are written to `grads_out`, which must be the contiguous flat block
+ *               [ln.beta H | ln.gamma H | W H*H | b H | ...]  in the order
+ *               (ffn_bwd) ln2.beta, ln2.gamma, ffn1.w, ffn1.b, ffn2.w, ffn2.b
+ *               (qkv_bwd) ln1.beta, ln1.gamma, q.w, q.b, k.w, k.b, v.w, v.b          (all W stored [in,out]).
+ *               qkv_bwd adds `dres` (gradient of the `outputs += queries` residual, modules.py:269) to d(LN(x)). */
 size_t cast_block_bwd_workspace_bytes(long N, int H);
 /* cast_ffn_bwd / cast_qkv_bwd sum their per-CTA gradient partials (workspace layout [parts][count], count =
  * 2H + 2(H*H+H) resp. 2H + 3(H*H+H)) into grads_out with a fixed-order reduction launch.  With grads_out == NULL the
