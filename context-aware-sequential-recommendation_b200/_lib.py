@@ -79,6 +79,15 @@ SIGNATURES = {
     "cast_adam_tf_rows": (I, [P, P, P, P, L, I, F, F, F, F, P, P, P, P, P]),
     "cast_adam_tf_rows_peers": (I, [P, P, P, P, I, P, P, L, I, L, F, F, F, F, P, P]),
     "cast_adam_tf_range_peers": (I, [P, P, I, P, P, P, L, L, L, F, F, F, F, P, P]),
+    "cast_clip_parts": (I, []),
+    "cast_clip_sumsq_range": (I, [P, P, L, P, F, L, L, P, P]),
+    "cast_clip_sumsq_rows": (I, [P, L, I, P, P, P, P, P]),
+    "cast_clip_sumsq_rows_peers": (I, [P, P, P, I, L, I, L, P, P]),
+    "cast_clip_reduce_sumsq_peers": (I, [P, I, P, P, L, L, L, F, L, L, P, P]),
+    "cast_clip_finalize": (I, [P, I, P, I, C.c_double, P, P]),
+    "cast_adam_tf_range_clip": (I, [P, P, P, P, L, F, F, F, F, P, F, L, L, P, P, I, P]),
+    "cast_adam_tf_rows_clip": (I, [P, P, P, P, L, I, F, F, F, F, P, P, P, P, P, P]),
+    "cast_adam_tf_rows_peers_clip": (I, [P, P, P, P, I, P, P, L, I, L, F, F, F, F, P, P, P]),
     "cast_scatter_apply_lazy": (I, [I, L, P, P, P, I, I, P, P, SZ, P, SZ, P, P, P]),
     "cast_scatter_apply_range_lazy": (I, [I, L, P, P, P, I, P, P, P, C.c_uint, C.c_uint, P, SZ, P, P, P]),
     "cast_scatter_pull_range_lazy": (I, [I, L, P, P, P, I, P, P, P, C.c_uint, C.c_uint, P, SZ, P, SZ, P, P, P]),

@@ -334,6 +334,10 @@ def attach_sharded(engine, group=None, arena: "PeerArena | None" = None):
 
     engine.grad_allreduce = exchange
     engine.after_adam = px.barrier   # shards are updated; exported buffers may be overwritten
+    if engine.clip:
+        # clip_grad: every rank folds every rank's shard partials (peer mappings) after one more barrier
+        engine.clip_peers = (px.barrier, torch.tensor(arena.ptrs(engine.clip_shard_parts), dtype=torch.int64,
+                                                      device=engine.device))
     if engine.device.type == "cuda":
         torch.cuda.synchronize(engine.device)
     dist.barrier(group=group)      # every shard is initialised before anybody gathers from it

@@ -144,7 +144,15 @@ class Engine:
         correction, and leaves every other row bit for bit as it was (row 0 and a shard's pad row never move); all other
         parameters keep dense TF-Adam.  The step's table cost then follows the batch instead of the catalog.  It is a
         different optimizer (m and v of a row decay only when the row is touched), so it is opt-in; it refuses
-        l2_emb != 0, whose table-wide decay cannot be lazy."""
+        l2_emb != 0, whose table-wide decay cannot be lazy.
+
+        args.clip_grad (default False): global-norm gradient clipping with the threshold args.max_norm (the reference's
+        flag, default 5.0), as tf.clip_by_global_norm over every parameter's gradient as Adam consumes it (divided by
+        the global sum(istarget), plus l2_emb * w on the tables; under lazy_adam untouched rows count as 0; under data
+        parallelism the rank-ordered sum; with a row-sharded table every shard).  norm = sqrt(sum g^2) in fp64, Adam
+        steps on g * scale with scale = max_norm / norm if norm > max_norm else 1 (NaN for a non-finite norm).  The
+        norm, the scale and the update run on the device inside the step; a step below the threshold gives the bits of
+        clipping off."""
         self.lib = lib if lib is not None else _lib.load_library()
         self.timing = None
         if device is None:
@@ -217,6 +225,20 @@ class Engine:
         if self.optimizer == "lazy_adam":
             self.grad_epoch = torch.zeros(1, dtype=torch.int32, device=self.device)
             self.stamp = torch.zeros(self.P["item_emb"].shape[0], dtype=torch.int32, device=self.device)
+        # clip_grad: fp64 sum-of-squares partials (cast_clip_parts() per pass; a row shard's go to peer-visible memory
+        # that the other ranks fold) and the step's {scale, pre-clip norm}
+        self.clip = bool(getattr(args, "clip_grad", False))
+        self.max_norm = float(getattr(args, "max_norm", 5.0))
+        self.clip_out = self.clip_parts = self.clip_shard_parts = None
+        self.clip_peers = None      # set by dist.attach_sharded(): (barrier, device array of the ranks' shard partials)
+        if self.clip:
+            if not (math.isfinite(self.max_norm) and self.max_norm > 0):
+                raise ValueError(f"clip_grad needs a finite max_norm > 0, got {self.max_norm}")
+            self.clip_nparts = int(self.lib.cast_clip_parts())
+            self.clip_parts = torch.zeros(2 * self.clip_nparts, dtype=torch.float64, device=self.device)
+            self.clip_out = torch.zeros(2, dtype=torch.float32, device=self.device)
+            if self.item_shard is not None:
+                self.clip_shard_parts = self._peer_zeros(self.clip_nparts, torch.float64)
         self.sinus = torch.from_numpy(sinusoid_table(self.H, self.T)).to(self.device)
         self.init_parameters(self.seed or 42)
         self._call(self.lib.cast_adam_init_state, self.adam_state.data_ptr(), self.beta1, self.beta2, self._stream())
@@ -861,12 +883,12 @@ class Engine:
 
         @contextlib.contextmanager
         def cm():
-            saved = (self.grad_allreduce, self.after_adam, self.before_backward, self.peer_adam)
-            self.grad_allreduce = self.after_adam = self.before_backward = self.peer_adam = None
+            saved = (self.grad_allreduce, self.after_adam, self.before_backward, self.peer_adam, self.clip_peers)
+            self.grad_allreduce = self.after_adam = self.before_backward = self.peer_adam = self.clip_peers = None
             try:
                 yield self
             finally:
-                self.grad_allreduce, self.after_adam, self.before_backward, self.peer_adam = saved
+                self.grad_allreduce, self.after_adam, self.before_backward, self.peer_adam, self.clip_peers = saved
         return cm()
 
     def flush_reduce_jobs(self, c):
@@ -886,6 +908,9 @@ class Engine:
     def adam(self, c):
         # gradients are divided by sums[2] = sum(istarget) (global under data parallelism) inside the kernel; with a
         # row-sharded item table the flat buffers hold this rank's shard first, so the same launch updates it
+        if self.clip:
+            self.adam_clipped()
+            return
         if self.stamp is not None:
             self.adam_lazy()
             return
@@ -922,6 +947,67 @@ class Engine:
         self._call(self.lib.cast_adam_tf_range, self.w[region:].data_ptr(), g[region:].data_ptr(),
                    self.m[region:].data_ptr(), self.v[region:].data_ptr(), n - region, self.lr, self.beta1, self.beta2,
                    self.eps, gden, 0.0, 0, 0, self.adam_state.data_ptr(), 1, self._stream())
+
+    def adam_clipped(self):
+        """clip_grad: sum-of-squares passes over the gradient Adam consumes, one finalize launch that writes {scale,
+        norm} to clip_out, then the update of adam() / adam_lazy() with g * scale.  Replicated data parallelism forms
+        the rank-ordered sum into g_red in the sum-of-squares pass (the order of cast_adam_tf_step_peers) and updates
+        from there; a row-sharded table's partials go to peer-visible memory, and one more barrier lets every rank fold
+        all shards in rank order."""
+        lib, P, n, H = self.lib, self.clip_nparts, self.n_params, self.H
+        rows, region = self.P["item_emb"].shape[0], self.P["item_emb"].numel()
+        lazy = self.stamp is not None
+        l2_hi = self.l2_hi if self.l2 else 0       # lazy_adam refuses l2_emb, so 0 there
+        w, m, v, st, clip = self.w, self.m, self.v, self.adam_state.data_ptr(), self.clip_out.data_ptr()
+        part = lambda k: self.clip_parts.data_ptr() + 8 * P * k   # noqa: E731
+        opt = (self.lr, self.beta1, self.beta2, self.eps)
+        s = self._stream()
+        if self.peer_adam is not None:
+            ptrs, n_ranks, g_red = self.peer_adam
+            lo = region if lazy else 0
+            if lazy:
+                sp, ep = self.peer_stamps
+                self._call(lib.cast_clip_sumsq_rows_peers, ptrs.data_ptr(), sp.data_ptr(), ep.data_ptr(), n_ranks,
+                           rows, H, n, part(1), s)
+            self._call(lib.cast_clip_reduce_sumsq_peers, ptrs.data_ptr(), n_ranks, g_red.data_ptr(), w.data_ptr(), lo,
+                       n, g_red.numel() - n, self.l2, 0, l2_hi, part(0), s)
+            self._call(lib.cast_clip_finalize, part(0), (2 if lazy else 1) * P, None, 0, self.max_norm, clip, s)
+            if lazy:
+                self._call(lib.cast_adam_tf_rows_peers_clip, w.data_ptr(), ptrs.data_ptr(), sp.data_ptr(),
+                           ep.data_ptr(), n_ranks, m.data_ptr(), v.data_ptr(), rows, H, n, *opt, clip, st, s)
+            self._call(lib.cast_adam_tf_range_clip, w[lo:].data_ptr(), g_red[lo:].data_ptr(), m[lo:].data_ptr(),
+                       v[lo:].data_ptr(), n - lo, *opt, g_red[n + 2:].data_ptr(), self.l2, 0, l2_hi, clip, st, 1, s)
+            return
+        g, gden = self.adam_g, self.adam_g[n + 2:].data_ptr()
+        # the item table's partials: peer-visible with a row-sharded table that is attached, local otherwise
+        peers = self.clip_peers if self.item_shard is not None else None
+        tparts = self.clip_shard_parts.data_ptr() if peers is not None else part(1)
+        if lazy:
+            self._call(lib.cast_clip_sumsq_rows, g.data_ptr(), rows, H, gden, self.stamp.data_ptr(),
+                       self.grad_epoch.data_ptr(), tparts, s)
+        elif peers is not None:
+            self._call(lib.cast_clip_sumsq_range, g.data_ptr(), w.data_ptr(), region, gden, self.l2, 0,
+                       min(l2_hi, region), tparts, s)
+        else:   # one pass over the whole buffer (part(1) stays zero)
+            self._call(lib.cast_clip_sumsq_range, g.data_ptr(), w.data_ptr(), n, gden, self.l2, 0, l2_hi, part(0), s)
+        if lazy or peers is not None:
+            self._call(lib.cast_clip_sumsq_range, g[region:].data_ptr(), w[region:].data_ptr(), n - region, gden,
+                       self.l2, 0, max(l2_hi - region, 0), part(0), s)
+        if peers is not None:
+            barrier, shard_ptrs = peers
+            barrier()       # every rank's shard partials are final
+            self._call(lib.cast_clip_finalize, part(0), P, shard_ptrs.data_ptr(), self.item_shard[1], self.max_norm,
+                       clip, s)
+        else:
+            self._call(lib.cast_clip_finalize, part(0), (2 if lazy else 1) * P, None, 0, self.max_norm, clip, s)
+        if lazy:
+            self._call(lib.cast_adam_tf_rows_clip, w.data_ptr(), g.data_ptr(), m.data_ptr(), v.data_ptr(), rows, H,
+                       *opt, gden, self.stamp.data_ptr(), self.grad_epoch.data_ptr(), clip, st, s)
+            self._call(lib.cast_adam_tf_range_clip, w[region:].data_ptr(), g[region:].data_ptr(), m[region:].data_ptr(),
+                       v[region:].data_ptr(), n - region, *opt, gden, 0.0, 0, 0, clip, st, 1, s)
+        else:
+            self._call(lib.cast_adam_tf_range_clip, w.data_ptr(), g.data_ptr(), m.data_ptr(), v.data_ptr(), n, *opt,
+                       gden, self.l2, 0, l2_hi, clip, st, 1, s)
 
     def launch_fwd_bwd(self, c):
         # The sort of the (item id, entry) pairs for the embedding gradient depends on the ids only: it runs on a side

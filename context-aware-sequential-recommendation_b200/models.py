@@ -347,6 +347,14 @@ class _Model:
             return getattr(self, "_lag_cpu", None)
         return self._read_metrics(self._lag)
 
+    def last_grad_norm(self):
+        """Pre-clip global gradient norm of the most recent training step (waits for it); None when the model was built
+        without args.clip_grad."""
+        eng = self.engine
+        if not eng.clip:
+            return None
+        return float(eng.clip_out[1].item())
+
     def forward_eval(self, seq, time_seq=None, hours=None, days=None, want_attn=False, timestamps=None):
         """is_training=False forward; returns the device buffer seq_emb [B*T, H] (and fills attention weights)."""
         eng = self.engine

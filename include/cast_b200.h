@@ -369,6 +369,43 @@ int cast_adam_tf_rows_peers(float* w, const void* const* grads, const void* cons
 int cast_adam_tf_range_peers(float* w, const void* const* grads, int n_ranks, float* g_red, float* m, float* v, long lo,
                              long n, long tail, float lr, float beta1, float beta2, float eps, void* state,
                              void* stream);
+/* Global-norm gradient clipping (tf.clip_by_global_norm over the gradient Adam consumes: numerators / gdenom, plus
+ * l2*w on the l2 range), computed on the device inside the step:
+ *   cast_clip_parts                  number of fp64 partials every cast_clip_sumsq* call writes (`parts` holds that
+ *                                    many: block sums in a grid that depends on the shape only, zeros after it).
+ *   cast_clip_sumsq_range            sum of g_i^2 over i < n, g_i = grad[i] / *gdenom (+ l2*w[i] on [l2_lo, l2_hi)).
+ *   cast_clip_sumsq_rows             rows [1, rows) of a [rows, H] gradient with stamp == *epoch (lazy_adam).
+ *   cast_clip_sumsq_rows_peers       the rows of cast_adam_tf_rows_peers: rank-ordered sums over the touching ranks.
+ *   cast_clip_reduce_sumsq_peers     the reduction of cast_adam_tf_range_peers over [lo, n + tail) into g_red (rank
+ *                                    order) without the update, plus the squares of the parameters [lo, n).
+ *   cast_clip_finalize               folds nparts local partials in order and, if peer_parts is a DEVICE array of
+ *                                    n_ranks pointers to every rank's cast_clip_parts() shard partials, those rank by
+ *                                    rank; out = {scale, norm}: norm = sqrt(sum), scale = norm > max_norm ?
+ *                                    (float)(max_norm / norm) : 1, NaN if the norm is not finite.
+ *   cast_adam_tf_range_clip, cast_adam_tf_rows_clip, cast_adam_tf_rows_peers_clip
+ *                                    cast_adam_tf_range / _rows / _rows_peers with g (l2 term included) multiplied by
+ *                                    clip[0]; a scale of 1 gives their bits. */
+int cast_clip_parts(void);
+int cast_clip_sumsq_range(const float* grad, const float* w, long n, const float* gdenom, float l2, long l2_lo,
+                          long l2_hi, double* parts, void* stream);
+int cast_clip_sumsq_rows(const float* grad, long rows, int H, const float* gdenom, const unsigned* stamp,
+                         const unsigned* epoch, double* parts, void* stream);
+int cast_clip_sumsq_rows_peers(const void* const* grads, const void* const* stamps, const void* const* epochs,
+                               int n_ranks, long rows, int H, long np, double* parts, void* stream);
+int cast_clip_reduce_sumsq_peers(const void* const* grads, int n_ranks, float* g_red, const float* w, long lo, long n,
+                                 long tail, float l2, long l2_lo, long l2_hi, double* parts, void* stream);
+int cast_clip_finalize(const double* parts, int nparts, const void* const* peer_parts, int n_ranks, double max_norm,
+                       float* out, void* stream);
+int cast_adam_tf_range_clip(float* w, const float* grad, float* m, float* v, long n, float lr, float beta1,
+                            float beta2, float eps, const float* gdenom, float l2, long l2_lo, long l2_hi,
+                            const float* clip, void* state, int advance, void* stream);
+int cast_adam_tf_rows_clip(float* w, const float* grad, float* m, float* v, long rows, int H, float lr, float beta1,
+                           float beta2, float eps, const float* gdenom, const unsigned* stamp, const unsigned* epoch,
+                           const float* clip, void* state, void* stream);
+int cast_adam_tf_rows_peers_clip(float* w, const void* const* grads, const void* const* stamps,
+                                 const void* const* epochs, int n_ranks, float* m, float* v, long rows, int H, long np,
+                                 float lr, float beta1, float beta2, float eps, const float* clip, void* state,
+                                 void* stream);
 int cast_scatter_apply_lazy(int nsrc, long N, const float* const* rows, const float* const* rowscale,
                             const float* scale, int V, int H, float* dtable, void* workspace, size_t workspace_bytes,
                             void* partial, size_t partial_bytes, unsigned* stamp, const unsigned* epoch, void* stream);

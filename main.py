@@ -9,7 +9,7 @@ evaluate(test) + evaluate_valid, writing the same `params.txt` / `log.txt` files
     python -m torch.distributed.run --nproc-per-node 8 main.py ...        # data parallel, one process per GPU
 
 New flags have new names (`--eval_mode`, `--eval_every`, `--eval_batch`); every reference flag keeps its name,
-default and quirks (`--max_norm` unused, `--log_scale` / `--input_context` are `type=bool`, `--seed 0` = unseeded,
+default and quirks (`--max_norm` takes effect only with the new `--clip_grad`, `--log_scale` / `--input_context` are `type=bool`, `--seed 0` = unseeded,
 `num_batch = round(len(train) / batch_size)`).
 """
 from __future__ import annotations
@@ -41,7 +41,8 @@ def build_parser():
     p.add_argument("--batch_size", default=128, type=int, help="Batch size")
     p.add_argument("--lr", type=float, default=1e-3, help="Learning rate")
     p.add_argument("--num_epochs", type=int, default=201, help="Number of epochs")
-    p.add_argument("--max_norm", type=float, default=5.0, help="(unused, as in the reference)")
+    p.add_argument("--max_norm", type=float, default=5.0,
+                   help="global gradient norm threshold; takes effect only with --clip_grad (unused by the reference)")
     p.add_argument("--hidden_units", default=50, type=int)
     p.add_argument("--num_blocks", default=2, type=int)
     p.add_argument("--num_heads", default=1, type=int)
@@ -71,6 +72,8 @@ def build_parser():
     p.add_argument("--optimizer", default="adam", choices=["adam", "lazy_adam"],
                    help="adam = the reference's dense TF-Adam; lazy_adam = LazyAdam on the item table (only the rows a "
                    "batch touches are updated; step cost no longer grows with the catalog), dense TF-Adam elsewhere")
+    p.add_argument("--clip_grad", action="store_true", help="clip the gradient to global norm --max_norm before Adam "
+                   "(tf.clip_by_global_norm); the epoch log line then also reports TRAIN/grad_norm of its last step")
     return p
 
 
@@ -227,7 +230,10 @@ def run(args, device=None, lib=None, logger=None):
             if num_batch > 0:
                 auc, loss = model.last_metrics()
             if auc is not None:
-                logger.info("epoch:%d TRAIN/loss %.6f TRAIN/auc %.6f" % (epoch, loss, auc))
+                line = "epoch:%d TRAIN/loss %.6f TRAIN/auc %.6f" % (epoch, loss, auc)
+                if getattr(args, "clip_grad", False):
+                    line += " TRAIN/grad_norm %.6f" % model.last_grad_norm()
+                logger.info(line)
             if epoch % args.eval_every == 0:
                 if rank == 0:
                     logger.info("Model saved in path: %s" % save_checkpoint(model, args, save_path))
