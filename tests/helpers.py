@@ -85,6 +85,32 @@ def rel_err(a, b):
     return float(np.abs(a - b).max() / max(np.abs(b).max(), 1e-30))
 
 
+class WorstErrors:
+    """Largest relative error per (backend, kernel, tensor) that a test module has seen; `report` prints them (at the
+    module's teardown) past pytest's output capture, so a test log records what the tolerances had to cover."""
+
+    def __init__(self, title):
+        self.title, self.worst = title, {}
+
+    def note(self, kind, kernel, what, err, where=""):
+        key = (kind, kernel, what)
+        if err >= self.worst.get(key, (-1.0, ""))[0]:
+            self.worst[key] = (err, where)
+        return err
+
+    def report(self, config):
+        tr = config.pluginmanager.get_plugin("terminalreporter")
+        cm = config.pluginmanager.get_plugin("capturemanager")
+        if tr is None or cm is None or not self.worst:
+            return
+        with cm.global_and_fixture_disabled():
+            tr.write_line("")
+            for kind in sorted({k[0] for k in self.worst}):
+                parts = [f"{kern} {what} {e:.2e}" + (f" ({w})" if w else "")
+                         for (kd, kern, what), (e, w) in sorted(self.worst.items()) if kd == kind]
+                tr.write_line(f"{self.title} [{kind}] worst relative error vs float64: " + ", ".join(parts))
+
+
 def synth_batch(B, T, itemnum, seed, mean_len=None, max_bins=200):
     """Seeded synthetic batch in the sampler's layout (left-padded seq/pos/neg + time bins, hours, days) for parity
     runs at BASELINE.json shapes the golden fixtures (T=50, B=16) do not reach: ragged lengths (some shorter than
