@@ -113,6 +113,10 @@ SIGNATURES = {
     "cast_topk_full_workspace_bytes": (SZ, [L, I, I, I]),
     "cast_topk_full": (I, [P, L, P, I, I, L, I, P, P, I, P, P, P, P, SZ, P]),
     "cast_topk_full_status": (I, [P, L, I, I, I, P, P]),
+    "cast_item_rows": (I, [P, L, P, P, I, I, I, I, P, P]),
+    "cast_similar_items_workspace_bytes": (SZ, [L, I, I, I, I]),
+    "cast_similar_items": (I, [P, L, P, I, P, I, I, I, I, I, P, P, I, P, P, P, P, SZ, P]),
+    "cast_similar_items_status": (I, [P, L, I, I, I, P, P]),
 }
 
 

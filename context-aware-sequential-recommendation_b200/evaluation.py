@@ -185,6 +185,27 @@ def recommend_users(model, inputs, k: int, batch_users: int = 256, lo: int = 0, 
     return ids, scores
 
 
+def similar_items_all(model, k: int, batch: int = 4096, lo: int = 0, hi: Optional[int] = None,
+                      metric: str = "cosine", mode: int = 0):
+    """model.similar_items for the query items lo+1 .. hi (rows [lo, hi) of the ids 1..itemnum; hi defaults to
+    itemnum) in fixed-shape batches, the tail batch padded with item 1 (its results are dropped).
+    Returns (items [n] int32, neighbours [n,k] int32, scores [n,k] float32)."""
+    hi = model.itemnum if hi is None else hi
+    items = np.arange(lo + 1, hi + 1, dtype=np.int32)
+    n = len(items)
+    nbr = np.zeros((n, k), np.int32)
+    scores = np.zeros((n, k), np.float32)
+    B = max(1, min(batch, n))
+    for s in range(0, n, B):
+        e = min(n, s + B)
+        q = np.ones(B, np.int32)
+        q[:e - s] = items[s:e]
+        i, sc = model.similar_items(q, k, metric, mode=mode)
+        nbr[s:e] = i[:e - s]
+        scores[s:e] = sc[:e - s]
+    return items, nbr, scores
+
+
 def reference_rank(logits_row: np.ndarray) -> int:
     """util.py:318-321 verbatim semantics: rank of candidate 0 under numpy's default argsort."""
     return int((-logits_row).argsort().argsort()[0])

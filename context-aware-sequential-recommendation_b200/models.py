@@ -281,13 +281,64 @@ class _Model:
             if mode == 0:
                 self._check_watchdog(eng.lib.cast_topk_full_status, "topk_full", ws.data_ptr(), U, V, eng.H, k)
             ids = eng.global_ids(ids)
+        return self._merge_topk(ids, scores, k, c.B)
+
+    def _merge_topk(self, ids, scores, k, n):
+        """per-call top-k lists (global ids) -> (ids, scores) numpy arrays of this rank's n rows; with a row-sharded item
+        table the rows are every rank's (rank-major) and each rank's per-shard lists are merged per row by (score desc,
+        id asc)"""
+        eng = self.engine
         if eng.item_shard is None:
             return ids.cpu().numpy(), scores.cpu().numpy()
         rank, world = eng.item_shard
         all_i, all_s = (np.hstack(np.split(_all_gather(t).cpu().numpy(), world)) for t in (ids, scores))
         order = np.lexsort((all_i, -all_s), axis=-1)[:, :k]
-        mine = slice(rank * c.B, (rank + 1) * c.B)
+        mine = slice(rank * n, (rank + 1) * n)
         return np.take_along_axis(all_i, order, 1)[mine], np.take_along_axis(all_s, order, 1)[mine]
+
+    SIMILARITY = {"dot": 0, "cosine": 1}     # include/cast_b200.h CAST_SIM_*
+
+    def similar_items(self, ids, k=10, metric="cosine", mode: int = 0):
+        """Exact item-to-item top-k: for each query item q of ids, the k items j in [1, itemnum], j != q, with the
+        largest canonical score, ties broken by item id ascending (the order of recommend).  metric "dot": the
+        canonical fp32 dot of the raw item_emb rows (the training logits' rows, no sqrt(H) factor); "cosine": the
+        canonical dot of the rows normalised canonically (n = sqrt_rn of the k-ascending, separately rounded sum of
+        squares, each element divided by n, a zero row stays zero).  mode 0 = tcgen05 tensor cores as an exact filter,
+        mode 1 = exact brute force; both return the same bits.  Returns (ids [U,k] int32, scores [U,k] float32); fewer
+        than k eligible items pad the tail with id 0 and score -inf.  With a row-sharded item table this is a
+        collective call (every rank passes its own queries, the same count on every rank): the query rows are read
+        from their owners' shards, each rank takes the top k of its own shard for all queries and the lists are merged
+        as in recommend."""
+        eng = self.engine
+        dev = eng.device
+        if metric not in self.SIMILARITY:
+            raise ValueError(f"metric must be one of {sorted(self.SIMILARITY)}, got {metric!r}")
+        if not 1 <= int(k) <= 256:
+            raise ValueError(f"k must be in [1, 256], got {k}")
+        k = int(k)
+        q = np.asarray(ids).reshape(-1)
+        if q.size and (not np.issubdtype(q.dtype, np.integer) or q.min() < 1 or q.max() > self.itemnum):
+            raise ValueError(f"query ids must be integers in [1, {self.itemnum}]")
+        qd = torch.from_numpy(q.astype(np.int32)).to(dev)
+        B = qd.shape[0]
+        if eng.item_shard is not None:
+            qd = _all_gather(qd)
+        U, V = qd.shape[0], eng.item_rows
+        nbr = torch.zeros(U, k, dtype=torch.int32, device=dev)
+        scores = torch.full((U, k), float("-inf"), dtype=torch.float32, device=dev)
+        if U > 0 and V > 1:     # a shard of a catalog smaller than the world may hold no item
+            eptr, eidx = self._id_csr(qd.cpu().numpy().reshape(U, 1), U)       # the query itself, if this shard holds it
+            metric_id = self.SIMILARITY[metric]
+            wsb = eng.lib.cast_similar_items_workspace_bytes(U, V, eng.H, k, metric_id)
+            ws = self._workspace(wsb)
+            shards = (eng.shard_ptrs.data_ptr(), eng.item_shard[1]) if eng.item_shard is not None else (None, 0)
+            eng._call(eng.lib.cast_similar_items, qd.data_ptr(), U, eng.P["item_emb"].data_ptr(), V, *shards,
+                      eng.V_items, eng.H, k, metric_id, eptr.data_ptr(), eidx.data_ptr(), mode, nbr.data_ptr(),
+                      scores.data_ptr(), None, ws.data_ptr(), wsb, eng._stream())
+            if mode == 0:
+                self._check_watchdog(eng.lib.cast_similar_items_status, "similar_items", ws.data_ptr(), U, V, eng.H, k)
+            nbr = eng.global_ids(nbr)
+        return self._merge_topk(nbr, scores, k, B)
 
     # ------------------------------------------------------------------ reference protocol
     def _stage_all(self, c, seq, pos, neg, time_seq, hours, days, timestamps):

@@ -461,6 +461,32 @@ int cast_topk_full(const float* seq_last, long ld, const float* table, int V, in
 /* Synchronises the stream and reports the tensor-core passes' watchdog flag (0 = ok). */
 int cast_topk_full_status(const void* workspace, long U, int V, int H, int K, int* host_flag, void* stream);
 
+/* Rows of the item table by id: out[i] [H] = row ids[i] (ids NULL: row i), ids outside [0, V) give a zero row.  The
+ * rows come from `table` [V, H], or, when shards != NULL, from the table row-sharded over nshards ranks (device array
+ * of the shards' pointers, peer mappings included; global ids).  normalize != 0 applies the canonical normalisation:
+ * n = sqrt_rn(sum_k e_k * e_k), k ascending, multiply and add rounded separately; out_k = e_k / n (IEEE division);
+ * n == 0 gives the zero vector.  A row gets the same bits wherever it is read.  H <= 1536. */
+int cast_item_rows(const int* ids, long n, const float* table, const float* const* shards, int nshards, int V, int H,
+                   int normalize, float* out, void* stream);
+
+/* Exact item-to-item top-K.  For each query id q = ids[u] (device, [U]): the K rows j in [1, V) of `table` not in the
+ * query's exclusion row, by canonical score descending, then row ascending; top_scores are the scores bit for bit,
+ * and fewer than K eligible rows pad the tail with (0, -inf).  Score: metric CAST_SIM_DOT = the canonical dot of the
+ * raw rows e_q . e_j, CAST_SIM_COSINE = the canonical dot of the rows normalised as in cast_item_rows.  The query rows
+ * are read from `table` (global ids in [1, V)), or, when shards != NULL, from the row-sharded table of nshards ranks
+ * (global ids in [1, V_items)); `table` [V, H] is then this rank's shard and rows are its local rows.  The caller
+ * passes each query's own row in its exclusion row (excl_ptr [U+1] / excl_idx, as in cast_topk_full) to leave the
+ * query out.  mode, stats and 1 <= K <= 256 as in cast_topk_full; both modes return the same bits. */
+#define CAST_SIM_DOT 0
+#define CAST_SIM_COSINE 1
+size_t cast_similar_items_workspace_bytes(long U, int V, int H, int K, int metric);
+int cast_similar_items(const int* ids, long U, const float* table, int V, const float* const* shards, int nshards,
+                       int V_items, int H, int K, int metric, const int* excl_ptr, const int* excl_idx, int mode,
+                       int* top_ids, float* top_scores, unsigned long long* stats, void* workspace,
+                       size_t workspace_bytes, void* stream);
+/* Synchronises the stream and reports the tensor-core passes' watchdog flag (0 = ok). */
+int cast_similar_items_status(const void* workspace, long U, int V, int H, int K, int* host_flag, void* stream);
+
 #ifdef __cplusplus
 }
 #endif

@@ -69,6 +69,10 @@ def build_parser():
                    "hand raw timestamps to the device, which derives time bins / hours / weekdays there")
     p.add_argument("--recommend", default=0, type=int, help="with --test_model: after the evaluation, write the top K "
                    "items of every user (whole history excluded) to recommendations_top{K}.npz next to the checkpoint")
+    p.add_argument("--similar_items", default=0, type=int, help="with --test_model: after the evaluation, write the "
+                   "top K most similar items of every item to similar_items_top{K}.npz next to the checkpoint")
+    p.add_argument("--similarity", default="cosine", choices=["cosine", "dot"],
+                   help="item-to-item score of --similar_items: cosine of the item_emb rows, or their dot product")
     p.add_argument("--optimizer", default="adam", choices=["adam", "lazy_adam"],
                    help="adam = the reference's dense TF-Adam; lazy_adam = LazyAdam on the item table (only the rows a "
                    "batch touches are updated; step cost no longer grows with the catalog), dense TF-Adam elsewhere")
@@ -94,6 +98,24 @@ def write_recommendations(model, dataset, args, rank, world):
         scores = np.concatenate([p[1] for p in parts])
     if rank == 0:
         np.savez(os.path.join(args.test_model, "recommendations_top{}.npz".format(K)), users=rec["u"], items=ids,
+                 scores=scores)
+
+
+def write_similar_items(model, args, rank, world):
+    """--similar_items K: exact top-K neighbours (--similarity) of every item; the items are sharded over the ranks and
+    gathered; rank 0 writes items / neighbours / scores."""
+    from cast_b200 import dist as cdist
+    from cast_b200.evaluation import similar_items_all
+    K = int(args.similar_items)
+    lo, hi = cdist.shard_users(model.itemnum, rank, world)
+    items, nbr, scores = similar_items_all(model, K, args.eval_batch, lo, hi, args.similarity)
+    if world > 1:
+        import torch.distributed as tdist
+        parts = [None] * world
+        tdist.all_gather_object(parts, (items, nbr, scores))
+        items, nbr, scores = (np.concatenate([p[j] for p in parts]) for j in range(3))
+    if rank == 0:
+        np.savez(os.path.join(args.test_model, "similar_items_top{}.npz".format(K)), items=items, neighbours=nbr,
                  scores=scores)
 
 
@@ -207,6 +229,8 @@ def run(args, device=None, lib=None, logger=None):
                         f.write("{},{},{}\n".format(args.test_seq_len, t_test[0], t_test[1]))
                 if getattr(args, "recommend", 0) > 0:
                     write_recommendations(model, dataset, args, rank, world)
+                if getattr(args, "similar_items", 0) > 0:
+                    write_similar_items(model, args, rank, world)
             else:
                 print("{} not found".format(args.test_model))
         finally:
