@@ -112,10 +112,12 @@ SIGNATURES = {
     "cast_score_rank_full_status": (I, [P, L, I, P, P]),
     "cast_topk_full_workspace_bytes": (SZ, [L, I, I, I]),
     "cast_topk_full": (I, [P, L, P, I, I, L, I, P, P, I, P, P, P, P, SZ, P]),
+    "cast_topk_full_biased": (I, [P, L, P, I, I, L, I, P, P, P, I, P, P, P, P, SZ, P]),
     "cast_topk_full_status": (I, [P, L, I, I, I, P, P]),
     "cast_item_rows": (I, [P, L, P, P, I, I, I, I, P, P]),
     "cast_similar_items_workspace_bytes": (SZ, [L, I, I, I, I]),
     "cast_similar_items": (I, [P, L, P, I, P, I, I, I, I, I, P, P, I, P, P, P, P, SZ, P]),
+    "cast_similar_items_biased": (I, [P, L, P, I, P, I, I, I, I, I, P, P, P, I, P, P, P, P, SZ, P]),
     "cast_similar_items_status": (I, [P, L, I, I, I, P, P]),
 }
 

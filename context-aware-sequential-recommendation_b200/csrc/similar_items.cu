@@ -7,7 +7,8 @@
 // Canonical normalisation (the same bits for a row wherever it is read): n = sqrt_rn(sum_k e_k * e_k), k ascending,
 // multiply and add rounded separately (as canonical_dot); ê_k = e_k / n (IEEE division); n == 0 -> the zero vector.
 // Scores are then canonical_dot(ê_q, ê_j) (cosine) or canonical_dot(e_q, e_j) (dot), so both tensor-core filter and
-// brute force return those bits.
+// brute force return those bits.  cast_similar_items_biased adds a per-item offset b_j (local rows) to every score
+// exactly as cast_topk_full_biased does.
 #include "cast_rt.cuh"
 
 namespace cast {
@@ -82,16 +83,19 @@ extern "C" size_t cast_similar_items_workspace_bytes(long U, int V, int H, int K
   return si_layout(U, V, H, K, metric).total;
 }
 
-extern "C" int cast_similar_items(const int* ids, long U, const float* table, int V, const float* const* shards,
-                                  int nshards, int V_items, int H, int K, int metric, const int* excl_ptr,
-                                  const int* excl_idx, int mode, int* top_ids, float* top_scores,
-                                  unsigned long long* stats, void* workspace, size_t workspace_bytes, void* stream) {
+extern "C" int cast_similar_items_biased(const int* ids, long U, const float* table, int V, const float* const* shards,
+                                         int nshards, int V_items, int H, int K, int metric, const int* excl_ptr,
+                                         const int* excl_idx, const float* item_bias, int mode, int* top_ids,
+                                         float* top_scores, unsigned long long* stats, void* workspace,
+                                         size_t workspace_bytes, void* stream) {
   if (K < 1 || K > 256) return set_error(CAST_ERR_BAD_ARG, "similar_items: K must be in [1, 256]");
   if (metric != CAST_SIM_DOT && metric != CAST_SIM_COSINE)
     return set_error(CAST_ERR_BAD_ARG, "similar_items: metric must be CAST_SIM_DOT or CAST_SIM_COSINE");
   if (!ids || !table || U <= 0 || V <= 1 || H <= 0 || (shards && (nshards < 1 || V_items <= 1)) ||
       (size_t)SI_WARPS * H * sizeof(float) > 48 * 1024)
     return set_error(CAST_ERR_BAD_ARG, "similar_items");
+  if ((uintptr_t)item_bias % 16 != 0)
+    return set_error(CAST_ERR_BAD_ARG, "similar_items: item_bias must be 16-byte aligned");
   const SiLayout l = si_layout(U, V, H, K, metric);
   if (!workspace || workspace_bytes < l.total)
     return set_error(CAST_ERR_WORKSPACE, "similar_items: workspace too small");
@@ -108,8 +112,16 @@ extern "C" int cast_similar_items(const int* ids, long U, const float* table, in
     if ((rc = launch_item_rows(nullptr, V, table_ref(table), V, H, 1, ehat, st))) return rc;
     scored = ehat;
   }
-  return cast_topk_full(q, H, scored, V, H, U, K, excl_ptr, excl_idx, mode, top_ids, top_scores, stats, w + l.topk,
-                        l.q - l.topk, stream);
+  return cast_topk_full_biased(q, H, scored, V, H, U, K, excl_ptr, excl_idx, item_bias, mode, top_ids, top_scores,
+                               stats, w + l.topk, l.q - l.topk, stream);
+}
+
+extern "C" int cast_similar_items(const int* ids, long U, const float* table, int V, const float* const* shards,
+                                  int nshards, int V_items, int H, int K, int metric, const int* excl_ptr,
+                                  const int* excl_idx, int mode, int* top_ids, float* top_scores,
+                                  unsigned long long* stats, void* workspace, size_t workspace_bytes, void* stream) {
+  return cast_similar_items_biased(ids, U, table, V, shards, nshards, V_items, H, K, metric, excl_ptr, excl_idx,
+                                   nullptr, mode, top_ids, top_scores, stats, workspace, workspace_bytes, stream);
 }
 
 extern "C" int cast_similar_items_status(const void* workspace, long U, int V, int H, int K, int* host_flag,

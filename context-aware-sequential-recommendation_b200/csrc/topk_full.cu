@@ -15,6 +15,12 @@
 //   3. select           tk_select_kernel: canonical dot per candidate, rank by (score desc, id asc), write the top K.
 //                       A user whose buffer overflowed (or whose tau_u is -inf) takes the exact path instead.
 // Exact path (mode 1, and the fallback): brute-force canonical dots with a block-wide running top K.
+//
+// Item bias (the `Biased` instantiations, cast_topk_full_biased): the score of item j becomes fl(s(u,j) + b_j), one
+// fp32 addition rounded to nearest, and b_j == -inf removes item j.  x -> fl(x + b_j) is monotone, so the biased
+// bounds fl(fl(s~ - d) + b_j) <= fl(s + b_j) <= fl(fl(s~ + d) + b_j) keep every step above exact; an item with
+// b_j == -inf has no finite bound, so it never enters a list or a buffer.  Without a bias the unbiased
+// instantiations run, the kernels of the unbiased library.
 #include "score_full.cuh"
 
 namespace cast {
@@ -41,6 +47,22 @@ __device__ __forceinline__ bool tk_excluded(const int* __restrict__ eptr, const 
   return lo < end && eidx[lo] == j;
 }
 
+// b[j .. j+31] of a chunk: each lane of a warp is a different user on the same 32 columns, so these are broadcast
+// loads (16-byte aligned: j is a multiple of 32 and the bias array 16-byte aligned); items at or past `end` read -inf
+__device__ __forceinline__ void tk_bias_chunk(const float* __restrict__ bias, int j, int end, float (&b)[32]) {
+  if (j + 32 <= end) {
+    const float4* q = reinterpret_cast<const float4*>(bias + j);
+#pragma unroll
+    for (int i = 0; i < 8; ++i) {
+      const float4 x = __ldg(q + i);
+      b[4 * i] = x.x; b[4 * i + 1] = x.y; b[4 * i + 2] = x.z; b[4 * i + 3] = x.w;
+    }
+  } else {
+#pragma unroll
+    for (int e = 0; e < 32; ++e) b[e] = j + e < end ? __ldg(bias + j + e) : tk_ninf();
+  }
+}
+
 // result order: score descending, then id ascending (ids are distinct, so this is a strict total order)
 __device__ __forceinline__ bool tk_before(float s, int i, float t, int j) { return s > t || (s == t && i < j); }
 
@@ -57,10 +79,12 @@ __device__ __forceinline__ void tk_rank_scatter(const float* s, const int* id, i
 
 // Exact top K of user u by brute force (whole block).  Items arrive in id order, so a new item enters the list only
 // with a score strictly above the current K-th.  smem: H floats, then two (score, id) arrays of K + blockDim entries.
+// Biased: eligibility (b_j != -inf, not excluded) is tested before the dot, so ineligible items cost one load.
+template <bool Biased>
 __device__ void tk_exact_user(const float* __restrict__ urow, const float* __restrict__ table, int V, int H, int K,
                               const int* __restrict__ eptr, const int* __restrict__ eidx, long u,
                               unsigned char* smem, int* n_sh, int* add_sh, int* __restrict__ out_id,
-                              float* __restrict__ out_s) {
+                              float* __restrict__ out_s, const float* __restrict__ bias) {
   const int T = blockDim.x;
   float* us = reinterpret_cast<float*>(smem);
   float* as = us + ((H + 3) & ~3);
@@ -76,7 +100,13 @@ __device__ void tk_exact_user(const float* __restrict__ urow, const float* __res
     const long j = base + threadIdx.x;
     bool take = false;
     float s = 0.f;
-    if (j < V && !tk_excluded(eptr, eidx, u, (int)j)) {
+    if constexpr (Biased) {
+      const float b = j < V ? __ldg(bias + j) : tk_ninf();
+      if (b != tk_ninf() && !tk_excluded(eptr, eidx, u, (int)j)) {
+        s = __fadd_rn(canonical_dot(us, table + j * H, H), b);
+        take = n < K || s > kth;
+      }
+    } else if (j < V && !tk_excluded(eptr, eidx, u, (int)j)) {
       s = canonical_dot(us, table + j * H, H);
       take = n < K || s > kth;
     }
@@ -105,28 +135,33 @@ __device__ void tk_exact_user(const float* __restrict__ urow, const float* __res
 
 static size_t tk_exact_smem(int H, int K) { return (size_t)((H + 3) & ~3) * 4 + 4 * (size_t)(K + TK_THREADS) * 4; }
 
-// mode 1: one CTA per user
+// mode 1: one CTA per user (the bias is the last parameter, so the unbiased kernel's parameter layout is unchanged)
+template <bool Biased>
 __global__ void __launch_bounds__(TK_THREADS) tk_exact_kernel(const float* __restrict__ users, long ldu,
                                                                const float* __restrict__ table, int V, int H, int K,
                                                                const int* __restrict__ eptr,
                                                                const int* __restrict__ eidx, int* __restrict__ top_ids,
-                                                               float* __restrict__ top_scores) {
+                                                               float* __restrict__ top_scores,
+                                                               const float* __restrict__ bias) {
   CAST_DYN_SMEM(unsigned char, sm);
   __shared__ int n_sh, add_sh;
   const long u = blockIdx.x;
-  tk_exact_user(users + u * ldu, table, V, H, K, eptr, eidx, u, sm, &n_sh, &add_sh, top_ids + u * K,
-                top_scores + u * K);
+  tk_exact_user<Biased>(users + u * ldu, table, V, H, K, eptr, eidx, u, sm, &n_sh, &add_sh, top_ids + u * K,
+                        top_scores + u * K, bias);
 }
 
 #ifndef CAST_EMU
 // ------------------------------------------------------------------------------------------------ tensor-core path
-// threshold pass: top-TK_R lower bounds s~ - d per (thread, work unit), written to lbs[user][split][half][TK_R]
+// threshold pass: top-TK_R lower bounds s~ - d (biased: fl(fl(s~ - d) + b_j)) per (thread, work unit), written to
+// lbs[user][split][half][TK_R]
+template <bool Biased>
 struct BoundEpi {
   struct Params {
     const int* eptr;
     const int* eidx;
     float* lbs;
     int nslot;   // 2 * nsplit
+    const float* bias;
   };
   const Params& p;
   const long me;
@@ -144,6 +179,33 @@ struct BoundEpi {
   __device__ __forceinline__ void tile(int, float d_) { d = d_; }
 
   __device__ __forceinline__ void chunk(const float (&v)[32], int j) {
+    if constexpr (Biased) {
+      float w[32];   // the chunk's biased lower bounds; b_j == -inf gives -inf, which never enters the list
+      tk_bias_chunk(p.bias, j, je, w);
+      unsigned m = 0;
+#pragma unroll
+      for (int e = 0; e < 32; ++e) {
+        w[e] = __fadd_rn(v[e] - d, w[e]);
+        m |= (w[e] > top[TK_R - 1]) ? (1u << e) : 0u;
+      }
+      while (m) {
+        const int e = __ffs((int)m) - 1;
+        m &= m - 1;
+        float x = w[0];
+#pragma unroll
+        for (int k = 1; k < 32; ++k) x = k == e ? w[k] : x;
+        const int item = j + e;
+        if (x > top[TK_R - 1] && item >= 1 && item < je && !tk_excluded(p.eptr, p.eidx, me, item)) {
+#pragma unroll
+          for (int i = 0; i < TK_R; ++i) {
+            const float hi = fmaxf(top[i], x);
+            x = fminf(top[i], x);
+            top[i] = hi;
+          }
+        }
+      }
+      return;
+    }
     unsigned m = 0;
 #pragma unroll
     for (int e = 0; e < 32; ++e) m |= (v[e] - d > top[TK_R - 1]) ? (1u << e) : 0u;
@@ -173,7 +235,9 @@ struct BoundEpi {
   }
 };
 
-// admission pass: eligible items with s~ + d >= tau_u are appended to the user's candidate buffer
+// admission pass: eligible items with s~ + d >= tau_u (biased: fl(fl(s~ + d) + b_j) >= tau_u) are appended to the
+// user's candidate buffer
+template <bool Biased>
 struct AdmitEpi {
   struct Params {
     const int* eptr;
@@ -182,6 +246,7 @@ struct AdmitEpi {
     int* cnt;
     int* cand;   // [U, cap]
     int cap;
+    const float* bias;
   };
   const Params& p;
   const long me;
@@ -197,8 +262,15 @@ struct AdmitEpi {
   __device__ __forceinline__ void chunk(const float (&v)[32], int j) {
     if (tau == tk_ninf()) return;   // the user is already on the exact path
     unsigned m = 0;
+    if constexpr (Biased) {   // tau_u is finite here, so b_j == -inf never passes
+      float b[32];
+      tk_bias_chunk(p.bias, j, je, b);
 #pragma unroll
-    for (int e = 0; e < 32; ++e) m |= (v[e] + d >= tau) ? (1u << e) : 0u;
+      for (int e = 0; e < 32; ++e) m |= (__fadd_rn(v[e] + d, b[e]) >= tau) ? (1u << e) : 0u;
+    } else {
+#pragma unroll
+      for (int e = 0; e < 32; ++e) m |= (v[e] + d >= tau) ? (1u << e) : 0u;
+    }
     while (m) {
       const int e = __ffs((int)m) - 1;
       m &= m - 1;
@@ -260,7 +332,9 @@ __global__ void tk_tau_kernel(const float* __restrict__ lbs, int n, long U, int 
   }
 }
 
-// one CTA per user: canonical dots of the admitted candidates, ranked; overflowed users take the exact path
+// one CTA per user: canonical dots (biased: + b_j) of the admitted candidates, ranked; overflowed users take the
+// exact path
+template <bool Biased>
 __global__ void __launch_bounds__(TK_THREADS) tk_select_kernel(const float* __restrict__ users, long ldu,
                                                                 const float* __restrict__ table, int V, int H, int K,
                                                                 const int* __restrict__ eptr,
@@ -269,7 +343,8 @@ __global__ void __launch_bounds__(TK_THREADS) tk_select_kernel(const float* __re
                                                                 const int* __restrict__ cand, int cap,
                                                                 int* __restrict__ top_ids,
                                                                 float* __restrict__ top_scores,
-                                                                unsigned long long* __restrict__ stats) {
+                                                                unsigned long long* __restrict__ stats,
+                                                                const float* __restrict__ bias) {
   CAST_DYN_SMEM(unsigned char, sm);
   __shared__ int n_sh, add_sh;
   const long u = blockIdx.x;
@@ -278,7 +353,7 @@ __global__ void __launch_bounds__(TK_THREADS) tk_select_kernel(const float* __re
   float* osc = top_scores + u * K;
   if (c > cap) {
     if (stats && threadIdx.x == 0) atomicAdd(&stats[1], 1ull);
-    tk_exact_user(users + u * ldu, table, V, H, K, eptr, eidx, u, sm, &n_sh, &add_sh, oid, osc);
+    tk_exact_user<Biased>(users + u * ldu, table, V, H, K, eptr, eidx, u, sm, &n_sh, &add_sh, oid, osc, bias);
     return;
   }
   if (stats && threadIdx.x == 0 && c) atomicAdd(&stats[0], (unsigned long long)c);
@@ -287,7 +362,8 @@ __global__ void __launch_bounds__(TK_THREADS) tk_select_kernel(const float* __re
   const float* ur = users + u * ldu;
   for (int i = threadIdx.x; i < c; i += blockDim.x) {
     const int j = cand[(size_t)u * cap + i];
-    cs[i] = canonical_dot(ur, table + (long)j * H, H);
+    const float s = canonical_dot(ur, table + (long)j * H, H);
+    cs[i] = Biased ? __fadd_rn(s, __ldg(bias + j)) : s;
     ci[i] = j;
   }
   __syncthreads();
@@ -330,25 +406,11 @@ static TkLayout tk_layout(long U, int V, int H, int K) {
   return l;
 }
 
-}  // namespace cast
-
-using namespace cast;
-
-extern "C" size_t cast_topk_full_workspace_bytes(long U, int V, int H, int K) {
-  if (U <= 0 || V <= 1 || H <= 0 || K < 1 || K > TK_MAXK) return 0;
-  return tk_layout(U, V, H, K).total;
-}
-
-extern "C" int cast_topk_full(const float* seq_last, long ld, const float* table, int V, int H, long U, int K,
-                              const int* excl_ptr, const int* excl_idx, int mode, int* top_ids, float* top_scores,
-                              unsigned long long* stats, void* workspace, size_t workspace_bytes, void* stream) {
-  if (K < 1 || K > TK_MAXK) return set_error(CAST_ERR_BAD_ARG, "topk_full: K must be in [1, 256]");
-  if (!seq_last || !table || !top_ids || !top_scores || V <= 1 || H <= 0 || U <= 0 || ld < H ||
-      (mode != 0 && mode != 1) || (excl_ptr && !excl_idx))
-    return set_error(CAST_ERR_BAD_ARG, "topk_full");
-  const TkLayout l = tk_layout(U, V, H, K);
-  if (!workspace || workspace_bytes < l.total) return set_error(CAST_ERR_WORKSPACE, "topk_full: workspace too small");
-  cudaStream_t st = (cudaStream_t)stream;
+// the launches of one call, arguments checked by the caller
+template <bool Biased>
+static int tk_run(const float* seq_last, long ld, const float* table, int V, int H, long U, int K, const int* excl_ptr,
+                  const int* excl_idx, const float* bias, int mode, int* top_ids, float* top_scores,
+                  unsigned long long* stats, void* workspace, const TkLayout& l, cudaStream_t st) {
   unsigned char* w = static_cast<unsigned char*>(workspace);
   int* err = reinterpret_cast<int*>(w);
   int rc;
@@ -358,8 +420,8 @@ extern "C" int cast_topk_full(const float* seq_last, long ld, const float* table
   mode = 1;  // the host emulation has no tensor cores; the exact path defines the same result
 #endif
   if (mode == 1) {
-    CAST_LAUNCH(tk_exact_kernel, dim3((unsigned)U), dim3(TK_THREADS), tk_exact_smem(H, K), st, seq_last, ld, table, V,
-                H, K, excl_ptr, excl_idx, top_ids, top_scores);
+    CAST_LAUNCH(tk_exact_kernel<Biased>, dim3((unsigned)U), dim3(TK_THREADS), tk_exact_smem(H, K), st, seq_last, ld,
+                table, V, H, K, excl_ptr, excl_idx, top_ids, top_scores, bias);
     return check_launch("topk_full(exact)");
   }
 #ifndef CAST_EMU
@@ -378,21 +440,57 @@ extern "C" int cast_topk_full(const float* seq_last, long ld, const float* table
   const long nsplit = tk_nsplit(U, V, K);
   sf_set_split(a, nsplit);
   if (a.nsplit != nsplit) return set_error(CAST_ERR_BAD_ARG, "topk_full: split plan mismatch");
-  BoundEpi::Params bp{excl_ptr, excl_idx, lbs, 2 * a.nsplit};
-  if ((rc = sf_launch<BoundEpi>(a, bp, st, "topk_full(threshold)"))) return rc;
+  const typename BoundEpi<Biased>::Params bp{excl_ptr, excl_idx, lbs, 2 * a.nsplit, bias};
+  if ((rc = sf_launch<BoundEpi<Biased>>(a, bp, st, "topk_full(threshold)"))) return rc;
   const int cap = tk_cap(K);
   tk_tau_kernel<<<dim3((unsigned)cdiv(U, 4)), dim3(128), 0, st>>>(lbs, 2 * a.nsplit * TK_R, U, K, cap, tau, cnt);
   if ((rc = check_launch("topk_full(tau)"))) return rc;
-  AdmitEpi::Params ap{excl_ptr, excl_idx, tau, cnt, cand, cap};
-  if ((rc = sf_launch<AdmitEpi>(a, ap, st, "topk_full(admit)"))) return rc;
+  const typename AdmitEpi<Biased>::Params ap{excl_ptr, excl_idx, tau, cnt, cand, cap, bias};
+  if ((rc = sf_launch<AdmitEpi<Biased>>(a, ap, st, "topk_full(admit)"))) return rc;
   size_t smem = tk_exact_smem(H, K);
   if (smem < (size_t)cap * 8) smem = (size_t)cap * 8;
-  tk_select_kernel<<<dim3((unsigned)U), dim3(TK_THREADS), smem, st>>>(seq_last, ld, table, V, H, K, excl_ptr, excl_idx,
-                                                                      cnt, cand, cap, top_ids, top_scores, stats);
+  tk_select_kernel<Biased><<<dim3((unsigned)U), dim3(TK_THREADS), smem, st>>>(
+      seq_last, ld, table, V, H, K, excl_ptr, excl_idx, cnt, cand, cap, top_ids, top_scores, stats, bias);
   return check_launch("topk_full(select)");
 #else
   return CAST_OK;
 #endif
+}
+
+}  // namespace cast
+
+using namespace cast;
+
+extern "C" size_t cast_topk_full_workspace_bytes(long U, int V, int H, int K) {
+  if (U <= 0 || V <= 1 || H <= 0 || K < 1 || K > TK_MAXK) return 0;
+  return tk_layout(U, V, H, K).total;
+}
+
+extern "C" int cast_topk_full_biased(const float* seq_last, long ld, const float* table, int V, int H, long U, int K,
+                                     const int* excl_ptr, const int* excl_idx, const float* item_bias, int mode,
+                                     int* top_ids, float* top_scores, unsigned long long* stats, void* workspace,
+                                     size_t workspace_bytes, void* stream) {
+  if (K < 1 || K > TK_MAXK) return set_error(CAST_ERR_BAD_ARG, "topk_full: K must be in [1, 256]");
+  if (!seq_last || !table || !top_ids || !top_scores || V <= 1 || H <= 0 || U <= 0 || ld < H ||
+      (mode != 0 && mode != 1) || (excl_ptr && !excl_idx))
+    return set_error(CAST_ERR_BAD_ARG, "topk_full");
+  if ((uintptr_t)item_bias % 16 != 0)
+    return set_error(CAST_ERR_BAD_ARG, "topk_full: item_bias must be 16-byte aligned");
+  const TkLayout l = tk_layout(U, V, H, K);
+  if (!workspace || workspace_bytes < l.total) return set_error(CAST_ERR_WORKSPACE, "topk_full: workspace too small");
+  cudaStream_t st = (cudaStream_t)stream;
+  if (item_bias)
+    return tk_run<true>(seq_last, ld, table, V, H, U, K, excl_ptr, excl_idx, item_bias, mode, top_ids, top_scores,
+                        stats, workspace, l, st);
+  return tk_run<false>(seq_last, ld, table, V, H, U, K, excl_ptr, excl_idx, nullptr, mode, top_ids, top_scores, stats,
+                       workspace, l, st);
+}
+
+extern "C" int cast_topk_full(const float* seq_last, long ld, const float* table, int V, int H, long U, int K,
+                              const int* excl_ptr, const int* excl_idx, int mode, int* top_ids, float* top_scores,
+                              unsigned long long* stats, void* workspace, size_t workspace_bytes, void* stream) {
+  return cast_topk_full_biased(seq_last, ld, table, V, H, U, K, excl_ptr, excl_idx, nullptr, mode, top_ids, top_scores,
+                               stats, workspace, workspace_bytes, stream);
 }
 
 // 0 = ok; non-zero = a tensor-core pass timed out waiting for its MMAs (never expected; results invalid)

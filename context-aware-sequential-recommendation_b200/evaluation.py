@@ -171,26 +171,30 @@ def _batches(model, rows, batch_users: int, lo: int, hi: int):
 
 
 def recommend_users(model, inputs, k: int, batch_users: int = 256, lo: int = 0, hi: Optional[int] = None,
-                    mode: int = 0):
+                    mode: int = 0, item_bias=None):
     """model.recommend over rows [lo, hi) of build_recommend_inputs' output, with each user's history excluded; fixed
-    batch shape (tail padded as in score_users).  Returns (ids [n,k] int32, scores [n,k] float32)."""
+    batch shape (tail padded as in score_users); item_bias as in model.recommend, validated and moved to the device
+    once for all batches.  Returns (ids [n,k] int32, scores [n,k] float32)."""
     hi = len(inputs["u"]) if hi is None else hi
+    bias = model.prepare_item_bias(item_bias)
     ids = np.zeros((max(0, hi - lo), k), np.int32)
     scores = np.zeros((max(0, hi - lo), k), np.float32)
     for out, pad, feats in _batches(model, inputs, batch_users, lo, hi):
         n = out.stop - out.start
-        i, sc = model.recommend(pad("seq"), k, pad("rated"), mode=mode, **feats)
+        i, sc = model.recommend(pad("seq"), k, pad("rated"), mode=mode, item_bias=bias, **feats)
         ids[out] = i[:n]
         scores[out] = sc[:n]
     return ids, scores
 
 
 def similar_items_all(model, k: int, batch: int = 4096, lo: int = 0, hi: Optional[int] = None,
-                      metric: str = "cosine", mode: int = 0):
+                      metric: str = "cosine", mode: int = 0, item_bias=None):
     """model.similar_items for the query items lo+1 .. hi (rows [lo, hi) of the ids 1..itemnum; hi defaults to
-    itemnum) in fixed-shape batches, the tail batch padded with item 1 (its results are dropped).
+    itemnum) in fixed-shape batches, the tail batch padded with item 1 (its results are dropped); item_bias as in
+    model.similar_items, validated and moved to the device once for all batches.
     Returns (items [n] int32, neighbours [n,k] int32, scores [n,k] float32)."""
     hi = model.itemnum if hi is None else hi
+    bias = model.prepare_item_bias(item_bias)
     items = np.arange(lo + 1, hi + 1, dtype=np.int32)
     n = len(items)
     nbr = np.zeros((n, k), np.int32)
@@ -200,7 +204,7 @@ def similar_items_all(model, k: int, batch: int = 4096, lo: int = 0, hi: Optiona
         e = min(n, s + B)
         q = np.ones(B, np.int32)
         q[:e - s] = items[s:e]
-        i, sc = model.similar_items(q, k, metric, mode=mode)
+        i, sc = model.similar_items(q, k, metric, mode=mode, item_bias=bias)
         nbr[s:e] = i[:e - s]
         scores[s:e] = sc[:e - s]
     return items, nbr, scores

@@ -33,6 +33,36 @@ def _all_gather_lists(lists):
     return None if lists is None else [r for p in parts for r in p]
 
 
+def check_item_bias(item_bias, itemnum: int) -> torch.Tensor:
+    """An item_bias of recommend / similar_items (numpy array or torch tensor of itemnum + 1 reals; entry 0 is ignored)
+    rounded once to float32, on the device it came from.  Raises ValueError for a wrong shape, a non-real dtype, or a
+    NaN or +inf anywhere after the rounding (-inf removes an item)."""
+    if isinstance(item_bias, torch.Tensor):
+        t = item_bias
+        real = not (t.dtype == torch.bool or t.is_complex())
+    else:
+        a = np.asarray(item_bias)
+        real = a.dtype.kind in "fiu"
+        t = torch.from_numpy(np.ascontiguousarray(a)) if real else None
+    if not real:
+        raise ValueError(f"item_bias must hold real numbers, got dtype {(t if t is not None else a).dtype}")
+    if t.dim() != 1 or t.shape[0] != itemnum + 1:
+        raise ValueError(f"item_bias must have shape ({itemnum + 1},) (itemnum + 1), got {tuple(t.shape)}")
+    t = t.to(torch.float32)
+    if bool((torch.isnan(t) | torch.isposinf(t)).any()):
+        raise ValueError("item_bias must hold no NaN or +inf (-inf removes an item)")
+    return t
+
+
+class ItemBias:
+    """An item_bias validated and laid out for one model's item table: float32 on its device, one entry per row of
+    this process's table (b[global id of the row]).  Model.prepare_item_bias makes one; recommend / similar_items
+    accept it in place of the array, so a loop of calls validates and copies the bias once."""
+
+    def __init__(self, engine, rows: torch.Tensor):
+        self.engine, self.rows = engine, rows
+
+
 class _Model:
     registry_name = "sasrec"
 
@@ -185,6 +215,18 @@ class _Model:
         idx = np.concatenate(flat + [np.zeros(1, np.int64)]).astype(np.int32)
         return torch.from_numpy(ptr).to(eng.device), torch.from_numpy(idx).to(eng.device)
 
+    def prepare_item_bias(self, item_bias) -> Optional[ItemBias]:
+        """item_bias (see check_item_bias; None -> None) -> ItemBias for this model.  With a row-sharded item table each
+        rank keeps b[global ids of its local rows], gathered on the device; every rank passes the same array."""
+        if item_bias is None or isinstance(item_bias, ItemBias):
+            if item_bias is not None and item_bias.engine is not self.engine:
+                raise ValueError("item_bias was prepared for another model")
+            return item_bias
+        eng = self.engine
+        full = check_item_bias(item_bias, self.itemnum).to(eng.device)
+        rows = eng.global_ids(torch.arange(eng.item_rows, device=eng.device))
+        return ItemBias(eng, full[rows])     # a new contiguous tensor: 16-byte aligned, as the kernels require
+
     # ------------------------------------------------------------------ full catalog
     # With a row-sharded item table (SURVEY §8e row 3, config 5) score_full_catalog and recommend are collective calls:
     # every rank passes its own users (the same count on every rank), the last-position rows of all ranks are
@@ -254,16 +296,23 @@ class _Model:
         mine = slice(rank * c.B, (rank + 1) * c.B)
         return both[0, mine].cpu().numpy(), both[1, mine].cpu().numpy()
 
-    def recommend(self, seq, k=10, exclude=None, time_seq=None, hours=None, days=None, timestamps=None, mode: int = 0):
+    def recommend(self, seq, k=10, exclude=None, time_seq=None, hours=None, days=None, timestamps=None, mode: int = 0,
+                  item_bias=None):
         """Exact top-k recommendation from the last position of each sequence: the k items of [1, itemnum] not in
         exclude[u] (optional, one id collection per user) with the largest canonical fp32 logits (the logits of
         score_candidates / predict), ties broken by item id ascending.  mode 0 = tcgen05 tensor cores as an exact
         filter, mode 1 = exact brute force; both return the same bits.  Returns (ids [U,k] int32, scores [U,k] float32);
         fewer than k eligible items pad the tail with id 0 and score -inf.  With a row-sharded item table each rank
         takes the top k of its own shard (local rows -> global ids, an increasing map, so the tie order holds) and the
-        ranks' lists are merged per user by (score desc, id asc)."""
+        ranks' lists are merged per user by (score desc, id asc).
+        item_bias (optional, itemnum + 1 reals or an ItemBias): the score of item j becomes fl(logit + b_j), one fp32
+        addition, and b_j = -inf removes item j (catalog-wide deny / allow lists, popularity corrections, boosts).  A
+        zero bias returns the same ids and equal scores (in IEEE arithmetic fl(-0 + 0) = +0; the canonical logit is never
+        -0, so in practice the bits are equal too)."""
         eng = self.engine
         dev = eng.device
+        bias = self.prepare_item_bias(item_bias)
+        brows = None if bias is None else bias.rows
         c = self.forward_eval(seq, time_seq, hours, days, timestamps=timestamps)
         last, ld = self._last_rows(c)
         U, V = last.shape[0], eng.item_rows
@@ -275,9 +324,9 @@ class _Model:
             eptr, eidx = self._id_csr(exclude, U) if exclude is not None else (None, None)
             wsb = eng.lib.cast_topk_full_workspace_bytes(U, V, eng.H, k)
             ws = self._workspace(wsb)
-            eng._call(eng.lib.cast_topk_full, last.data_ptr(), ld, eng.P["item_emb"].data_ptr(), V, eng.H, U, k,
-                      eng._p(eptr), eng._p(eidx), mode, ids.data_ptr(), scores.data_ptr(), None, ws.data_ptr(), wsb,
-                      eng._stream())
+            eng._call(eng.lib.cast_topk_full_biased, last.data_ptr(), ld, eng.P["item_emb"].data_ptr(), V, eng.H, U, k,
+                      eng._p(eptr), eng._p(eidx), eng._p(brows), mode, ids.data_ptr(), scores.data_ptr(),
+                      None, ws.data_ptr(), wsb, eng._stream())
             if mode == 0:
                 self._check_watchdog(eng.lib.cast_topk_full_status, "topk_full", ws.data_ptr(), U, V, eng.H, k)
             ids = eng.global_ids(ids)
@@ -298,7 +347,7 @@ class _Model:
 
     SIMILARITY = {"dot": 0, "cosine": 1}     # include/cast_b200.h CAST_SIM_*
 
-    def similar_items(self, ids, k=10, metric="cosine", mode: int = 0):
+    def similar_items(self, ids, k=10, metric="cosine", mode: int = 0, item_bias=None):
         """Exact item-to-item top-k: for each query item q of ids, the k items j in [1, itemnum], j != q, with the
         largest canonical score, ties broken by item id ascending (the order of recommend).  metric "dot": the
         canonical fp32 dot of the raw item_emb rows (the training logits' rows, no sqrt(H) factor); "cosine": the
@@ -308,7 +357,7 @@ class _Model:
         than k eligible items pad the tail with id 0 and score -inf.  With a row-sharded item table this is a
         collective call (every rank passes its own queries, the same count on every rank): the query rows are read
         from their owners' shards, each rank takes the top k of its own shard for all queries and the lists are merged
-        as in recommend."""
+        as in recommend.  item_bias as in recommend: the score of j becomes fl(score + b_j), b_j = -inf removes j."""
         eng = self.engine
         dev = eng.device
         if metric not in self.SIMILARITY:
@@ -319,6 +368,8 @@ class _Model:
         q = np.asarray(ids).reshape(-1)
         if q.size and (not np.issubdtype(q.dtype, np.integer) or q.min() < 1 or q.max() > self.itemnum):
             raise ValueError(f"query ids must be integers in [1, {self.itemnum}]")
+        bias = self.prepare_item_bias(item_bias)
+        brows = None if bias is None else bias.rows
         qd = torch.from_numpy(q.astype(np.int32)).to(dev)
         B = qd.shape[0]
         if eng.item_shard is not None:
@@ -332,9 +383,9 @@ class _Model:
             wsb = eng.lib.cast_similar_items_workspace_bytes(U, V, eng.H, k, metric_id)
             ws = self._workspace(wsb)
             shards = (eng.shard_ptrs.data_ptr(), eng.item_shard[1]) if eng.item_shard is not None else (None, 0)
-            eng._call(eng.lib.cast_similar_items, qd.data_ptr(), U, eng.P["item_emb"].data_ptr(), V, *shards,
-                      eng.V_items, eng.H, k, metric_id, eptr.data_ptr(), eidx.data_ptr(), mode, nbr.data_ptr(),
-                      scores.data_ptr(), None, ws.data_ptr(), wsb, eng._stream())
+            eng._call(eng.lib.cast_similar_items_biased, qd.data_ptr(), U, eng.P["item_emb"].data_ptr(), V, *shards,
+                      eng.V_items, eng.H, k, metric_id, eptr.data_ptr(), eidx.data_ptr(), eng._p(brows),
+                      mode, nbr.data_ptr(), scores.data_ptr(), None, ws.data_ptr(), wsb, eng._stream())
             if mode == 0:
                 self._check_watchdog(eng.lib.cast_similar_items_status, "similar_items", ws.data_ptr(), U, V, eng.H, k)
             nbr = eng.global_ids(nbr)

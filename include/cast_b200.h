@@ -458,6 +458,14 @@ size_t cast_topk_full_workspace_bytes(long U, int V, int H, int K);
 int cast_topk_full(const float* seq_last, long ld, const float* table, int V, int H, long U, int K,
                    const int* excl_ptr, const int* excl_idx, int mode, int* top_ids, float* top_scores,
                    unsigned long long* stats, void* workspace, size_t workspace_bytes, void* stream);
+/* cast_topk_full with a per-item score offset: item_bias (device, [V], 16-byte aligned, NULL = none) in the rows of
+ * `table`.  The score of row j is fl(s(u,j) + item_bias[j]), one fp32 addition rounded to nearest; rows with
+ * item_bias[j] == -inf are never returned; order, padding, modes and stats as in cast_topk_full (both modes return the
+ * same bits).  item_bias must hold no NaN or +inf.  Workspace and status as for cast_topk_full. */
+int cast_topk_full_biased(const float* seq_last, long ld, const float* table, int V, int H, long U, int K,
+                          const int* excl_ptr, const int* excl_idx, const float* item_bias, int mode, int* top_ids,
+                          float* top_scores, unsigned long long* stats, void* workspace, size_t workspace_bytes,
+                          void* stream);
 /* Synchronises the stream and reports the tensor-core passes' watchdog flag (0 = ok). */
 int cast_topk_full_status(const void* workspace, long U, int V, int H, int K, int* host_flag, void* stream);
 
@@ -484,6 +492,12 @@ int cast_similar_items(const int* ids, long U, const float* table, int V, const 
                        int V_items, int H, int K, int metric, const int* excl_ptr, const int* excl_idx, int mode,
                        int* top_ids, float* top_scores, unsigned long long* stats, void* workspace,
                        size_t workspace_bytes, void* stream);
+/* cast_similar_items with a per-item score offset item_bias (device, [V] in the rows of `table`, 16-byte aligned,
+ * NULL = none), applied as in cast_topk_full_biased.  Workspace and status as for cast_similar_items. */
+int cast_similar_items_biased(const int* ids, long U, const float* table, int V, const float* const* shards,
+                              int nshards, int V_items, int H, int K, int metric, const int* excl_ptr,
+                              const int* excl_idx, const float* item_bias, int mode, int* top_ids, float* top_scores,
+                              unsigned long long* stats, void* workspace, size_t workspace_bytes, void* stream);
 /* Synchronises the stream and reports the tensor-core passes' watchdog flag (0 = ok). */
 int cast_similar_items_status(const void* workspace, long U, int V, int H, int K, int* host_flag, void* stream);
 

@@ -73,12 +73,24 @@ def build_parser():
                    "top K most similar items of every item to similar_items_top{K}.npz next to the checkpoint")
     p.add_argument("--similarity", default="cosine", choices=["cosine", "dot"],
                    help="item-to-item score of --similar_items: cosine of the item_emb rows, or their dot product")
+    p.add_argument("--item_bias", default=None, help="with --recommend / --similar_items: a .npy of itemnum + 1 "
+                   "reals (entry 0 ignored) added to every score of item j (-inf removes item j: deny / allow lists; "
+                   "e.g. -a*log(1+count) corrects for popularity); NaN or +inf is rejected")
     p.add_argument("--optimizer", default="adam", choices=["adam", "lazy_adam"],
                    help="adam = the reference's dense TF-Adam; lazy_adam = LazyAdam on the item table (only the rows a "
                    "batch touches are updated; step cost no longer grows with the catalog), dense TF-Adam elsewhere")
     p.add_argument("--clip_grad", action="store_true", help="clip the gradient to global norm --max_norm before Adam "
                    "(tf.clip_by_global_norm); the epoch log line then also reports TRAIN/grad_norm of its last step")
     return p
+
+
+def load_item_bias(args, itemnum):
+    """--item_bias FILE.npy -> validated float32 tensor (None without the flag); raises ValueError on a wrong shape, a
+    non-real dtype, NaN or +inf"""
+    if not getattr(args, "item_bias", None):
+        return None
+    from cast_b200.models import check_item_bias
+    return check_item_bias(np.load(args.item_bias), itemnum)
 
 
 def write_recommendations(model, dataset, args, rank, world):
@@ -89,7 +101,8 @@ def write_recommendations(model, dataset, args, rank, world):
     K = int(args.recommend)
     rec = build_recommend_inputs(dataset, args)
     lo, hi = cdist.shard_users(len(rec["u"]), rank, world)
-    ids, scores = recommend_users(model, rec, K, args.eval_batch, lo, hi)
+    ids, scores = recommend_users(model, rec, K, args.eval_batch, lo, hi,
+                                  item_bias=load_item_bias(args, model.itemnum))
     if world > 1:
         import torch.distributed as tdist
         parts = [None] * world
@@ -108,7 +121,8 @@ def write_similar_items(model, args, rank, world):
     from cast_b200.evaluation import similar_items_all
     K = int(args.similar_items)
     lo, hi = cdist.shard_users(model.itemnum, rank, world)
-    items, nbr, scores = similar_items_all(model, K, args.eval_batch, lo, hi, args.similarity)
+    items, nbr, scores = similar_items_all(model, K, args.eval_batch, lo, hi, args.similarity,
+                                           item_bias=load_item_bias(args, model.itemnum))
     if world > 1:
         import torch.distributed as tdist
         parts = [None] * world
@@ -167,6 +181,7 @@ def run(args, device=None, lib=None, logger=None):
     rank, world, local = cdist.init_from_env() if device is None else (0, 1, 0)
     dataset = data_partition(args.dataset, args.log_scale)
     train, valid, test, usernum, itemnum, ratingnum = dataset
+    load_item_bias(args, itemnum)    # a bad --item_bias fails here, before any training or evaluation
     num_batch = round(len(train) / args.batch_size)
     print("usernum", usernum, "itemnum", itemnum)
     cc = sum(len(v) for v in train.values())
