@@ -179,6 +179,15 @@ __device__ __forceinline__ void am_block(const AttnDims& dm, int& b, int& hh, in
   tile = ntile - 1 - (int)blockIdx.y;
 }
 
+// the same for key tiles (dK/dV): blockIdx.y = 0 is the FIRST key tile, the heaviest one -- keys are reached by every
+// later query, so the early live key tiles loop over the most query chunks and must be scheduled first
+__device__ __forceinline__ void am_block_keys(const AttnDims& dm, int& b, int& hh, int& ntile, int& tile) {
+  b = (int)blockIdx.x / dm.h;
+  hh = (int)blockIdx.x - b * dm.h;
+  ntile = (int)gridDim.y;
+  tile = (int)blockIdx.y;
+}
+
 // ------------------------------------------------------------------------------------------------ forward
 // Warps w and w+4 own the same 16 rows and split every staged chunk of 64 keys in halves (each keeps its own running
 // max / sum / O), merged through shared memory at the end -- the critical path of the late (long) row tiles halves.
@@ -668,7 +677,7 @@ __global__ void __launch_bounds__(AM_THREADS, KS <= 7 ? 2 : 1) attn_bwd_dkv_mma_
   const int t = threadIdx.x, lane = t & 31, wid = t >> 5, warp = wid & 3, kg = wid >> 2, g = lane >> 2, tig = lane & 3;
   const int T = dm.T, d = dm.d;
   int b, hh, ntile, tile;
-  am_block(dm, b, hh, ntile, tile);
+  am_block_keys(dm, b, hh, ntile, tile);
   const int k0 = am_row0(T, ntile, tile, AM_T);
   const long rowbase = (long)b * T;
   const long sbase = ((long)b * dm.h + hh) * T;
@@ -860,7 +869,7 @@ __global__ void __launch_bounds__(AW_THREADS, 2) attn_bwd_dkv_ws_kernel(AttnBwdM
   const int t = threadIdx.x, lane = t & 31, wid = t >> 5, warp = wid & 3, qg = wid >> 2, g = lane >> 2, tig = lane & 3;
   const int T = dm.T, d = dm.d;
   int b, hh, ntile, tile;
-  am_block(dm, b, hh, ntile, tile);
+  am_block_keys(dm, b, hh, ntile, tile);
   const int k0 = am_row0(T, ntile, tile, AM_T);
   const long rowbase = (long)b * T;
   int first_key, qstart;
